@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — scan-to-map registration hot path on B200 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline (every N, so that the driver's 1 -> 8 scaling is computed on ONE metric): BASELINE.json's sharded metric,
@@ -34,6 +34,10 @@ fullmap    configs[4]: construct_full_map over --fullmap-frames keyframes x 100k
 scan2map   jueying_slam's LOAM-style scan2MapOptimization for one scan (N = 1).
 gicp       pclomp GICP align of a 20k-point scan against a 1M-point map (N = 1).
 summary    the headline numbers of every leg once more, last on the line.
+
+--dump-outputs DIR writes what the headline path returned to its caller in the last timed step, the global winner's index
+and score, as DIR/reloc_best_index.npy and DIR/reloc_best_score.npy (float64).  The inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -49,6 +53,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 PARAMS = {
     # jueying_lio/config/livox.yaml:19,41-48 and config/horizon.yaml:18,37-42
@@ -155,6 +160,14 @@ def ncu_traffic(kernel):
 
 def mean(v):
     return float(np.mean(v)) if len(v) else float("nan")
+
+
+def dump_outputs(path, arrays):
+    """Writes each array as <path>/<name>.npy in float64, so that two builds run with the same arguments (hence the same
+    seeded inputs) can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), np.atleast_1d(np.asarray(a, dtype=np.float64)))
 
 
 # =============================================================================================== CPU oracle legs
@@ -773,7 +786,7 @@ def gicp_leg(args, local_rank, api, synth):
     g.covariances("target")                       # the reference computes them inside the first align (gicp_omp_impl.hpp:383-394)
     t_first = (time.perf_counter() - t0) * 1e3
     dev, wall = [], []
-    for k in range(min(args.steps, 20) + 3):
+    for k in range(args.steps + 3):
         api.flush_l2(local_rank)
         t0 = time.perf_counter()
         rc = g.align(guess)
@@ -954,6 +967,8 @@ def run_b200(args, rank, local_rank, world):
         gi = extra["gicp"]
         summ.update({"gicp_align_ms": gi["align_ms"]["device"], "gicp_cpu_align_ms": (gi.get("cpu_baseline") or {}).get("align_ms"), "gicp_parity": gi.get("parity")})
     line["summary"] = summ
+    if args.dump_outputs:   # what the caller of the headline path received in the last timed step
+        dump_outputs(args.dump_outputs, {"reloc_best_index": rel["best"], "reloc_best_score": rel["best_score"]})
     print(json.dumps(line), flush=True)
     if world > 1:
         torch.distributed.barrier()
@@ -978,7 +993,13 @@ def main():
     ap.add_argument("--fullmap-host-frames", type=int, default=800, help="keyframes of the host-buffer (e2e) pass of the configs[4] leg")
     ap.add_argument("--ref-sample", type=int, default=256, help="--impl reference: hypotheses scored per step")
     ap.add_argument("--small", action="store_true", help="DEV ONLY: shrink the maps 10x (not a valid bench number)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the headline's result of the last timed step "
+                                                         "(winning hypothesis index and score) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank, local_rank, world = dist_env()
     if args.small:
         global N_MAP, N_PRIOR
