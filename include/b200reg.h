@@ -205,6 +205,35 @@ int32_t b200_ndt_align_batch(b200_ndt* ndt, const float* guesses16, int64_t h, f
 /* min_b_ / div_b_ of the voxel grid (voxel_grid_covariance_omp_impl.hpp:86-96) */
 int32_t b200_ndt_grid(b200_ndt* ndt, int32_t* min_b3, int32_t* div_b3);
 
+/* Batched registration of independent (source, target, guess) pairs — the loop-closure call site
+ * (jueying_slam/src/mapOptmization.cpp:683-693: a fresh NDT per candidate, the keyframe as source, the history submap as
+ * target, align(guess), accepted when hasConverged() && getFitnessScore() <= historyKeyframeFitnessScore) for a whole batch
+ * of candidates in one call, everything on the device from upload to results.  A separate handle: a b200_ndt's own target
+ * and source are never touched.  A pair's result does not depend on the other pairs, on the chunking or on the ranks. */
+typedef struct b200_comm b200_comm; /* NCCL communicator (sharded paths, below) */
+typedef struct b200_ndt_pairs b200_ndt_pairs;
+typedef struct {
+    int32_t status;       /* B200_OK / B200_NOT_CONVERGED, or the error set_target / set_source / align would return for this pair alone */
+    b200_ndt_result ndt;  /* as b200_ndt_align fills it; gpu_ms = device time of the whole call */
+    double fitness;       /* getFitnessScore(max_range) at the final transformation; DBL_MAX when nothing is in range */
+    int64_t n_in_range;
+    float final16[16];    /* column-major */
+} b200_ndt_pair_result;
+
+int32_t b200_ndt_pairs_create(const b200_ndt_params* params, int32_t device, b200_ndt_pairs** out);
+int32_t b200_ndt_pairs_destroy(b200_ndt_pairs* h);
+/* Pair p: source = records src_off[p] .. src_off[p+1]-1 of src_xyz, target = records tgt_off[p] .. tgt_off[p+1]-1 of tgt_xyz
+ * (stride_bytes as everywhere); guesses16 = P x 16 column-major, NULL = identity.  comm may be NULL.  With a communicator every
+ * rank passes the same arguments, rank r registers the pairs p = r (mod N), uploads only their clouds, and every rank returns all P results.
+ * Malformed arguments (null pointers, P < 1, decreasing offsets, stride < 12) fail the whole call with B200_ERR_ARG; a problem in
+ * one pair's clouds (empty source, no finite target point, grid too large) is reported in that pair's status only. */
+int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* src_xyz, const int64_t* src_off, const float* tgt_xyz,
+                             const int64_t* tgt_off, int64_t stride_bytes, int64_t P, const float* guesses16, double max_range,
+                             b200_ndt_pair_result* results);
+/* parity probe: the valid leaves of pair p's target from the last call on this rank (as b200_ndt_leaves, leaf ids local to
+ * the pair), when pair p was built in the last chunk of that call; -1 otherwise */
+int64_t b200_ndt_pairs_leaves(b200_ndt_pairs* h, int64_t p, int64_t max, int64_t* ids, int32_t* npts, double* mean3, double* cov9, double* icov9);
+
 /* ------------------------------------------------------------------------- *
  * B3 (alternative) — Generalized ICP.  Replaces pclomp::GeneralizedIterativeClosestPoint<PointT, PointT>
  * (pointcloud_match/ndt_omp/include/pclomp/gicp_omp.h:60-135, gicp_omp_impl.hpp), the registration object
@@ -259,7 +288,6 @@ int32_t b200_gicp_index_info(b200_gicp* h, int32_t which, float* leaf, int64_t* 
  * Sharded paths (one process per GPU, NCCL over NVLink).  The reference is single-process and has no
  * counterpart (SURVEY.md F4): each hypothesis is scored with the reference's calculateScore arithmetic.
  * ------------------------------------------------------------------------- */
-typedef struct b200_comm b200_comm;
 #define B200_NCCL_ID_BYTES 128
 int32_t b200_comm_unique_id(uint8_t* id128);   /* on one rank; ship the 128 bytes to the others out of band */
 int32_t b200_comm_init_rank(int32_t nranks, int32_t rank, const uint8_t* id128, int32_t device, b200_comm** out);

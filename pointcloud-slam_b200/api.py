@@ -52,6 +52,12 @@ class NdtResult(C.Structure):
                 ("p_final", C.c_double * 6), ("gpu_ms", C.c_float)]
 
 
+class NdtPairResult(C.Structure):
+    """b200_ndt_pair_result (include/b200reg.h)."""
+    _fields_ = [("status", C.c_int32), ("ndt", NdtResult), ("fitness", C.c_double), ("n_in_range", C.c_int64),
+                ("final16", C.c_float * 16)]
+
+
 class GicpParams(C.Structure):
     _fields_ = [("k_correspondences", C.c_int32), ("gicp_epsilon", C.c_double), ("rotation_epsilon", C.c_double),
                 ("transformation_epsilon", C.c_double), ("corr_dist_threshold", C.c_double), ("max_iterations", C.c_int32),
@@ -163,6 +169,12 @@ def lib():
         L.b200_ndt_last_score_kernel_ms.argtypes = [vp]
         L.b200_ndt_score_pairs.argtypes = [vp, vp, i64, vp]
         L.b200_ndt_stream_barrier.argtypes = [vp, vp]
+    if hasattr(L, "b200_ndt_pairs_create"):  # absent from builds older than the batched pair registration (B200REG_LIB A/B timing)
+        L.b200_ndt_pairs_create.argtypes = [C.POINTER(NdtParams), i32, C.POINTER(vp)]
+        L.b200_ndt_pairs_destroy.argtypes = [vp]
+        L.b200_ndt_pairs_align.argtypes = [vp, vp, vp, vp, vp, vp, i64, i64, vp, C.c_double, vp]
+        L.b200_ndt_pairs_leaves.restype = i64
+        L.b200_ndt_pairs_leaves.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp]
     L.b200_downsampler_create.argtypes = [i32, C.POINTER(vp)]
     L.b200_downsampler_destroy.argtypes = [vp]
     L.b200_voxel_downsample.argtypes = [vp, vp, i64, i64, C.c_float, i32, vp, vp, i64, vp]
@@ -654,6 +666,104 @@ class NormalDistributionsTransform:
     def stream_barrier(self, comm):
         """Device-side rendezvous of the ranks on this handle's stream (no-op without a communicator)."""
         _check(lib().b200_ndt_stream_barrier(comm.h if comm is not None else None, self._handle()))
+
+
+class NdtPairBatch:
+    """Registration of P independent (source, target, guess) pairs in one call - the loop-closure gate of
+    mapOptmization.cpp:683-693 (a fresh NDT per candidate, align(guess), hasConverged() && getFitnessScore() <= threshold)
+    for a whole batch of candidates.  Keyword arguments are the NDT setters: resolution, step_size, outlier_ratio,
+    trans_eps, max_iter, search ("KDTREE" / "DIRECT1" / "DIRECT7" / "DIRECT26" or 0 / 1 / 7 / 27), min_pts, eig_ratio."""
+
+    _DEFAULTS = dict(resolution=1.0, step_size=0.1, outlier_ratio=0.55, trans_eps=0.1, max_iter=35, search=7, min_pts=6, eig_ratio=0.01)
+
+    def __init__(self, device=0, **setters):
+        kw = dict(self._DEFAULTS)
+        unknown = set(setters) - set(kw)
+        if unknown:
+            raise TypeError(f"unknown NDT parameter(s): {sorted(unknown)}")
+        kw.update(setters)
+        kw["search"] = {"KDTREE": 0, "DIRECT1": 1, "DIRECT7": 7, "DIRECT26": 27}.get(kw["search"], kw["search"])
+        self._p = NdtParams(kw["resolution"], kw["step_size"], kw["outlier_ratio"], kw["trans_eps"], kw["max_iter"], kw["search"],
+                            kw["min_pts"], kw["eig_ratio"])
+        self.h = C.c_void_p()
+        _check(lib().b200_ndt_pairs_create(C.byref(self._p), device, C.byref(self.h)))
+
+    def close(self):
+        if getattr(self, "h", None):
+            try:
+                lib().b200_ndt_pairs_destroy(self.h)
+            except TypeError:  # interpreter shutdown: module globals are already torn down
+                pass
+            self.h = None
+
+    __del__ = close
+
+    @staticmethod
+    def pack(clouds):
+        """A list of [n_i, 3+] clouds -> (one contiguous float32 [sum n_i, 3] array, int64 offsets [P + 1])."""
+        clouds = [np.asarray(c, dtype=np.float32) for c in clouds]
+        clouds = [c.reshape(-1, 3) if c.ndim == 1 else c[:, :3] for c in clouds]
+        off = np.zeros(len(clouds) + 1, np.int64)
+        off[1:] = np.cumsum([len(c) for c in clouds])
+        xyz = np.ascontiguousarray(np.concatenate(clouds, 0) if off[-1] else np.zeros((1, 3), np.float32), dtype=np.float32)
+        return xyz, off
+
+    def align(self, sources, targets, guesses=None, max_range=1.7976931348623157e308, comm=None):
+        """Registers pair p = (sources[p], targets[p], guesses[p] (4x4 row-major; None = identity)).  Returns a dict of
+        per-pair arrays: status, converged, iters, evals, hess_evals, final [P,4,4] (row-major), fitness, n_in_range, p_final
+        [P,6], trans_probability, score, gpu_ms, and the raw ctypes records under "records"."""
+        if len(sources) != len(targets):
+            raise ValueError("sources and targets differ in length")
+        P = len(sources)
+        src, soff = self.pack(sources)
+        tgt, toff = self.pack(targets)
+        g = None
+        if guesses is not None:
+            g = np.ascontiguousarray(np.stack([np.asarray(m, dtype=np.float32).T.reshape(16) for m in guesses]), dtype=np.float32)
+            if g.shape[0] != P:
+                raise ValueError("one guess per pair")
+        return self.align_packed(src, soff, tgt, toff, P, g, max_range, comm)
+
+    def align_packed(self, src, soff, tgt, toff, P, guesses_cm16=None, max_range=1.7976931348623157e308, comm=None):
+        """align() on clouds already in the offset layout of b200_ndt_pairs_align (guesses_cm16 = [P,16] column-major)."""
+        res = (NdtPairResult * max(P, 1))()
+        soff = np.ascontiguousarray(soff, dtype=np.int64)
+        toff = np.ascontiguousarray(toff, dtype=np.int64)
+        rc = lib().b200_ndt_pairs_align(comm.h if comm is not None else None, self.h, _p(src), _p(soff), _p(tgt), _p(toff), src.strides[0], P,
+                                        None if guesses_cm16 is None else _p(guesses_cm16), max_range, res)
+        _check(rc)
+        return self.unpack(res, P)
+
+    @staticmethod
+    def unpack(res, P):
+        out = dict(records=res)
+        out["status"] = np.array([r.status for r in res[:P]], np.int32)
+        out["converged"] = np.array([r.ndt.converged for r in res[:P]], np.int32)
+        out["iters"] = np.array([r.ndt.iters for r in res[:P]], np.int32)
+        out["evals"] = np.array([r.ndt.evals for r in res[:P]], np.int32)
+        out["hess_evals"] = np.array([r.ndt.hess_evals for r in res[:P]], np.int32)
+        out["final"] = np.array([np.array(r.final16, np.float32).reshape(4, 4).T for r in res[:P]], np.float32).reshape(P, 4, 4)
+        out["fitness"] = np.array([r.fitness for r in res[:P]])
+        out["n_in_range"] = np.array([r.n_in_range for r in res[:P]], np.int64)
+        out["p_final"] = np.array([list(r.ndt.p_final) for r in res[:P]]).reshape(P, 6)
+        out["trans_probability"] = np.array([r.ndt.trans_probability for r in res[:P]])
+        out["score"] = np.array([r.ndt.score for r in res[:P]])
+        out["gpu_ms"] = float(res[0].ndt.gpu_ms) if P else 0.0
+        return out
+
+    def leaves(self, p):
+        """The valid leaves of pair p's target from the last align() (as NormalDistributionsTransform.leaves()), or None
+        when pair p was not built in the last chunk of that call on this rank."""
+        n = lib().b200_ndt_pairs_leaves(self.h, p, 0, None, None, None, None, None)
+        if n < 0:
+            return None
+        ids = np.empty(n, np.int64)
+        npts = np.empty(n, np.int32)
+        mean = np.empty((n, 3))
+        cov = np.empty((n, 3, 3))
+        icov = np.empty((n, 3, 3))
+        lib().b200_ndt_pairs_leaves(self.h, p, n, _p(ids), _p(npts), _p(mean), _p(cov), _p(icov))
+        return dict(ids=ids, npts=npts, mean=mean, cov=cov, icov=icov)
 
 
 class Communicator:

@@ -64,10 +64,12 @@ __device__ __forceinline__ int f2ord(float f) {  // order-preserving float -> in
 }
 __device__ __forceinline__ float ord2f(int i) { return __int_as_float(i >= 0 ? i : i ^ 0x7fffffff); }
 
-// pcl::getMinMax3D over the finite points (voxel_grid_covariance_omp_impl.hpp:72)
-__global__ void k_ndt_minmax(const float4* __restrict__ pts, int64_t n, int* __restrict__ mm /*[6]: min xyz, max xyz (ordered ints)*/) {
+// pcl::getMinMax3D over the finite points of pts[0, n) (voxel_grid_covariance_omp_impl.hpp:72); this block covers the
+// indices x0, x0 + xstride, ...
+__device__ __forceinline__ void minmax_range(const float4* __restrict__ pts, int64_t n, int64_t x0, int64_t xstride,
+                                             int* __restrict__ mm /*[6]: min xyz, max xyz (ordered ints)*/) {
     float mn[3] = {3.402823466e+38f, 3.402823466e+38f, 3.402823466e+38f}, mx[3] = {-3.402823466e+38f, -3.402823466e+38f, -3.402823466e+38f};
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    for (int64_t i = x0; i < n; i += xstride) {
         const float4 p = __ldg(pts + i);
         if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) continue;
         mn[0] = fminf(mn[0], p.x); mn[1] = fminf(mn[1], p.y); mn[2] = fminf(mn[2], p.z);
@@ -87,6 +89,9 @@ __global__ void k_ndt_minmax(const float4* __restrict__ pts, int64_t n, int* __r
         }
     }
 }
+__global__ void k_ndt_minmax(const float4* __restrict__ pts, int64_t n, int* __restrict__ mm) {
+    minmax_range(pts, n, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, mm);
+}
 __global__ void k_ndt_minmax_init(int* mm) {
     if (threadIdx.x < 3) mm[threadIdx.x] = 0x7fffffff;
     else if (threadIdx.x < 6) mm[threadIdx.x] = (int)0x80000000;
@@ -97,12 +102,8 @@ struct GridDims {
     float inv_leaf;
 };
 
-// leaf id of every point (:218-223); non-finite points get the sentinel key and sort last
-__global__ void k_ndt_keys(const float4* __restrict__ pts, int n, GridDims gd, uint32_t sentinel, uint32_t* __restrict__ keys,
-                           int32_t* __restrict__ vals) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 p = __ldg(pts + i);
+// leaf id of a point (:218-223); non-finite points get the sentinel key and sort last
+__device__ __forceinline__ uint32_t leaf_key(const float4 p, const GridDims& gd, uint32_t sentinel) {
     uint32_t key = sentinel;
     if (isfinite(p.x) && isfinite(p.y) && isfinite(p.z)) {
         const int i0 = (int)(floorf(p.x * gd.inv_leaf) - (float)gd.min_b[0]);
@@ -110,7 +111,13 @@ __global__ void k_ndt_keys(const float4* __restrict__ pts, int n, GridDims gd, u
         const int i2 = (int)(floorf(p.z * gd.inv_leaf) - (float)gd.min_b[2]);
         key = (uint32_t)(i0 * gd.mul[0] + i1 * gd.mul[1] + i2 * gd.mul[2]);
     }
-    keys[i] = key;
+    return key;
+}
+__global__ void k_ndt_keys(const float4* __restrict__ pts, int n, GridDims gd, uint32_t sentinel, uint32_t* __restrict__ keys,
+                           int32_t* __restrict__ vals) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    keys[i] = leaf_key(__ldg(pts + i), gd, sentinel);
     vals[i] = i;
 }
 
@@ -248,22 +255,65 @@ __device__ __forceinline__ uint32_t spread10(uint32_t v) {
     v = (v | (v << 2)) & 0x09249249u;
     return v;
 }
-__global__ void k_ndt_source_keys(const float4* __restrict__ pts, int n, float inv_cell, uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    const float4 p = __ldg(pts + i);
+__device__ __forceinline__ uint32_t morton_key(const float4 p, float inv_cell) {
     uint32_t key = 0xFFFFFFFFu;
     if (isfinite(p.x) && isfinite(p.y) && isfinite(p.z)) {
         const int cx = min(max((int)floorf(p.x * inv_cell) + 512, 0), 1023), cy = min(max((int)floorf(p.y * inv_cell) + 512, 0), 1023),
                   cz = min(max((int)floorf(p.z * inv_cell) + 512, 0), 1023);
         key = spread10((uint32_t)cx) | (spread10((uint32_t)cy) << 1) | (spread10((uint32_t)cz) << 2);
     }
-    keys[i] = key;
+    return key;
+}
+__global__ void k_ndt_source_keys(const float4* __restrict__ pts, int n, float inv_cell, uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    keys[i] = morton_key(__ldg(pts + i), inv_cell);
     vals[i] = i;
 }
 __global__ void k_ndt_gather(const float4* __restrict__ in, const int32_t* __restrict__ idx, int n, float4* __restrict__ out) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < n) out[i] = __ldg(in + __ldg(idx + i));
+}
+
+// ------------------------------------------------------------------ independent (source, target) pairs
+// The clouds of a chunk of pairs lie end to end; off[j] .. off[j+1]-1 are pair j's points, grid row y = pair y.  The dense
+// cell tables of the targets are laid out end to end as well: pair j's leaf id l becomes the key cell_base + l, so ONE
+// stable sort, run-length encoding and scan serve every target, and k_ndt_accumulate / k_ndt_finalize run unchanged.
+struct PairGrid {
+    GridDims gd;
+    uint32_t cell_base;
+    int live;  // 0: the pair is not built (its target failed); its points take the sentinel key
+};
+__global__ void k_ndt_minmax_init_pairs(int* mm, int np) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 6 * np) mm[i] = (i % 6) < 3 ? 0x7fffffff : (int)0x80000000;
+}
+__global__ void k_ndt_minmax_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, int* __restrict__ mm) {
+    const int64_t b = off[blockIdx.y];
+    minmax_range(pts + b, off[blockIdx.y + 1] - b, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, mm + 6 * blockIdx.y);
+}
+__global__ void k_ndt_keys_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, const PairGrid* __restrict__ pg, uint32_t sentinel,
+                                 uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
+    const int64_t b = off[blockIdx.y], n = off[blockIdx.y + 1] - b;
+    const PairGrid g = pg[blockIdx.y];
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        uint32_t key = sentinel;
+        if (g.live) {
+            const uint32_t l = leaf_key(__ldg(pts + b + i), g.gd, 0xFFFFFFFFu);
+            if (l != 0xFFFFFFFFu) key = g.cell_base + l;
+        }
+        keys[b + i] = key;
+        vals[b + i] = (int32_t)(b + i);
+    }
+}
+// sources: key = (pair, Morton key of the voxel), so that one stable sort orders every pair's points as set_source does
+__global__ void k_ndt_source_keys_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, float inv_cell, uint64_t* __restrict__ keys,
+                                        int32_t* __restrict__ vals) {
+    const int64_t b = off[blockIdx.y], n = off[blockIdx.y + 1] - b;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        keys[b + i] = ((uint64_t)blockIdx.y << 32) | morton_key(__ldg(pts + b + i), inv_cell);
+        vals[b + i] = (int32_t)(b + i);
+    }
 }
 
 // ------------------------------------------------------------------ Newton / More-Thuente state machine (thread 0 of the last block)
@@ -690,12 +740,38 @@ struct EvalSmem {
 // arrive advances the state machine and releases a generation counter the other blocks wait on (all blocks are resident:
 // the launch is cooperative and the grid is one wave), so an align pays neither launch gaps, nor no-op launches after
 // convergence, nor done-flag polls from the host.  Control-block reads bypass L1 (ld.cg): it changes between evaluations.
-template <bool LOOP>
-__global__ void __launch_bounds__(EVAL_THREADS, 1) k_ndt_eval(View v, Ctl* ctls, AlignConsts k, double* partials /*[h][NACC][nbx]*/,
-                                                              unsigned int* gen /*LOOP: generation counter, zero at launch*/, int max_evals) {
+// Alignment blockIdx.y = blocks 0 .. nbx-1 of grid row y.  PAIRS = false: one target and source, every row spans the grid
+// (nbx = gridDim.x), partials [h][NACC][nbx].  PAIRS = true: independent (source, target) pairs (b200_ndt_pairs_align):
+// row y = pair y with its own view pe[y].v (source range, n_src, cell2leaf base, grid bounds, KDTREE centroids) and its
+// own block count pe[y].nbx, fixed by its own source size - blocks past it leave at once; partials [pairs][part_stride];
+// one evaluation per launch.  The work split (items per block, the ticket that elects the last block, the fixed-order
+// reduction) depends on nbx and the view alone.
+struct PairEval {
+    View v;
+    int nbx;
+};
+template <bool LOOP, bool PAIRS = false>
+__global__ void __launch_bounds__(EVAL_THREADS, 1) k_ndt_eval(View v_arg, Ctl* ctls, AlignConsts k_arg, double* partials /*[h][NACC][nbx]*/,
+                                                              unsigned int* gen /*LOOP: generation counter, zero at launch*/, int max_evals,
+                                                              const PairEval* __restrict__ pe = nullptr, int part_stride = 0) {
     Ctl* ctl = ctls + blockIdx.y;
     __shared__ EvalSmem sm;
-    const int tid = threadIdx.x, nbx = gridDim.x;
+    const int tid = threadIdx.x;
+    __shared__ View pair_view;
+    int pair_nbx = 0;
+    AlignConsts pair_k = k_arg;
+    if (PAIRS) {
+        pair_nbx = __ldg(&pe[blockIdx.y].nbx);
+        if ((int)blockIdx.x >= pair_nbx) return;
+        static_assert(sizeof(View) % 4 == 0 && sizeof(View) / 4 <= EVAL_THREADS, "View is copied word by word");
+        if (tid < (int)(sizeof(View) / 4)) ((int*)&pair_view)[tid] = __ldg((const int*)&pe[blockIdx.y].v + tid);
+        __syncthreads();
+        pair_k.n_src = pair_view.n_src;  // trans_probability = score / n_src of this pair
+    }
+    const View& v = PAIRS ? pair_view : v_arg;
+    const AlignConsts& k = PAIRS ? pair_k : k_arg;
+    const int nbx = PAIRS ? pair_nbx : gridDim.x;
+    double* const part = partials + (size_t)blockIdx.y * part_stride;  // PAIRS only
   for (int ev = 0; ev < max_evals; ++ev) {
     if (__ldcg(&ctl->done)) return;
     if (tid < 12) sm.M[tid] = __ldcg(&ctl->M[tid]);
@@ -795,7 +871,8 @@ __global__ void __launch_bounds__(EVAL_THREADS, 1) k_ndt_eval(View v, Ctl* ctls,
         double a = sm.red[0][tid];
 #pragma unroll
         for (int w = 1; w < EVAL_THREADS / 32; ++w) a += sm.red[w][tid];
-        __stcg(partials + ((size_t)blockIdx.y * NACC + tid) * nbx + blockIdx.x, a);
+        if (PAIRS) __stcg(part + (size_t)tid * nbx + blockIdx.x, a);
+        else __stcg(partials + ((size_t)blockIdx.y * NACC + tid) * nbx + blockIdx.x, a);
     }
     __threadfence();
     __syncthreads();
@@ -833,7 +910,7 @@ __global__ void __launch_bounds__(EVAL_THREADS, 1) k_ndt_eval(View v, Ctl* ctls,
     {
         const int lane = tid & 31, warp = tid >> 5;
         for (int col = warp; col < NACC; col += EVAL_THREADS / 32) {
-            const double* src = partials + ((size_t)blockIdx.y * NACC + col) * nbx;
+            const double* src = PAIRS ? part + (size_t)col * nbx : partials + ((size_t)blockIdx.y * NACC + col) * nbx;
             double a = 0.0;
             for (int b = lane; b < nbx; b += 32) a += __ldcg(src + b);
 #pragma unroll
@@ -1064,16 +1141,8 @@ struct FitView {
     float leaf, inv_leaf;
 };
 
-__global__ void __launch_bounds__(256) k_ndt_fitness(FitView f, const float4* __restrict__ src, int n, const float* __restrict__ M12g, double* __restrict__ d2_out) {
-    __shared__ float M[12];
-    if (threadIdx.x < 12) M[threadIdx.x] = M12g[threadIdx.x];
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (q >= n) return;
-    const float4 p = __ldg(src + q);
-    float x, y, z;
-    xform(M, p.x, p.y, p.z, x, y, z);
+// squared distance from (x, y, z) to its nearest target point; one warp, the result in every lane
+__device__ __forceinline__ float fitness_nn(const FitView& f, float x, float y, float z, int lane) {
     float best = 3.402823466e+38f;
     if (isfinite(x) && isfinite(y) && isfinite(z)) {
         // start cell, clamped into the grid
@@ -1118,11 +1187,48 @@ __global__ void __launch_bounds__(256) k_ndt_fitness(FitView f, const float4* __
             if (lb > 0.f && best <= (lb - 1e-4f * f.leaf) * (lb - 1e-4f * f.leaf)) break;
         }
     }
+    return best;
+}
+
+__global__ void __launch_bounds__(256) k_ndt_fitness(FitView f, const float4* __restrict__ src, int n, const float* __restrict__ M12g, double* __restrict__ d2_out) {
+    __shared__ float M[12];
+    if (threadIdx.x < 12) M[threadIdx.x] = M12g[threadIdx.x];
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (q >= n) return;
+    const float4 p = __ldg(src + q);
+    float x, y, z;
+    xform(M, p.x, p.y, p.z, x, y, z);
+    const float best = fitness_nn(f, x, y, z, lane);
     if (lane == 0) d2_out[q] = (double)best;
 }
 
-__global__ void k_ndt_fitness_reduce(const double* __restrict__ d2, int n, double max_range, double* __restrict__ out /*sum, count*/) {
-    // single block, fixed order: deterministic
+// Independent pairs: grid row y = pair y; its source range, its target index and its final transformation, read from its
+// control block on the device (row-major; the first 12 floats are the 3x4 the source is moved by).
+struct PairFit {
+    FitView f;
+    const float4* src;
+    int n;
+};
+__global__ void __launch_bounds__(256) k_ndt_fitness_pairs(const PairFit* __restrict__ pf, const Ctl* __restrict__ ctls, const int64_t* __restrict__ d2_off,
+                                                           double* __restrict__ d2_out) {
+    __shared__ float M[12];
+    if (threadIdx.x < 12) M[threadIdx.x] = ctls[blockIdx.y].final_T[threadIdx.x];
+    __syncthreads();
+    const PairFit& P = pf[blockIdx.y];
+    const int lane = threadIdx.x & 31;
+    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (q >= P.n) return;
+    const float4 p = __ldg(P.src + q);
+    float x, y, z;
+    xform(M, p.x, p.y, p.z, x, y, z);
+    const float best = fitness_nn(P.f, x, y, z, lane);
+    if (lane == 0) d2_out[d2_off[blockIdx.y] + q] = (double)best;
+}
+
+// one block, fixed order: deterministic, and the same for a pair as for the single-target path
+__device__ __forceinline__ void fitness_reduce_block(const double* __restrict__ d2, int n, double max_range, double* __restrict__ out /*sum, count*/) {
     __shared__ double ssum[256];
     __shared__ double scnt[256];
     double s = 0.0, c = 0.0;
@@ -1141,6 +1247,14 @@ __global__ void k_ndt_fitness_reduce(const double* __restrict__ d2, int n, doubl
         out[0] = S;
         out[1] = C;
     }
+}
+__global__ void k_ndt_fitness_reduce(const double* __restrict__ d2, int n, double max_range, double* __restrict__ out) {
+    fitness_reduce_block(d2, n, max_range, out);
+}
+// block y = pair y: d2[d2_off[y] .. d2_off[y + 1]) -> out[2y], out[2y + 1]
+__global__ void k_ndt_fitness_reduce_pairs(const double* __restrict__ d2, const int64_t* __restrict__ d2_off, double max_range, double* __restrict__ out) {
+    const int64_t b = d2_off[blockIdx.x], e = d2_off[blockIdx.x + 1];
+    fitness_reduce_block(d2 + b, (int)(e - b), max_range, out + 2 * blockIdx.x);
 }
 
 // ------------------------------------------------------------------ host object
@@ -1204,6 +1318,8 @@ struct Ndt {
     int32_t build_target(int64_t n);
     int32_t set_source(const float* xyz, int64_t n, int64_t stride);
     int32_t run(int h, const float* d_guesses, const double* d_p, int phase);
+    template <class Launch>
+    int32_t until_done(int h, int max_launches, int& launches, Launch launch);
     int32_t score_batch_device(const float* d_poses16, int64_t h, double* d_out);
     int32_t fitness(const float* T16_colmajor, double max_range, double* score, int64_t* nr);
 };
@@ -1352,27 +1468,18 @@ int32_t Ndt::set_target(const float* xyz, int64_t n, int64_t stride) {
     return build_target(n);
 }
 
-int32_t Ndt::build_target(int64_t n) {
-    have_target = false;
-    have_fitness_index = false;
-    n_tgt = n;
-    CUDA_TRY(cudaEventRecord(ev0, stream));
-    int* mm = d_small.p;
-    k_ndt_minmax_init<<<1, 32, 0, stream>>>(mm);
-    k_ndt_minmax<<<sm_count * 8, 256, 0, stream>>>(d_tgt.p, n, mm);
-    CUDA_TRY(cudaMemcpyAsync(h_small.p, mm, 6 * sizeof(int), cudaMemcpyDeviceToHost, stream));
-    CUDA_TRY(cudaStreamSynchronize(stream));
+// applyFilter's grid (:67-103) from the min / max of the finite points (ordered ints, as k_ndt_minmax leaves them)
+static int32_t grid_from_minmax(const int* mm6, float resolution, GridDims& gd, int64_t& ncells) {
     float mn[3], mx[3];
     for (int k = 0; k < 3; ++k) {
-        int a = h_small.p[k], b = h_small.p[3 + k];
+        int a = mm6[k], b = mm6[3 + k];
         a = a >= 0 ? a : a ^ 0x7fffffff;
         b = b >= 0 ? b : b ^ 0x7fffffff;
         memcpy(&mn[k], &a, 4);
         memcpy(&mx[k], &b, 4);
     }
     if (!(mn[0] <= mx[0])) B200_FAIL(B200_ERR_ARG, "target cloud has no finite point");
-    // applyFilter (:67-103)
-    const float inv_leaf = 1.0f / prm.resolution;
+    const float inv_leaf = 1.0f / resolution;
     const int64_t dx = (int64_t)((mx[0] - mn[0]) * inv_leaf) + 1, dy = (int64_t)((mx[1] - mn[1]) * inv_leaf) + 1,
                   dz = (int64_t)((mx[2] - mn[2]) * inv_leaf) + 1;
     if ((double)dx * (double)dy * (double)dz > (double)INT32_MAX) B200_FAIL(B200_ERR_RANGE, "leaf size too small for the target: integer leaf indices would overflow");
@@ -1385,6 +1492,21 @@ int32_t Ndt::build_target(int64_t n) {
     gd.mul[0] = 1; gd.mul[1] = gd.div_b[0]; gd.mul[2] = gd.div_b[0] * gd.div_b[1];
     ncells = (int64_t)gd.div_b[0] * gd.div_b[1] * gd.div_b[2];
     if (ncells > ((int64_t)1 << 30)) B200_FAIL(B200_ERR_RANGE, "NDT grid too large for the dense cell table (> 2^30 cells)");
+    return B200_OK;
+}
+
+int32_t Ndt::build_target(int64_t n) {
+    have_target = false;
+    have_fitness_index = false;
+    n_tgt = n;
+    CUDA_TRY(cudaEventRecord(ev0, stream));
+    int* mm = d_small.p;
+    k_ndt_minmax_init<<<1, 32, 0, stream>>>(mm);
+    k_ndt_minmax<<<sm_count * 8, 256, 0, stream>>>(d_tgt.p, n, mm);
+    CUDA_TRY(cudaMemcpyAsync(h_small.p, mm, 6 * sizeof(int), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaStreamSynchronize(stream));
+    const int32_t grc = grid_from_minmax(h_small.p, prm.resolution, gd, ncells);
+    if (grc) return grc;
     CUDA_TRY(d_cell2leaf.reserve((size_t)ncells));
     CUDA_TRY(cudaMemsetAsync(d_cell2leaf.p, 0xFF, (size_t)ncells * sizeof(int32_t), stream));
     CUDA_TRY(d_keys_in.reserve(n)); CUDA_TRY(d_keys_out.reserve(n)); CUDA_TRY(d_uniq.reserve(n));
@@ -1456,6 +1578,27 @@ int32_t Ndt::set_source(const float* xyz, int64_t n, int64_t stride) {
     return B200_OK;
 }
 
+// Enqueues evaluations of the h alignments in d_ctl until every one is done (or max_launches): batches of launches between
+// polls of the done count.
+template <class Launch>
+int32_t Ndt::until_done(int h, int max_launches, int& launches, Launch launch) {
+    int* d_left = d_small.p + 10;
+    while (launches - 1 < max_launches) {
+        // first poll after 12 evaluations: a typical relocalization align (8 iterations, 9-10 evaluations) then ends with one
+        // poll and two or three no-op launches instead of two polls and seven no-ops
+        const int batch = launches == 1 ? LAUNCH_BATCH + 4 : LAUNCH_BATCH;
+        for (int b = 0; b < batch; ++b) launch();
+        launches += batch;
+        CUDA_TRY(cudaMemsetAsync(d_left, 0, sizeof(int), stream));
+        k_ndt_count_done<<<std::min((h + 255) / 256, 64), 256, 0, stream>>>(d_ctl.p, h, d_left);
+        ++launches;
+        CUDA_TRY(cudaMemcpyAsync(h_small.p, d_left, sizeof(int), cudaMemcpyDeviceToHost, stream));
+        CUDA_TRY(cudaStreamSynchronize(stream));
+        if (h_small.p[0] == 0) break;
+    }
+    return B200_OK;
+}
+
 // Runs h independent state machines to completion.  d_guesses (h x 16, col-major) for PH_INIT, d_p (h x 6) otherwise.
 int32_t Ndt::run(int h, const float* d_guesses, const double* d_p, int phase) {
     if (!have_target) B200_FAIL(B200_ERR_ARG, "no target set");
@@ -1478,7 +1621,6 @@ int32_t Ndt::run(int h, const float* d_guesses, const double* d_p, int phase) {
     k_ndt_init<<<(h + 63) / 64, 64, 0, stream>>>(d_ctl.p, h, d_guesses, d_p, phase);
     int launches = 1;
     const bool single = phase != PH_INIT;
-    int* d_left = d_small.p + 10;
     // worst case per alignment: (max_iter + 2) iterations x (1 + 10 trials + 1 Hessian) evaluations
     const int max_launches = single ? 1 : (prm.max_iter + 3) * 12 + 1;
     static const bool persistent_ok = !(getenv("B200_NDT_LOOP") && atoi(getenv("B200_NDT_LOOP")) == 0);
@@ -1488,23 +1630,19 @@ int32_t Ndt::run(int h, const float* d_guesses, const double* d_p, int phase) {
         Ctl* ctls = d_ctl.p;
         double* parts = d_partials.p;
         int max_evals = max_launches;
-        void* args[] = {(void*)&v, (void*)&ctls, (void*)&k, (void*)&parts, (void*)&d_gen, (void*)&max_evals};
+        const PairEval* no_pairs = nullptr;
+        int no_stride = 0;
+        void* args[] = {(void*)&v, (void*)&ctls, (void*)&k, (void*)&parts, (void*)&d_gen, (void*)&max_evals, (void*)&no_pairs, (void*)&no_stride};
         CUDA_TRY(cudaLaunchCooperativeKernel((const void*)k_ndt_eval<true>, dim3(nbx, 1), dim3(EVAL_THREADS), args, 0, stream));
         ++launches;
-    } else
-    while (launches - 1 < max_launches) {
-        // first poll after 12 evaluations: a typical relocalization align (8 iterations, 9-10 evaluations) then ends with one
-        // poll and two or three no-op launches instead of two polls and seven no-ops
-        const int batch = single ? 1 : (launches == 1 ? LAUNCH_BATCH + 4 : LAUNCH_BATCH);
-        for (int b = 0; b < batch; ++b) k_ndt_eval<false><<<dim3(nbx, h), EVAL_THREADS, 0, stream>>>(v, d_ctl.p, k, d_partials.p, nullptr, 1);
-        launches += batch;
-        if (single) break;
-        CUDA_TRY(cudaMemsetAsync(d_left, 0, sizeof(int), stream));
-        k_ndt_count_done<<<std::min((h + 255) / 256, 64), 256, 0, stream>>>(d_ctl.p, h, d_left);
+    } else if (single) {
+        k_ndt_eval<false><<<dim3(nbx, h), EVAL_THREADS, 0, stream>>>(v, d_ctl.p, k, d_partials.p, nullptr, 1);
         ++launches;
-        CUDA_TRY(cudaMemcpyAsync(h_small.p, d_left, sizeof(int), cudaMemcpyDeviceToHost, stream));
-        CUDA_TRY(cudaStreamSynchronize(stream));
-        if (h_small.p[0] == 0) break;
+    } else {
+        const int32_t rc = until_done(h, max_launches, launches, [&]() {
+            k_ndt_eval<false><<<dim3(nbx, h), EVAL_THREADS, 0, stream>>>(v, d_ctl.p, k, d_partials.p, nullptr, 1);
+        });
+        if (rc) return rc;
     }
     CUDA_TRY(cudaEventRecord(ev1, stream));
     CUDA_TRY(cudaMemcpyAsync(h_ctl.p, d_ctl.p, (size_t)h * sizeof(Ctl), cudaMemcpyDeviceToHost, stream));
@@ -1602,6 +1740,325 @@ static void fill_result(const ndt::Ctl& c, float* final16, b200_ndt_result* r, f
         memcpy(r->p_final, c.p, sizeof(double) * 6);
         r->gpu_ms = ms;
     }
+}
+
+// ------------------------------------------------------------------ batched registration of independent (source, target) pairs
+// The loop-closure call site (mapOptmization.cpp:683-693) registers a keyframe against a submap and gates on
+// hasConverged() && getFitnessScore() <= threshold.  Here a whole batch of such pairs is built, aligned and scored in one
+// pass per chunk: one upload, one min / max read-back, one sort of all targets, one sort of all sources, the Newton /
+// line-search loop of every pair in the same launches, and the fitness of every pair at its final transformation on the
+// device.  A pair's work split depends on its own sizes and the parameters only, so its result is bit-identical whatever
+// else is in the batch, in which chunk it lands and on which rank it runs.
+namespace {
+constexpr int64_t kPairTgtBytes = 400;  // device bytes per target point (cloud, sorted copy, sort buffers, leaf records in the worst case)
+constexpr int64_t kPairSrcBytes = 64;   // per source point (cloud, sorted copy, 64-bit keys, indices, distances)
+constexpr int kPairMaxItemsPerThread = 8;  // (point, cell) items per thread of an evaluation: the block's pair list always holds them
+
+int pairs_chunk_max() {  // B200_NDT_PAIRS_CHUNK = most pairs per chunk (development switch; results do not depend on it)
+    static const int v = getenv("B200_NDT_PAIRS_CHUNK") ? atoi(getenv("B200_NDT_PAIRS_CHUNK")) : 0;
+    return v > 0 ? std::min(v, 65535) : 65535;
+}
+
+void pack_ranges(const float* xyz, int64_t stride, const int64_t* off, const int64_t* ids, int64_t np, const int64_t* dst_off, float4* dst) {
+    const int nt = dst_off[np] > (1 << 20) ? 8 : 1;
+    auto work = [=](int t) {
+        for (int64_t j = t; j < np; j += nt)
+            pack_xyz_float4((const float*)((const char*)xyz + off[ids[j]] * stride), dst_off[j + 1] - dst_off[j], stride, dst + dst_off[j]);
+    };
+    if (nt == 1) { work(0); return; }
+    std::vector<std::thread> th;
+    for (int t = 0; t < nt; ++t) th.emplace_back(work, t);
+    for (auto& t : th) t.join();
+}
+}  // namespace
+
+struct b200_ndt_pairs {
+    Ndt k;  // parameters, stream, events, staging and the target / source / alignment buffers, reused by every chunk
+    DevBuf<uint64_t> d_skeys_in, d_skeys_out;
+    DevBuf<int64_t> d_off, d_d2off;
+    PinnedBuf<int64_t> h_off;
+    DevBuf<int32_t> d_mm;
+    PinnedBuf<int32_t> h_mm;
+    DevBuf<ndt::PairGrid> d_pg;
+    PinnedBuf<ndt::PairGrid> h_pg;
+    DevBuf<ndt::PairEval> d_pe;
+    PinnedBuf<ndt::PairEval> h_pe;
+    DevBuf<ndt::PairFit> d_pf;
+    PinnedBuf<ndt::PairFit> h_pf;
+    DevBuf<double> d_fitsum;
+    PinnedBuf<double> h_fitsum;
+    DevBuf<uint8_t> d_xchg;
+    PinnedBuf<uint8_t> h_xchg;
+    // the last chunk this rank built (b200_ndt_pairs_leaves)
+    std::vector<int64_t> last_ids;
+    std::vector<uint32_t> last_base;
+    std::vector<int64_t> last_ncells;
+    std::vector<int> last_live;
+    int last_nruns = 0;
+
+    struct Call {
+        const float *src_xyz, *tgt_xyz;
+        const int64_t *src_off, *tgt_off;
+        int64_t stride;
+        const float* guesses16;
+        double max_range;
+        b200_ndt_pair_result* results;
+    };
+    int32_t chunk(const Call& c, const int64_t* ids, int64_t np, int64_t cell_limit, int64_t& used);
+    int32_t local(const Call& c, int64_t P, int64_t first, int64_t step);
+    void destroy() {
+        cudaSetDevice(k.device);
+        if (k.stream) cudaStreamSynchronize(k.stream);
+        d_skeys_in.release(); d_skeys_out.release(); d_off.release(); d_d2off.release(); h_off.release(); d_mm.release(); h_mm.release();
+        d_pg.release(); h_pg.release(); d_pe.release(); h_pe.release(); d_pf.release(); h_pf.release(); d_fitsum.release(); h_fitsum.release();
+        d_xchg.release(); h_xchg.release();
+        k.destroy();
+    }
+};
+
+// Builds, aligns and scores pairs ids[0 .. np-1] (all with a non-empty source and target); `used` = how many of them fit the
+// 32-bit key space / memory bound and were done (at least one).
+int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int64_t cell_limit, int64_t& used) {
+    using namespace ndt;
+    Ndt& K = k;
+    cudaStream_t s = K.stream;
+    std::vector<int64_t> toff(np + 1, 0), soff(np + 1, 0);
+    int64_t max_tn = 1, max_sn = 1;
+    for (int64_t j = 0; j < np; ++j) {
+        const int64_t tn = c.tgt_off[ids[j] + 1] - c.tgt_off[ids[j]], sn = c.src_off[ids[j] + 1] - c.src_off[ids[j]];
+        toff[j + 1] = toff[j] + tn;
+        soff[j + 1] = soff[j] + sn;
+        max_tn = std::max(max_tn, tn);
+        max_sn = std::max(max_sn, sn);
+    }
+    const int64_t nt = toff[np], ns = soff[np];
+    // one upload of every cloud of the chunk
+    CUDA_TRY(K.h_stage.reserve((size_t)(nt + ns)));
+    pack_ranges(c.tgt_xyz, c.stride, c.tgt_off, ids, np, toff.data(), K.h_stage.p);
+    pack_ranges(c.src_xyz, c.stride, c.src_off, ids, np, soff.data(), K.h_stage.p + nt);
+    CUDA_TRY(K.d_tgt.reserve((size_t)nt));
+    CUDA_TRY(K.d_src_raw.reserve((size_t)ns));
+    CUDA_TRY(cudaMemcpyAsync(K.d_tgt.p, K.h_stage.p, (size_t)nt * sizeof(float4), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(K.d_src_raw.p, K.h_stage.p + nt, (size_t)ns * sizeof(float4), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(h_off.reserve(2 * (size_t)(np + 1)));
+    CUDA_TRY(d_off.reserve(2 * (size_t)(np + 1)));
+    memcpy(h_off.p, toff.data(), (np + 1) * sizeof(int64_t));
+    memcpy(h_off.p + np + 1, soff.data(), (np + 1) * sizeof(int64_t));
+    CUDA_TRY(cudaMemcpyAsync(d_off.p, h_off.p, 2 * (np + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    const int64_t* d_toff = d_off.p;
+    const int64_t* d_soff = d_off.p + np + 1;
+    // per-target min / max, read back once for the whole chunk
+    CUDA_TRY(d_mm.reserve(6 * (size_t)np));
+    CUDA_TRY(h_mm.reserve(6 * (size_t)np));
+    k_ndt_minmax_init_pairs<<<(unsigned)((6 * np + 255) / 256), 256, 0, s>>>(d_mm.p, (int)np);
+    k_ndt_minmax_pairs<<<dim3((unsigned)std::min<int64_t>((max_tn + 1023) / 1024, 256), (unsigned)np), 256, 0, s>>>(K.d_tgt.p, d_toff, d_mm.p);
+    CUDA_TRY(cudaMemcpyAsync(h_mm.p, d_mm.p, 6 * np * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    LAUNCH_COUNT(2);
+    // every target's grid, as Ndt::build_target derives it; the dense tables end to end
+    CUDA_TRY(h_pg.reserve((size_t)np));
+    CUDA_TRY(d_pg.reserve((size_t)np));
+    int64_t cells = 0, n_live = 0;
+    used = np;
+    for (int64_t j = 0; j < np; ++j) {
+        PairGrid& g = h_pg.p[j];
+        memset(&g, 0, sizeof g);
+        int64_t nc = 0;
+        const int32_t st = grid_from_minmax(h_mm.p + 6 * j, K.prm.resolution, g.gd, nc);
+        if (st) {
+            memset(&g, 0, sizeof g);
+            c.results[ids[j]].status = st;
+            continue;
+        }
+        if (cells + nc > cell_limit && j > 0) { used = j; break; }
+        g.cell_base = (uint32_t)cells;
+        g.live = 1;
+        cells += nc;
+        ++n_live;
+    }
+    np = used;
+    last_ids.assign(ids, ids + np);
+    last_base.resize(np);
+    last_ncells.resize(np);
+    last_live.resize(np);
+    for (int64_t j = 0; j < np; ++j) {
+        const PairGrid& g = h_pg.p[j];
+        last_base[j] = g.cell_base;
+        last_ncells[j] = g.live ? (int64_t)g.gd.div_b[0] * g.gd.div_b[1] * g.gd.div_b[2] : 0;
+        last_live[j] = g.live;
+    }
+    last_nruns = 0;
+    if (!n_live) return B200_OK;
+    const int64_t nt_u = toff[np], ns_u = soff[np];
+    CUDA_TRY(cudaMemcpyAsync(d_pg.p, h_pg.p, np * sizeof(PairGrid), cudaMemcpyHostToDevice, s));
+    // segmented target build: one stable sort of (cell_base + leaf id) over every target, then the single-target kernels
+    const uint32_t sentinel = (uint32_t)cells;
+    CUDA_TRY(K.d_keys_in.reserve(nt_u)); CUDA_TRY(K.d_keys_out.reserve(nt_u)); CUDA_TRY(K.d_uniq.reserve(nt_u));
+    CUDA_TRY(K.d_vals_in.reserve(nt_u)); CUDA_TRY(K.d_vals_out.reserve(nt_u)); CUDA_TRY(K.d_run_cnt.reserve(nt_u)); CUDA_TRY(K.d_run_off.reserve(nt_u));
+    k_ndt_keys_pairs<<<dim3((unsigned)std::min<int64_t>((max_tn + 255) / 256, 1024), (unsigned)np), 256, 0, s>>>(K.d_tgt.p, d_toff, d_pg.p, sentinel,
+                                                                                                           K.d_keys_in.p, K.d_vals_in.p);
+    int end_bit = 1;
+    while (end_bit < 32 && ((int64_t)1 << end_bit) <= cells) ++end_bit;
+    int32_t* d_nruns = K.d_small.p + 8;
+    size_t t1 = 0, t2 = 0, t3 = 0;
+    cub::DeviceRadixSort::SortPairs(nullptr, t1, K.d_keys_in.p, K.d_keys_out.p, K.d_vals_in.p, K.d_vals_out.p, (int)nt_u, 0, end_bit, s);
+    cub::DeviceRunLengthEncode::Encode(nullptr, t2, K.d_keys_out.p, K.d_uniq.p, K.d_run_cnt.p, d_nruns, (int)nt_u, s);
+    cub::DeviceScan::ExclusiveSum(nullptr, t3, K.d_run_cnt.p, K.d_run_off.p, (int)nt_u, s);
+    size_t tmp = std::max(t1, std::max(t2, t3));
+    CUDA_TRY(K.cub_tmp.reserve(tmp));
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(K.cub_tmp.p, tmp, K.d_keys_in.p, K.d_keys_out.p, K.d_vals_in.p, K.d_vals_out.p, (int)nt_u, 0, end_bit, s));
+    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(K.cub_tmp.p, tmp, K.d_keys_out.p, K.d_uniq.p, K.d_run_cnt.p, d_nruns, (int)nt_u, s));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(K.cub_tmp.p, tmp, K.d_run_cnt.p, K.d_run_off.p, (int)nt_u, s));
+    CUDA_TRY(cudaMemcpyAsync(K.h_small.p, d_nruns, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    const int nruns = K.h_small.p[0];
+    CUDA_TRY(K.d_sums.reserve((size_t)nruns * 9));
+    CUDA_TRY(K.d_centroid.reserve((size_t)nruns * 3 + 4));
+    CUDA_TRY(K.d_leafF.reserve(nruns)); CUDA_TRY(K.d_leafD.reserve(nruns)); CUDA_TRY(K.d_cov.reserve((size_t)nruns * 9));
+    CUDA_TRY(K.d_npts.reserve(nruns)); CUDA_TRY(K.d_valid.reserve(nruns));
+    CUDA_TRY(K.d_cell2leaf.reserve((size_t)cells));
+    CUDA_TRY(K.d_cell2run.reserve((size_t)cells));
+    CUDA_TRY(cudaMemsetAsync(K.d_cell2leaf.p, 0xFF, (size_t)cells * sizeof(int32_t), s));
+    CUDA_TRY(cudaMemsetAsync(K.d_cell2run.p, 0xFF, (size_t)cells * sizeof(int32_t), s));
+    int32_t* d_nvalid = K.d_small.p + 9;
+    CUDA_TRY(cudaMemsetAsync(d_nvalid, 0, sizeof(int32_t), s));
+    CUDA_TRY(cudaMemsetAsync(K.d_cov.p, 0, (size_t)nruns * 9 * sizeof(double), s));
+    const int acc_blocks = std::min((nruns + 7) / 8, K.sm_count * 8);
+    k_ndt_accumulate<<<std::max(acc_blocks, 1), 256, 0, s>>>(K.d_tgt.p, K.d_vals_out.p, K.d_uniq.p, K.d_run_off.p, K.d_run_cnt.p, d_nruns, sentinel,
+                                                             K.d_sums.p, K.d_centroid.p);
+    k_ndt_finalize<<<(nruns + 127) / 128, 128, 0, s>>>(K.d_uniq.p, K.d_run_cnt.p, d_nruns, sentinel, K.d_sums.p, K.prm.min_pts, K.prm.eig_ratio,
+                                                       K.d_leafF.p, K.d_leafD.p, K.d_cov.p, K.d_npts.p, K.d_valid.p, K.d_cell2leaf.p, d_nvalid);
+    // fitness index: target points in cell order, cell -> run
+    CUDA_TRY(K.d_tgt_sorted.reserve((size_t)nt_u));
+    k_ndt_gather<<<(unsigned)((nt_u + 255) / 256), 256, 0, s>>>(K.d_tgt.p, K.d_vals_out.p, (int)nt_u, K.d_tgt_sorted.p);
+    k_ndt_cell_runs<<<(nruns + 255) / 256, 256, 0, s>>>(K.d_uniq.p, d_nruns, sentinel, K.d_cell2run.p);
+    last_nruns = nruns;
+    // sources: one stable sort by (pair, Morton key), so every pair is ordered as set_source orders it alone
+    CUDA_TRY(d_skeys_in.reserve(ns_u)); CUDA_TRY(d_skeys_out.reserve(ns_u));
+    CUDA_TRY(K.s_vals_in.reserve(ns_u)); CUDA_TRY(K.s_vals_out.reserve(ns_u)); CUDA_TRY(K.d_src.reserve((size_t)ns_u));
+    k_ndt_source_keys_pairs<<<dim3((unsigned)std::min<int64_t>((max_sn + 255) / 256, 1024), (unsigned)np), 256, 0, s>>>(
+        K.d_src_raw.p, d_soff, 1.0f / K.prm.resolution, d_skeys_in.p, K.s_vals_in.p);
+    int s_end = 33;
+    while (s_end < 64 && ((int64_t)1 << (s_end - 32)) < np) ++s_end;
+    tmp = 0;
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp, d_skeys_in.p, d_skeys_out.p, K.s_vals_in.p, K.s_vals_out.p, (int)ns_u, 0, s_end, s));
+    CUDA_TRY(K.s_tmp.reserve(tmp));
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(K.s_tmp.p, tmp, d_skeys_in.p, d_skeys_out.p, K.s_vals_in.p, K.s_vals_out.p, (int)ns_u, 0, s_end, s));
+    k_ndt_gather<<<(unsigned)((ns_u + 255) / 256), 256, 0, s>>>(K.d_src_raw.p, K.s_vals_out.p, (int)ns_u, K.d_src.p);
+    LAUNCH_COUNT(7);
+    // alignment: one control block and one view per built pair
+    K.gauss();  // recomputed at every computeTransformation (ndt_omp_impl.hpp:77-81)
+    View base = K.view();
+    base.nbr7 = nullptr;
+    CUDA_TRY(h_pe.reserve((size_t)n_live)); CUDA_TRY(d_pe.reserve((size_t)n_live));
+    CUDA_TRY(h_pf.reserve((size_t)n_live)); CUDA_TRY(d_pf.reserve((size_t)n_live));
+    CUDA_TRY(K.h_poses.reserve((size_t)n_live * 16)); CUDA_TRY(K.d_poses.reserve((size_t)n_live * 16));
+    std::vector<int64_t> live(n_live), d2off(n_live + 1, 0);
+    int max_nbx = 1;
+    int64_t max_live_sn = 1;
+    for (int64_t j = 0, a = 0; j < np; ++j) {
+        const PairGrid& g = h_pg.p[j];
+        if (!g.live) continue;
+        live[a] = j;
+        const int64_t sn = soff[j + 1] - soff[j];
+        PairEval& e = h_pe.p[a];
+        e.v = base;
+        e.v.src = K.d_src.p + soff[j];
+        e.v.n_src = (int)sn;
+        e.v.cell2leaf = K.d_cell2leaf.p + g.cell_base;
+        for (int q = 0; q < 3; ++q) { e.v.min_b[q] = g.gd.min_b[q]; e.v.max_b[q] = g.gd.max_b[q]; e.v.mul[q] = g.gd.mul[q]; }
+        const int64_t items = sn * K.nst();
+        e.nbx = (int)std::max<int64_t>(1, (items + EVAL_THREADS * kPairMaxItemsPerThread - 1) / (EVAL_THREADS * kPairMaxItemsPerThread));
+        max_nbx = std::max(max_nbx, e.nbx);
+        PairFit& f = h_pf.p[a];
+        f.f.pts = K.d_tgt_sorted.p; f.f.cell2run = K.d_cell2run.p + g.cell_base; f.f.run_off = K.d_run_off.p; f.f.run_cnt = K.d_run_cnt.p;
+        for (int q = 0; q < 3; ++q) { f.f.min_b[q] = g.gd.min_b[q]; f.f.div_b[q] = g.gd.div_b[q]; }
+        f.f.leaf = K.prm.resolution; f.f.inv_leaf = g.gd.inv_leaf;
+        f.src = e.v.src;
+        f.n = (int)sn;
+        d2off[a + 1] = d2off[a] + sn;
+        max_live_sn = std::max(max_live_sn, sn);
+        float* G = K.h_poses.p + a * 16;
+        if (c.guesses16) memcpy(G, c.guesses16 + ids[j] * 16, 16 * sizeof(float));
+        else for (int q = 0; q < 16; ++q) G[q] = (q % 5 == 0) ? 1.f : 0.f;
+        ++a;
+    }
+    CUDA_TRY(cudaMemcpyAsync(d_pe.p, h_pe.p, n_live * sizeof(PairEval), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(d_pf.p, h_pf.p, n_live * sizeof(PairFit), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(K.d_poses.p, K.h_poses.p, n_live * 16 * sizeof(float), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(K.d_ctl.reserve(n_live)); CUDA_TRY(K.h_ctl.reserve(n_live));
+    const int part_stride = NACC * max_nbx;
+    CUDA_TRY(K.d_partials.reserve((size_t)n_live * part_stride));
+    AlignConsts kc{K.prm.step_size, K.prm.trans_eps, K.prm.max_iter, 0};
+    k_ndt_init<<<(unsigned)((n_live + 63) / 64), 64, 0, s>>>(K.d_ctl.p, (int)n_live, K.d_poses.p, nullptr, PH_INIT);
+    int launches = 1;
+    const int max_launches = (K.prm.max_iter + 3) * 12 + 1;
+    int32_t rc = K.until_done((int)n_live, max_launches, launches, [&]() {
+        k_ndt_eval<false, true><<<dim3(max_nbx, (unsigned)n_live), EVAL_THREADS, 0, s>>>(View{}, K.d_ctl.p, kc, K.d_partials.p, nullptr, 1, d_pe.p,
+                                                                                            part_stride);
+    });
+    LAUNCH_COUNT(launches);
+    if (rc) return rc;
+    // getFitnessScore(max_range) of every pair at its final transformation, read from its control block on the device
+    CUDA_TRY(d_d2off.reserve((size_t)n_live + 1));
+    CUDA_TRY(h_off.reserve((size_t)n_live + 1));
+    memcpy(h_off.p, d2off.data(), (n_live + 1) * sizeof(int64_t));  // h_off's chunk offsets reached the device before the last poll
+    CUDA_TRY(cudaMemcpyAsync(d_d2off.p, h_off.p, (n_live + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(K.d_fit.reserve((size_t)d2off[n_live]));
+    CUDA_TRY(d_fitsum.reserve(2 * (size_t)n_live)); CUDA_TRY(h_fitsum.reserve(2 * (size_t)n_live));
+    k_ndt_fitness_pairs<<<dim3((unsigned)((max_live_sn * 32 + 255) / 256), (unsigned)n_live), 256, 0, s>>>(d_pf.p, K.d_ctl.p, d_d2off.p, K.d_fit.p);
+    k_ndt_fitness_reduce_pairs<<<(unsigned)n_live, 256, 0, s>>>(K.d_fit.p, d_d2off.p, c.max_range, d_fitsum.p);
+    LAUNCH_COUNT(3);
+    CUDA_TRY(cudaMemcpyAsync(K.h_ctl.p, K.d_ctl.p, n_live * sizeof(Ctl), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(h_fitsum.p, d_fitsum.p, 2 * n_live * sizeof(double), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    CUDA_TRY(cudaGetLastError());
+    for (int64_t a = 0; a < n_live; ++a) {
+        const Ctl& ct = K.h_ctl.p[a];
+        b200_ndt_pair_result& r = c.results[ids[live[a]]];
+        fill_result(ct, r.final16, &r.ndt, 0.f);
+        r.status = !ct.done ? B200_ERR_CUDA : ct.converged ? B200_OK : B200_NOT_CONVERGED;
+        const double S = h_fitsum.p[2 * a], Cn = h_fitsum.p[2 * a + 1];
+        r.n_in_range = (int64_t)Cn;
+        r.fitness = Cn > 0 ? S / Cn : 1.7976931348623157e308;  // PCL returns DBL_MAX when nothing is in range
+    }
+    return B200_OK;
+}
+
+// This rank's pairs first, first + step, ... < P: statuses of the pairs that fail on their own, then chunks of the rest.
+int32_t b200_ndt_pairs::local(const Call& c, int64_t P, int64_t first, int64_t step) {
+    std::vector<int64_t> cand;
+    for (int64_t p = first; p < P; p += step) {
+        b200_ndt_pair_result& r = c.results[p];
+        memset(&r, 0, sizeof r);
+        const int64_t tn = c.tgt_off[p + 1] - c.tgt_off[p], sn = c.src_off[p + 1] - c.src_off[p];
+        // the codes b200_ndt_set_target / b200_ndt_set_source return for these clouds
+        if (tn < 1 || tn > (int64_t)0x7fffff00) r.status = B200_ERR_ARG;
+        else if (sn < 1 || sn > (1 << 28)) r.status = B200_ERR_ARG;
+        else cand.push_back(p);
+    }
+    size_t free_b = 0, total_b = 0;
+    CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+    const int64_t budget = (int64_t)(0.6 * (double)free_b);
+    const int64_t cell_limit = std::min<int64_t>(((int64_t)1 << 32) - 2, std::max<int64_t>(budget / 4 / 8, (int64_t)1 << 30));
+    const int64_t max_np = pairs_chunk_max();
+    for (size_t i = 0; i < cand.size();) {
+        size_t e = i;
+        int64_t bytes = 0, nt = 0, ns = 0;
+        while (e < cand.size() && (int64_t)(e - i) < max_np) {
+            const int64_t p = cand[e];
+            const int64_t tn = c.tgt_off[p + 1] - c.tgt_off[p], sn = c.src_off[p + 1] - c.src_off[p];
+            const int64_t add = tn * kPairTgtBytes + sn * kPairSrcBytes;
+            if (e > i && (bytes + add > budget * 3 / 4 || nt + tn > (int64_t)0x7fffff00 || ns + sn > (int64_t)0x7fffff00)) break;
+            bytes += add; nt += tn; ns += sn;
+            ++e;
+        }
+        int64_t used = 0;
+        const int32_t rc = chunk(c, cand.data() + i, (int64_t)(e - i), cell_limit, used);
+        if (rc) return rc;
+        i += (size_t)std::max<int64_t>(used, 1);
+    }
+    return B200_OK;
 }
 
 extern "C" {
@@ -1992,6 +2449,121 @@ int32_t b200_reloc_argmin(b200_comm* comm, b200_ndt* n, const float* poses16, in
 int32_t b200_reloc_argmin_strided(b200_comm* comm, b200_ndt* n, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride, int64_t* best,
                                   double* best_score, float* gpu_ms) {
     return reloc_argmin_impl(comm, n, poses16, h, h_begin, h_stride, best, best_score, gpu_ms);
+}
+
+
+int32_t b200_ndt_pairs_create(const b200_ndt_params* params, int32_t device, b200_ndt_pairs** out) {
+    if (!params || !out) B200_FAIL(B200_ERR_ARG, "null argument");
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) B200_FAIL(B200_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) B200_FAIL(B200_ERR_ARG, "bad device ordinal");
+    b200_ndt_pairs* h = new b200_ndt_pairs();
+    const int32_t rc = h->k.init(params, device);
+    if (rc != B200_OK) { h->destroy(); delete h; return rc; }
+    *out = h;
+    return B200_OK;
+}
+int32_t b200_ndt_pairs_destroy(b200_ndt_pairs* h) {
+    if (!h) return B200_OK;
+    h->destroy();
+    delete h;
+    return B200_OK;
+}
+
+/* P independent registrations (loop-closure candidates): see include/b200reg.h.  With a communicator of N ranks, rank r
+ * registers the pairs p = r (mod N); the results and every rank's call status travel in ONE ncclAllGather of fixed-size
+ * slots (ceil(P / N) records each), so all ranks return the same code and the same P results, and a rank that failed
+ * locally still takes part in the collective. */
+int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* src_xyz, const int64_t* src_off, const float* tgt_xyz,
+                             const int64_t* tgt_off, int64_t stride_bytes, int64_t P, const float* guesses16, double max_range,
+                             b200_ndt_pair_result* results) {
+    if (!h || !src_xyz || !src_off || !tgt_xyz || !tgt_off || !results || P < 1 || stride_bytes < 12) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (src_off[0] < 0 || tgt_off[0] < 0) B200_FAIL(B200_ERR_ARG, "negative offset");
+    for (int64_t p = 0; p < P; ++p)
+        if (src_off[p + 1] < src_off[p] || tgt_off[p + 1] < tgt_off[p]) B200_FAIL(B200_ERR_ARG, "offsets must not decrease");
+    Ndt& K = h->k;
+    CUDA_SET_DEVICE(K.device);
+    const int R = comm && comm->nranks > 1 ? comm->nranks : 1, me = R > 1 ? comm->rank : 0;
+    const int64_t per = (P + R - 1) / R;
+    const size_t rec = sizeof(b200_ndt_pair_result), slot = 8 + (size_t)per * rec;
+    if (R > 1) {  // before any work: past this point every rank reaches the collective
+        CUDA_TRY(h->h_xchg.reserve(slot * (R + 1)));
+        CUDA_TRY(h->d_xchg.reserve(slot * (R + 1)));
+    }
+    const b200_ndt_pairs::Call c{src_xyz, tgt_xyz, src_off, tgt_off, stride_bytes, guesses16, max_range, results};
+    CUDA_TRY(cudaEventRecord(K.ev0, K.stream));
+    const int32_t rc_local = h->local(c, P, me, R);
+    const std::string err_local = rc_local ? g_last_error : std::string();
+    if (R == 1 && rc_local) return rc_local;
+    if (R > 1) {
+        uint8_t* hs = h->h_xchg.p;
+        memset(hs, 0, 8);
+        memcpy(hs, &rc_local, sizeof(int32_t));
+        for (int64_t i = 0, p = me; p < P; ++i, p += R) memcpy(hs + 8 + i * rec, &results[p], rec);
+        CUDA_TRY(cudaMemcpyAsync(h->d_xchg.p, hs, slot, cudaMemcpyHostToDevice, K.stream));
+        NCCL_TRY(comm, comm->AllGather(h->d_xchg.p, h->d_xchg.p + slot, slot, ncclChar, comm->comm, K.stream));
+        CUDA_TRY(cudaMemcpyAsync(hs + slot, h->d_xchg.p + slot, slot * R, cudaMemcpyDeviceToHost, K.stream));
+        CUDA_TRY(cudaStreamSynchronize(K.stream));
+        int32_t rc = B200_OK;
+        int bad = -1;
+        for (int q = 0; q < R; ++q) {
+            const uint8_t* b = hs + slot * (q + 1);
+            int32_t sq;
+            memcpy(&sq, b, sizeof sq);
+            if (sq && rc == B200_OK) { rc = sq; bad = q; }
+            for (int64_t i = 0, p = q; p < P; ++i, p += R) {
+                memcpy(&results[p], b + 8 + i * rec, rec);
+                if (sq) results[p].status = sq;
+            }
+        }
+        if (rc) {
+            if (bad == me) g_last_error = err_local;
+            else fail(rc, ("NDT pair registration failed on rank " + std::to_string(bad)).c_str(), __FILE__, __LINE__);
+            return rc;
+        }
+    }
+    CUDA_TRY(cudaEventRecord(K.ev1, K.stream));
+    CUDA_TRY(cudaEventSynchronize(K.ev1));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, K.ev0, K.ev1);
+    K.last_ms = ms;
+    for (int64_t p = 0; p < P; ++p) results[p].ndt.gpu_ms = ms;
+    return B200_OK;
+}
+
+int64_t b200_ndt_pairs_leaves(b200_ndt_pairs* h, int64_t p, int64_t max, int64_t* ids, int32_t* npts, double* mean3, double* cov9, double* icov9) {
+    if (!h) return -1;
+    size_t j = 0;
+    while (j < h->last_ids.size() && h->last_ids[j] != p) ++j;
+    if (j == h->last_ids.size() || !h->last_live[j]) return -1;
+    Ndt& k = h->k;
+    cudaSetDevice(k.device);
+    const int nr = h->last_nruns;
+    std::vector<uint8_t> valid(nr);
+    std::vector<uint32_t> uniq(nr);
+    std::vector<int32_t> np(nr);
+    std::vector<ndt::LeafD> L(nr);
+    std::vector<double> cov((size_t)nr * 9);
+    cudaStreamSynchronize(k.stream);
+    cudaMemcpy(valid.data(), k.d_valid.p, nr, cudaMemcpyDeviceToHost);
+    cudaMemcpy(uniq.data(), k.d_uniq.p, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(np.data(), k.d_npts.p, nr * sizeof(int32_t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(L.data(), k.d_leafD.p, nr * sizeof(ndt::LeafD), cudaMemcpyDeviceToHost);
+    cudaMemcpy(cov.data(), k.d_cov.p, (size_t)nr * 9 * sizeof(double), cudaMemcpyDeviceToHost);
+    const uint64_t lo = h->last_base[j], hi = lo + (uint64_t)h->last_ncells[j];
+    int64_t cnt = 0;
+    for (int r = 0; r < nr; ++r) {  // runs are sorted by key = cell_base + leaf id
+        if (!valid[r] || uniq[r] < lo || uniq[r] >= hi) continue;
+        if (cnt < max) {
+            if (ids) ids[cnt] = (int64_t)(uniq[r] - lo);
+            if (npts) npts[cnt] = np[r];
+            if (mean3) memcpy(mean3 + cnt * 3, L[r].mean, 24);
+            if (cov9) memcpy(cov9 + cnt * 9, &cov[(size_t)r * 9], 72);
+            if (icov9) memcpy(icov9 + cnt * 9, L[r].icov, 72);
+        }
+        ++cnt;
+    }
+    return cnt;
 }
 
 }  // extern "C"

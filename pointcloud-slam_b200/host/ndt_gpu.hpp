@@ -9,6 +9,8 @@
 // 4x4 transforms are float[16] column-major, i.e. Eigen::Matrix4f::data().
 #pragma once
 #include <memory>
+#include <stdexcept>
+#include <vector>
 
 #include "ivox_gpu.hpp"
 
@@ -109,6 +111,80 @@ class NormalDistributionsTransform {
     std::shared_ptr<const CloudT> target_, source_;
     float final_[16];
     b200_ndt_result result_{};
+};
+
+/// Batched loop-closure registration (b200_ndt_pairs_align): P independent (source, target, guess) pairs in one call, each
+/// exactly what a fresh pclomp NDT with these settings would compute for it alone.  A batched performLoopClosure thread or
+/// an offline loop-verification tool fills the candidate lists and reads hasConverged(p) / getFitnessScore(p) /
+/// getFinalTransformation(p), the three quantities mapOptmization.cpp:683-693 gates on.
+template <typename CloudT>
+class NdtPairBatch {
+   public:
+    explicit NdtPairBatch(int device = 0) : device_(device) {
+        prm_.resolution = 1.0f; prm_.step_size = 0.1; prm_.outlier_ratio = 0.55; prm_.trans_eps = 0.1;
+        prm_.max_iter = 35; prm_.search = 7; prm_.min_pts = 6; prm_.eig_ratio = 0.01;
+    }
+    ~NdtPairBatch() { b200_ndt_pairs_destroy(h_); }
+    NdtPairBatch(const NdtPairBatch&) = delete;
+    NdtPairBatch& operator=(const NdtPairBatch&) = delete;
+
+    void setResolution(float r) { prm_.resolution = r; dirty_ = true; }
+    void setStepSize(double s) { prm_.step_size = s; dirty_ = true; }
+    void setOutlierRatio(double o) { prm_.outlier_ratio = o; dirty_ = true; }
+    void setTransformationEpsilon(double e) { prm_.trans_eps = e; dirty_ = true; }
+    void setMaximumIterations(int n) { prm_.max_iter = n; dirty_ = true; }
+    void setNumThreads(int) {}
+    void setNeighborhoodSearchMethod(NeighborSearchMethod m) {
+        prm_.search = m == KDTREE ? 0 : m == DIRECT1 ? 1 : m == DIRECT26 ? 27 : 7;
+        dirty_ = true;
+    }
+
+    /// sources[p] / targets[p] = pair p; guesses16 = P x 16 column-major (NULL = identity, as the reference calls it);
+    /// max_range = the getFitnessScore argument.  Per-pair failures (an empty cloud, a target without a finite point) are in
+    /// status(p); a malformed call throws.
+    void align(const std::vector<const CloudT*>& sources, const std::vector<const CloudT*>& targets, const float* guesses16 = nullptr,
+               double max_range = 1.7976931348623157e308) {
+        if (sources.size() != targets.size() || sources.empty()) throw std::runtime_error("NdtPairBatch::align: one target per source, at least one pair");
+        if (!h_ || dirty_) {
+            if (h_) b200_ndt_pairs_destroy(h_);
+            h_ = nullptr;
+            check(b200_ndt_pairs_create(&prm_, device_, &h_), "b200_ndt_pairs_create");
+            dirty_ = false;
+        }
+        const size_t P = sources.size();
+        std::vector<int64_t> soff(P + 1, 0), toff(P + 1, 0);
+        for (size_t p = 0; p < P; ++p) {
+            soff[p + 1] = soff[p] + (int64_t)sources[p]->points.size();
+            toff[p + 1] = toff[p] + (int64_t)targets[p]->points.size();
+        }
+        src_.resize(3 * (size_t)std::max<int64_t>(soff[P], 1));
+        tgt_.resize(3 * (size_t)std::max<int64_t>(toff[P], 1));
+        for (size_t p = 0; p < P; ++p) {
+            float* s = src_.data() + 3 * soff[p];
+            for (const auto& q : sources[p]->points) { *s++ = q.x; *s++ = q.y; *s++ = q.z; }
+            float* t = tgt_.data() + 3 * toff[p];
+            for (const auto& q : targets[p]->points) { *t++ = q.x; *t++ = q.y; *t++ = q.z; }
+        }
+        res_.assign(P, b200_ndt_pair_result{});
+        check(b200_ndt_pairs_align(nullptr, h_, src_.data(), soff.data(), tgt_.data(), toff.data(), 12, (int64_t)P, guesses16, max_range, res_.data()),
+              "b200_ndt_pairs_align");
+    }
+    size_t size() const { return res_.size(); }
+    int status(size_t p) const { return res_.at(p).status; }
+    bool hasConverged(size_t p) const { return res_.at(p).status == B200_OK && res_[p].ndt.converged != 0; }
+    const float* getFinalTransformation(size_t p) const { return res_.at(p).final16; }   // column-major 4x4
+    double getFitnessScore(size_t p) const { return res_.at(p).fitness; }
+    int getFinalNumIteration(size_t p) const { return res_.at(p).ndt.iters; }
+    double getTransformationProbability(size_t p) const { return res_.at(p).ndt.trans_probability; }
+    const b200_ndt_pair_result& result(size_t p) const { return res_.at(p); }
+
+   private:
+    int device_;
+    b200_ndt_params prm_{};
+    b200_ndt_pairs* h_ = nullptr;
+    bool dirty_ = true;
+    std::vector<float> src_, tgt_;
+    std::vector<b200_ndt_pair_result> res_;
 };
 
 }  // namespace b200host

@@ -276,6 +276,33 @@ def hypothesis_grid(p_center, nx=32, ny=32, nyaw=4, pitch=1.0) -> np.ndarray:
     return np.ascontiguousarray(np.stack(out, 0))
 
 
+def loop_pairs(P, n_src, n_tgt, seed: int = SEED, drift=(0.3, 2.0), crop_radius=35.0, map_points=None):
+    """P loop-closure candidates as mapOptmization.cpp:683-693 registers them (keyframe = source, submap = target, identity
+    guess).  Pair p: an anchor pose in the warehouse; the target is the seeded prior map cropped to crop_radius (m, in x/y)
+    around the anchor and subsampled to n_tgt[p] points; the source is a raycast scan of n_src[p] points from the anchor,
+    moved into the map frame by a drifted pose (up to drift[0] m in x/y and drift[1] degrees in yaw off the anchor).
+    n_src / n_tgt are scalars or length-P sequences.  Returns dict(sources, targets, guesses, T_true): T_true[p] (4x4) is
+    the correction that undoes the drift, i.e. what align() should return."""
+    n_src = np.broadcast_to(np.asarray(n_src, dtype=np.int64), (P,))
+    n_tgt = np.broadcast_to(np.asarray(n_tgt, dtype=np.int64), (P,))
+    world = make_world(seed, beams=True)
+    mp = sample_map(map_points or max(2_000_000, 12 * int(n_tgt.max())), seed, world=world)
+    rng = np.random.default_rng(seed + 21)
+    sources, targets, T_true = [], [], []
+    for p in range(P):
+        anchor = np.array([rng.uniform(-45.0, 45.0), rng.uniform(-28.0, 28.0), rng.uniform(1.0, 2.0), 0.0, 0.0, rng.uniform(-np.pi, np.pi)])
+        Ta = pose_vec_to_matrix(anchor)
+        near = np.flatnonzero(np.hypot(mp[:, 0] - Ta[0, 3], mp[:, 1] - Ta[1, 3]) < crop_radius)
+        targets.append(np.ascontiguousarray(mp[np.sort(rng.choice(near, size=min(int(n_tgt[p]), len(near)), replace=False))]))
+        dirs = livox_dirs(int(n_src[p] * 1.5) + 64, seed + 1000 + p)
+        scan = raycast(Ta[:3, 3], Ta[:3, :3], dirs, world, seed=seed + 1000 + p)[: int(n_src[p])]
+        r, a = drift[0] * np.sqrt(rng.uniform()), rng.uniform(-np.pi, np.pi)
+        Td = Ta @ pose_vec_to_matrix([r * np.cos(a), r * np.sin(a), 0.0, 0.0, 0.0, np.deg2rad(drift[1]) * rng.uniform(-1.0, 1.0)])
+        sources.append(np.ascontiguousarray((scan.astype(np.float64) @ Td[:3, :3].T + Td[:3, 3]).astype(np.float32)))
+        T_true.append(Ta @ np.linalg.inv(Td))
+    return dict(sources=sources, targets=targets, guesses=[np.eye(4, dtype=np.float32)] * P, T_true=np.array(T_true))
+
+
 # ---- LOAM scene (jueying_slam scan-to-map): surface map + edge ("corner") map and a scan of both in the lidar frame ----
 def pcl_transform(t6):
     """pcl::getTransformation(x, y, z, roll, pitch, yaw) for t6 = (roll, pitch, yaw, x, y, z): (R[3,3], t[3]) in fp64."""
