@@ -325,7 +325,9 @@ typedef struct b200_downsampler b200_downsampler;
 int32_t b200_downsampler_create(int32_t device, b200_downsampler** out);
 int32_t b200_downsampler_destroy(b200_downsampler* d);
 /* records x, y, z[, intensity] at stride_bytes; out_xyzi 4 floats per voxel in ascending leaf-index order, out_count
- * points per voxel (either may be NULL), *n_out = number of voxels */
+ * points per voxel (either may be NULL; at most max_out are written), *n_out = number of voxels.  min_points < 0 is
+ * B200_ERR_ARG; a grid of more than 9e18 leaves is B200_ERR_RANGE.  The cloud replaces a scan staged by
+ * b200_scan_undistort: b200_voxel_downsample_staged then returns B200_ERR_ARG until the next undistort. */
 int32_t b200_voxel_downsample(b200_downsampler* d, const float* xyzi, int64_t n, int64_t stride_bytes, float leaf, int32_t min_points,
                               float* out_xyzi, int32_t* out_count, int64_t max_out, int64_t* n_out);
 /* ImuProcess::UndistortPcl, backward half (jueying_lio/include/imu_processing.hpp:175-177,247-284): time-sorts the raw
@@ -353,7 +355,8 @@ int32_t b200_mapbuild_add_keyframe_device(b200_mapbuild* h, const void* d_xyzi_f
 int32_t b200_mapbuild_add_keyframes_device(b200_mapbuild* h, const void* const* d_xyzi_float4, const int64_t* n, const double* poses7,
                                            int64_t count);
 int64_t b200_mapbuild_num_voxels(b200_mapbuild* h);
-/* collective: afterwards every voxel lives on exactly one rank with the sums of all ranks */
+/* collective: afterwards every voxel lives on exactly one rank with the sums of all ranks.  With comm NULL or one rank
+ * nothing is exchanged; the call still waits for the queued keyframes and returns the builder's error, like num_voxels */
 int32_t b200_mapbuild_merge(b200_comm* comm, b200_mapbuild* h);
 /* centroids held by this rank, ascending (z, y, x) voxel order; returns the voxel count */
 int64_t b200_mapbuild_extract(b200_mapbuild* h, float* out_xyzi, int32_t* out_count, int64_t max_out);

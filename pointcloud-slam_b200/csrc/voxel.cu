@@ -161,11 +161,13 @@ __device__ inline void und_step(const ImuPose& head, const ImuPose& tail, const 
     p[0] = (float)e[0]; p[1] = (float)e[1]; p[2] = (float)e[2];
 }
 
-// raw records -> (time key, index); time as an order-preserving uint so that a stable radix sort = ascending time
+// raw records -> (time key, index); time as an order-preserving uint so that a stable radix sort = ascending time.
+// -0.0 is keyed as +0.0: the two compare equal, so they tie and keep their input order like any other tie.
 __global__ void k_und_keys(const float* __restrict__ raw, int n, int stride_f, int time_index, uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    const uint32_t u = __float_as_uint(raw[(size_t)i * stride_f + time_index]);
+    uint32_t u = __float_as_uint(raw[(size_t)i * stride_f + time_index]);
+    if (u == 0x80000000u) u = 0u;
     keys[i] = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
     vals[i] = i;
 }
@@ -607,15 +609,20 @@ static int32_t downsample_run(b200_downsampler* d, int64_t n, float leaf, int32_
     if (!(mn[0] <= mx[0])) return B200_OK;  // no finite point: empty output
     Grid g;
     g.inv_leaf = 1.0f / leaf;
+    // The product of the extents is taken in integers: the last leaf index is cells - 1 and the sentinel is cells, so a
+    // product rounded in double (above 2^53) can make the max-corner leaf equal the sentinel and drop it.
+    unsigned long long cells = 1;
     for (int k = 0; k < 3; ++k) {
-        g.min_b[k] = (long long)std::floor(mn[k] * g.inv_leaf);
-        g.div_b[k] = (long long)std::floor(mx[k] * g.inv_leaf) - g.min_b[k] + 1;
+        const float lo = std::floor(mn[k] * g.inv_leaf), hi = std::floor(mx[k] * g.inv_leaf);
+        if (!(std::fabs(lo) < 4.0e18f && std::fabs(hi) < 4.0e18f)) B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
+        g.min_b[k] = (long long)lo;
+        g.div_b[k] = (long long)hi - g.min_b[k] + 1;
+        if (__builtin_mul_overflow(cells, (unsigned long long)g.div_b[k], &cells) || cells > 9000000000000000000ull)
+            B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
     }
-    const double cells = (double)g.div_b[0] * (double)g.div_b[1] * (double)g.div_b[2];
-    if (cells > 9.0e18) B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
-    const unsigned long long sentinel = (unsigned long long)cells;
+    const unsigned long long sentinel = cells;
     int end_bit = 1;
-    while (end_bit < 64 && (double)(1ull << end_bit) <= cells) ++end_bit;
+    while (end_bit < 64 && (1ull << end_bit) <= cells) ++end_bit;
     CUDA_TRY(d->k_in.reserve(n)); CUDA_TRY(d->k_out.reserve(n)); CUDA_TRY(d->k_uniq.reserve(n));
     CUDA_TRY(d->v_in.reserve(n)); CUDA_TRY(d->v_out.reserve(n)); CUDA_TRY(d->run_cnt.reserve(n)); CUDA_TRY(d->run_off.reserve(n));
     CUDA_TRY(d->d_out.reserve(n)); CUDA_TRY(d->d_cmp.reserve(n)); CUDA_TRY(d->d_cnt.reserve(n)); CUDA_TRY(d->d_cnt_cmp.reserve(n));
@@ -697,8 +704,9 @@ int32_t b200_downsampler_destroy(b200_downsampler* d) {
  * ascending leaf-index order, out_count: points per voxel (either may be NULL); *n_out = number of voxels. */
 int32_t b200_voxel_downsample(b200_downsampler* d, const float* xyzi, int64_t n, int64_t stride, float leaf, int32_t min_points, float* out_xyzi,
                               int32_t* out_count, int64_t max_out, int64_t* n_out) {
-    if (!d || !xyzi || n < 1 || stride < 12 || !(leaf > 0.f) || n > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (!d || !xyzi || n < 1 || stride < 12 || !(leaf > 0.f) || min_points < 0 || n > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_ARG, "bad argument");
     CUDA_SET_DEVICE(d->device);
+    d->n_staged = 0;  // d_in is about to hold this cloud: an undistorted scan staged there is gone
     CUDA_TRY(d->h_stage.reserve(n));
     CUDA_TRY(d->d_in.reserve(n));
     const char* src = (const char*)xyzi;
@@ -758,9 +766,11 @@ int32_t b200_scan_undistort(b200_downsampler* d, const float* points, int64_t n,
     d->n_staged = n;
     return B200_OK;
 }
-/* pcl::VoxelGrid::filter on the points staged by b200_scan_undistort (no host round trip in between) */
+/* pcl::VoxelGrid::filter on the points staged by b200_scan_undistort (no host round trip in between); a host-side
+ * b200_voxel_downsample since then has overwritten them, and this returns B200_ERR_ARG */
 int32_t b200_voxel_downsample_staged(b200_downsampler* d, float leaf, int32_t min_points, int64_t* n_out) {
-    if (!d || d->n_staged < 1 || !(leaf > 0.f)) B200_FAIL(B200_ERR_ARG, "nothing staged");
+    if (!d || !(leaf > 0.f) || min_points < 0) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (d->n_staged < 1) B200_FAIL(B200_ERR_ARG, "nothing staged");
     CUDA_SET_DEVICE(d->device);
     int32_t rc = downsample_run(d, d->n_staged, leaf, min_points);
     if (rc) return rc;
@@ -842,7 +852,10 @@ int64_t b200_mapbuild_num_voxels(b200_mapbuild* h) {
  * (owner = hash(key) mod nranks) with the sums of all ranks.  Collective; no-op for a single rank. */
 int32_t b200_mapbuild_merge(b200_comm* comm, b200_mapbuild* h) {
     if (!h) B200_FAIL(B200_ERR_ARG, "null handle");
-    if (!comm || comm->nranks < 2) return B200_OK;
+    if (!comm || comm->nranks < 2) {  // nothing to exchange; report the builder's errors like a multi-rank merge does
+        CUDA_SET_DEVICE(h->b.device);
+        return h->b.check();
+    }
     using namespace vox;
     Builder& b = h->b;
     CUDA_SET_DEVICE(b.device);
