@@ -83,9 +83,9 @@ struct DevBuf {  // grow-only device buffer
         return cudaSuccess;
     }
     // grow but keep the first `keep` elements
-    cudaError_t reserve_keep(size_t n, size_t keep, cudaStream_t s) {
+    cudaError_t reserve_keep(size_t n, size_t keep, cudaStream_t s, bool exact = false) {
         if (n <= cap) return cudaSuccess;
-        size_t ncap = n + n / 2 + 64;
+        size_t ncap = exact ? n : n + n / 2 + 64;
         T* q = nullptr;
         cudaError_t e = cudaMalloc(&q, ncap * sizeof(T));
         if (e != cudaSuccess) return e;
