@@ -216,6 +216,27 @@ __global__ void k_ndt_finalize(const uint32_t* __restrict__ uniq, const int32_t*
     atomicAdd(n_valid, 1);
 }
 
+// One thread per leaf: the score store (ndt.cuh) from leafD, indexed by the same leaf slot so cell2leaf and nbr7 address
+// it unchanged.  The off-diagonal pairs are stored summed: xt' C xt = xt' ((C + C') / 2) xt.  Leaves without a valid
+// Gaussian are never referenced by cell2leaf / nbr7 and get zeros.
+__global__ void k_ndt_score_store(const LeafD* __restrict__ leafD, const uint8_t* __restrict__ valid, int nruns, Dbl4* __restrict__ sA,
+                                  Dbl4* __restrict__ sB, double* __restrict__ sC) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r >= nruns) return;
+    Dbl4 a = {0.0, 0.0, 0.0, 0.0}, b = {0.0, 0.0, 0.0, 0.0};
+    double c = 0.0;
+    if (valid[r]) {
+        const LeafD L = leafD[r];
+        const double* C = L.icov;
+        a = {L.mean[0], L.mean[1], L.mean[2], C[0]};
+        b = {C[1] + C[3], C[2] + C[6], C[4], C[5] + C[7]};
+        c = C[8];
+    }
+    sA[r] = a;
+    sB[r] = b;
+    sC[r] = c;
+}
+
 // DIRECT7 neighbourhood table: one 32-byte record per grid cell = the leaf slots of the cell and its six face neighbours
 // in the reference's order (vgc_impl:423-430), -1 where the neighbour is outside the grid or holds no usable leaf, and the
 // number of leaves in [7].  A point whose own cell lies inside the grid then resolves its whole neighbourhood with ONE
@@ -242,7 +263,7 @@ __global__ void k_ndt_build_nbr7(const int32_t* __restrict__ cell2leaf, int64_t 
 }
 
 // ------------------------------------------------------------------ source ordering
-// The derivative and score kernels read, per source point, up to 7 cells of the dense table and a 64/96-byte leaf record
+// The derivative and score kernels read, per source point, up to 7 cells of the dense table and 64, 72 or 96 leaf bytes
 // for every hit.  In scan order (a Livox rosette) the 32 lanes of a warp touch 32 unrelated voxels and every load
 // instruction costs 32 L1 wavefronts (ncu: l1tex at 94 % of peak in k_ndt_score_batch).  Sorting the source once by the
 // Morton code of its voxel (in the sensor frame - a rigid transform keeps neighbours together) makes neighbouring
@@ -1089,16 +1110,17 @@ __global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_batch(View v, const
         // score_inc / neighborhood.size() (:876): the size is inverted once per point (<= 1 ulp per term, far inside the
         // 1e-12 score tolerance) - the fp64 division was 13 % of this kernel's instructions
         const double rcnt = cnt > 0 ? 1.0 / (double)cnt : 0.0;
+        // the quadratic form from the symmetric score store (ndt.cuh): 72 instead of 96 leaf bytes and 9 instead of 20
+        // fp64 operations per pair; it differs from the reference's xt' C xt by rounding only (~1e-14 relative per term)
 #pragma unroll
         for (int s = 0; s < NST; ++s) {
             if (lf[s] < 0) continue;
-            LeafD L;
-            load_leafD_256(v.leafD + lf[s], L);
-            const double xt[3] = {(double)tx - L.mean[0], (double)ty - L.mean[1], (double)tz - L.mean[2]};
-            double cx[3];
-#pragma unroll
-            for (int kk = 0; kk < 3; ++kk) cx[kk] = L.icov[kk * 3] * xt[0] + L.icov[kk * 3 + 1] * xt[1] + L.icov[kk * 3 + 2] * xt[2];
-            const double e = exp(-v.d2 * (xt[0] * cx[0] + xt[1] * cx[1] + xt[2] * cx[2]) / 2);
+            const Dbl4 a = load_dbl4_256(v.sA + lf[s]);   // mean, c00
+            const Dbl4 b = load_dbl4_256(v.sB + lf[s]);   // s01, s02, c11, s12
+            const double c22 = __ldg(v.sC + lf[s]);
+            const double x0 = (double)tx - a.x, x1 = (double)ty - a.y, x2 = (double)tz - a.z;
+            const double q = fma(x0, fma(b.y, x2, fma(b.x, x1, a.w * x0)), fma(x1, fma(b.w, x2, b.z * x1), x2 * (c22 * x2)));
+            const double e = exp(-v.d2 * q / 2);
             const double inc = -v.d1 * e - v.d3;
             acc += inc * rcnt;
         }
@@ -1347,6 +1369,8 @@ struct Ndt {
     DevBuf<int32_t> d_cell2leaf, d_nbr7;
     DevBuf<LeafF> d_leafF;
     DevBuf<LeafD> d_leafD;
+    DevBuf<Dbl4> d_sA, d_sB;   // score store (k_ndt_score_store)
+    DevBuf<double> d_sC;
     DevBuf<double> d_cov, d_sums;
     DevBuf<float> d_centroid;
     DevBuf<int32_t> d_npts, d_vals_in, d_vals_out, d_run_cnt, d_run_off, d_small;
@@ -1422,7 +1446,7 @@ void Ndt::destroy() {
     cudaSetDevice(device);
     if (stream) cudaStreamSynchronize(stream);
     d_tgt.release(); d_src.release(); d_src_raw.release(); d_tgt_sorted.release(); s_keys_in.release(); s_keys_out.release();
-    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_cov.release(); d_sums.release(); d_centroid.release();
+    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_sA.release(); d_sB.release(); d_sC.release(); d_cov.release(); d_sums.release(); d_centroid.release();
     d_npts.release(); d_vals_in.release(); d_vals_out.release(); d_run_cnt.release(); d_run_off.release(); d_small.release();
     d_keys_in.release(); d_keys_out.release(); d_uniq.release(); d_valid.release(); cub_tmp.release();
     h_stage.release(); h_small.release(); d_ctl.release(); d_partials.release(); d_p_in.release(); d_scores.release(); d_poses.release();
@@ -1454,6 +1478,7 @@ View Ndt::view() const {
     View v;
     v.src = d_src.p; v.n_src = n_src;
     v.cell2leaf = d_cell2leaf.p; v.leafF = d_leafF.p; v.leafD = d_leafD.p;
+    v.sA = d_sA.p; v.sB = d_sB.p; v.sC = d_sC.p;
     v.nbr7 = have_nbr7 ? d_nbr7.p : nullptr;
     for (int k = 0; k < 3; ++k) { v.min_b[k] = gd.min_b[k]; v.max_b[k] = gd.max_b[k]; v.mul[k] = gd.mul[k]; }
     v.leaf = prm.resolution;
@@ -1601,6 +1626,7 @@ int32_t Ndt::build_target(int64_t n) {
     CUDA_TRY(d_sums.reserve((size_t)nruns * 9));
     CUDA_TRY(d_centroid.reserve((size_t)nruns * 3 + 4));
     CUDA_TRY(d_leafF.reserve(nruns)); CUDA_TRY(d_leafD.reserve(nruns)); CUDA_TRY(d_cov.reserve((size_t)nruns * 9));
+    CUDA_TRY(d_sA.reserve(nruns)); CUDA_TRY(d_sB.reserve(nruns)); CUDA_TRY(d_sC.reserve(nruns));
     CUDA_TRY(d_npts.reserve(nruns)); CUDA_TRY(d_valid.reserve(nruns));
     int32_t* d_nvalid = d_small.p + 9;
     CUDA_TRY(cudaMemsetAsync(d_nvalid, 0, sizeof(int32_t), stream));
@@ -1609,7 +1635,8 @@ int32_t Ndt::build_target(int64_t n) {
     k_ndt_accumulate<<<std::max(acc_blocks, 1), 256, 0, stream>>>(d_tgt.p, d_vals_out.p, d_uniq.p, d_run_off.p, d_run_cnt.p, d_nruns, sentinel, d_sums.p, d_centroid.p);
     k_ndt_finalize<<<(nruns + 127) / 128, 128, 0, stream>>>(d_uniq.p, d_run_cnt.p, d_nruns, sentinel, d_sums.p, prm.min_pts, prm.eig_ratio, d_leafF.p,
                                                             d_leafD.p, d_cov.p, d_npts.p, d_valid.p, d_cell2leaf.p, d_nvalid);
-    LAUNCH_COUNT(5);
+    k_ndt_score_store<<<(nruns + 127) / 128, 128, 0, stream>>>(d_leafD.p, d_valid.p, nruns, d_sA.p, d_sB.p, d_sC.p);
+    LAUNCH_COUNT(6);
     have_nbr7 = prm.search == 7 && ncells <= ((int64_t)1 << 26);  // 32 B per cell: at most 2 GB
     if (have_nbr7) {
         CUDA_TRY(d_nbr7.reserve((size_t)ncells * 8));

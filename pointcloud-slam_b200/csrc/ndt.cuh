@@ -13,7 +13,11 @@
 //                                        leaf id = (ijk - min_b) . divb_mul indexes it directly): leaf slot or -1.
 //                                        One 4-byte load resolves a neighbourhood probe; 10M-pt / 1 m maps need a few MB.
 //   leafF[L]  64 B   {double mean[3]; float icov[9]; pad}   what the float derivative path reads (4 x 16-byte loads)
-//   leafD[L]  96 B   {double mean[3]; double icov[9]}        what computeHessian / calculateScore read (6 x 16-byte loads)
+//   leafD[L]  96 B   {double mean[3]; double icov[9]}        what computeHessian reads (6 x 16-byte loads)
+//   score store, 72 B per leaf in three arrays (what calculateScore reads: two 32-byte loads and one 8-byte load)
+//     sA[L]   32 B   {mean_x, mean_y, mean_z, icov00}
+//     sB[L]   32 B   {icov01 + icov10, icov02 + icov20, icov11, icov12 + icov21}
+//     sC[L]    8 B   icov22
 //   cov[L] 72 B, npts[L], ids[L], valid[L]                   only read back by b200_ndt_leaves
 // The TU is compiled with -fmad=false: every fp32/fp64 operation below is individually rounded, in the
 // evaluation order of the reference C++ (Eigen fixed-size products accumulate k = 0..3 left to right).
@@ -34,16 +38,19 @@ struct __align__(16) LeafD {
     double icov[9];
 };
 static_assert(sizeof(LeafF) == 64 && sizeof(LeafD) == 96, "leaf records are read with 16-byte loads");
-// One fp64 leaf record with three 256-bit loads (sm_100: ld.global.nc.v4.f64 -> LDG.E.256).  Records are 96 B apart in a
-// cudaMalloc'ed array, so every 32-byte piece is naturally aligned and never straddles a 128-byte line: half the load
-// instructions of the 16-byte version, and the L1 wavefronts of a warp request go with the instruction count.
-__device__ __forceinline__ void load_leafD_256(const LeafD* p, LeafD& L) {
-    double* d = reinterpret_cast<double*>(&L);
-#pragma unroll
-    for (int q = 0; q < 3; ++q)
-        asm volatile("ld.global.nc.v4.f64 {%0, %1, %2, %3}, [%4];"
-                     : "=d"(d[4 * q]), "=d"(d[4 * q + 1]), "=d"(d[4 * q + 2]), "=d"(d[4 * q + 3])
-                     : "l"(reinterpret_cast<const char*>(p) + 32 * q));
+
+// Score store of one leaf (built by k_ndt_score_store).  Split into arrays so that the same 32-byte piece of four
+// consecutive leaves shares a 128-byte line: a warp's load of neighbouring leaves touches fewer lines than the 96-byte
+// records, whose pieces of neighbouring leaves almost never share one.
+struct __align__(32) Dbl4 {
+    double x, y, z, w;
+};
+// One 256-bit load (sm_100: ld.global.nc.v4.f64 -> LDG.E.256): the L1 wavefronts of a warp request go with the number of
+// load instructions and the distinct lines they touch.  Dbl4 arrays are cudaMalloc'ed, so no piece straddles a line.
+__device__ __forceinline__ Dbl4 load_dbl4_256(const Dbl4* p) {
+    Dbl4 r;
+    asm volatile("ld.global.nc.v4.f64 {%0, %1, %2, %3}, [%4];" : "=d"(r.x), "=d"(r.y), "=d"(r.z), "=d"(r.w) : "l"(p));
+    return r;
 }
 
 struct AngleTables {   // computeAngleDerivatives: j_ang_a_..h_ / h_ang_a2_..f3_ (double) and j_ang / h_ang (float)
@@ -63,6 +70,9 @@ struct View {
     const int* nbr7;   // [cells][8]: leaf slot (or -1) of the DIRECT7 neighbourhood cells of every grid cell, [7] = how many exist
     const LeafF* leafF;
     const LeafD* leafD;
+    const Dbl4* sA;    // score store (see the layout above); set_target builds it, the batched pairs target does not
+    const Dbl4* sB;
+    const double* sC;
     int min_b[3], max_b[3], mul[3];
     float leaf;
     int nst;   // 1, 7, 27
