@@ -7,7 +7,9 @@
 // set_target  min/max reduction -> leaf id per point -> radix sort (point order preserved inside a leaf) ->
 //             run-length segments -> one warp per leaf accumulates sum(p), sum(p p^T) in fp64 *in input order*
 //             (9 lanes own the 9 sums, points are fetched 32 at a time) -> one thread per leaf: mean, covariance,
-//             3x3 eigen-decomposition, eigenvalue inflation, inverse -> dense cell -> leaf table.
+//             3x3 eigen-decomposition, eigenvalue inflation, inverse -> dense cell -> leaf table.  The build is
+//             segmented: set_target is one segment, a chunk of loop-closure pairs builds all its targets in the same
+//             launches (Ndt::target_minmax, Ndt::build_leaves), and both share one fitness index, search and reduction.
 // align       k_ndt_eval is launched back to back; every launch evaluates score/gradient/Hessian (or the fp64
 //             Hessian) at the pose the control block asks for, and the last block to finish reduces the block
 //             partials in a fixed order and advances the Newton / More-Thuente state machine (computeTransformation
@@ -89,12 +91,18 @@ __device__ __forceinline__ void minmax_range(const float4* __restrict__ pts, int
         }
     }
 }
-__global__ void k_ndt_minmax(const float4* __restrict__ pts, int64_t n, int* __restrict__ mm) {
-    minmax_range(pts, n, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, mm);
+
+// A build covers one or more clouds (segments) that lie end to end: off[j] .. off[j+1]-1 are segment j's points, grid row
+// y = segment y.  The dense cell tables of the segments lie end to end as well: segment j's leaf id l becomes the key
+// cell_base + l, so ONE stable sort, run-length encoding and scan serve every segment.  set_target is the one-segment case
+// (cell_base 0: the keys are the leaf ids); the loop-closure pairs build all targets of a chunk at once.
+__global__ void k_ndt_minmax_init(int* mm, int np) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 6 * np) mm[i] = (i % 6) < 3 ? 0x7fffffff : (int)0x80000000;
 }
-__global__ void k_ndt_minmax_init(int* mm) {
-    if (threadIdx.x < 3) mm[threadIdx.x] = 0x7fffffff;
-    else if (threadIdx.x < 6) mm[threadIdx.x] = (int)0x80000000;
+__global__ void k_ndt_minmax(const float4* __restrict__ pts, const int64_t* __restrict__ off, int* __restrict__ mm) {
+    const int64_t b = off[blockIdx.y];
+    minmax_range(pts + b, off[blockIdx.y + 1] - b, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, mm + 6 * blockIdx.y);
 }
 
 struct GridDims {
@@ -113,12 +121,27 @@ __device__ __forceinline__ uint32_t leaf_key(const float4 p, const GridDims& gd,
     }
     return key;
 }
-__global__ void k_ndt_keys(const float4* __restrict__ pts, int n, GridDims gd, uint32_t sentinel, uint32_t* __restrict__ keys,
-                           int32_t* __restrict__ vals) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    keys[i] = leaf_key(__ldg(pts + i), gd, sentinel);
-    vals[i] = i;
+struct PairGrid {
+    GridDims gd;
+    uint32_t cell_base;
+    int live;  // 0: the segment is not built (its target failed); its points take the sentinel key
+};
+__global__ void k_ndt_keys(const float4* __restrict__ pts, const int64_t* __restrict__ off, const PairGrid* __restrict__ pg, uint32_t sentinel,
+                           uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
+    const int64_t b = off[blockIdx.y], n = off[blockIdx.y + 1] - b;
+    const PairGrid g = pg[blockIdx.y];
+    // a set_target launch covers the cloud with one point per thread: an unrolled loop's 64-bit trip-count division would
+    // cost more than the loop body
+#pragma unroll 1
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        uint32_t key = sentinel;
+        if (g.live) {
+            const uint32_t l = leaf_key(__ldg(pts + b + i), g.gd, 0xFFFFFFFFu);
+            if (l != 0xFFFFFFFFu) key = g.cell_base + l;
+        }
+        keys[b + i] = key;
+        vals[b + i] = (int32_t)(b + i);
+    }
 }
 
 // One warp per leaf: fp64 sums of p and p p^T in input order (:233-237).  Lane c < 3 owns sum(p_c); lanes 3..8 own
@@ -341,36 +364,6 @@ __global__ void k_ndt_source_keys_yaw(const float4* __restrict__ pts, int n, flo
 }
 
 // ------------------------------------------------------------------ independent (source, target) pairs
-// The clouds of a chunk of pairs lie end to end; off[j] .. off[j+1]-1 are pair j's points, grid row y = pair y.  The dense
-// cell tables of the targets are laid out end to end as well: pair j's leaf id l becomes the key cell_base + l, so ONE
-// stable sort, run-length encoding and scan serve every target, and k_ndt_accumulate / k_ndt_finalize run unchanged.
-struct PairGrid {
-    GridDims gd;
-    uint32_t cell_base;
-    int live;  // 0: the pair is not built (its target failed); its points take the sentinel key
-};
-__global__ void k_ndt_minmax_init_pairs(int* mm, int np) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < 6 * np) mm[i] = (i % 6) < 3 ? 0x7fffffff : (int)0x80000000;
-}
-__global__ void k_ndt_minmax_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, int* __restrict__ mm) {
-    const int64_t b = off[blockIdx.y];
-    minmax_range(pts + b, off[blockIdx.y + 1] - b, (int64_t)blockIdx.x * blockDim.x + threadIdx.x, (int64_t)gridDim.x * blockDim.x, mm + 6 * blockIdx.y);
-}
-__global__ void k_ndt_keys_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, const PairGrid* __restrict__ pg, uint32_t sentinel,
-                                 uint32_t* __restrict__ keys, int32_t* __restrict__ vals) {
-    const int64_t b = off[blockIdx.y], n = off[blockIdx.y + 1] - b;
-    const PairGrid g = pg[blockIdx.y];
-    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
-        uint32_t key = sentinel;
-        if (g.live) {
-            const uint32_t l = leaf_key(__ldg(pts + b + i), g.gd, 0xFFFFFFFFu);
-            if (l != 0xFFFFFFFFu) key = g.cell_base + l;
-        }
-        keys[b + i] = key;
-        vals[b + i] = (int32_t)(b + i);
-    }
-}
 // sources: key = (pair, Morton key of the voxel), so that one stable sort orders every pair's points as set_source does
 __global__ void k_ndt_source_keys_pairs(const float4* __restrict__ pts, const int64_t* __restrict__ off, float inv_cell, uint64_t* __restrict__ keys,
                                         int32_t* __restrict__ vals) {
@@ -1143,20 +1136,8 @@ __global__ void k_ndt_score_finish(const double* __restrict__ partial, int nchun
     scores[a] = s / (double)n_src;
 }
 
-// number of (point, voxel) pairs and probes of one evaluation at the poses' transforms (roofline bookkeeping)
-__global__ void k_ndt_nbhd_total(View v, const float* __restrict__ M16_rowmajor, unsigned long long* out) {
-    unsigned long long cnt = 0;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < v.n_src; i += gridDim.x * blockDim.x) {
-        const float4 p = __ldg(v.src + i);
-        float tx, ty, tz;
-        xform(M16_rowmajor, p.x, p.y, p.z, tx, ty, tz);
-        for (int s = 0; s < v.nst; ++s) cnt += nbr_leaf(v, tx, ty, tz, s) >= 0 ? 1 : 0;
-    }
-    for (int o = 16; o > 0; o >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, o);
-    if ((threadIdx.x & 31) == 0 && cnt) atomicAdd(out, cnt);
-}
-
-// same count for a batch of poses (col-major 4x4 each): grid = (point chunks, hypotheses)
+// number of occupied (point, voxel) pairs of one evaluation, summed over a batch of poses (col-major 4x4 each; roofline
+// bookkeeping): grid = (point chunks, hypotheses)
 __global__ void k_ndt_pairs_batch(View v, const float* __restrict__ poses, unsigned long long* out) {
     __shared__ float M[12];
     const int h = blockIdx.y;
@@ -1271,47 +1252,39 @@ __device__ __forceinline__ float fitness_nn(const FitView& f, float x, float y, 
     return best;
 }
 
-__global__ void __launch_bounds__(256) k_ndt_fitness(FitView f, const float4* __restrict__ src, int n, const float* __restrict__ M12g, double* __restrict__ d2_out) {
-    __shared__ float M[12];
-    if (threadIdx.x < 12) M[threadIdx.x] = M12g[threadIdx.x];
-    __syncthreads();
-    const int lane = threadIdx.x & 31;
-    const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (q >= n) return;
-    const float4 p = __ldg(src + q);
-    float x, y, z;
-    xform(M, p.x, p.y, p.z, x, y, z);
-    const float best = fitness_nn(f, x, y, z, lane);
-    if (lane == 0) d2_out[q] = (double)best;
-}
-
-// Independent pairs: grid row y = pair y; its source range, its target index and its final transformation, read from its
-// control block on the device (row-major; the first 12 floats are the 3x4 the source is moved by).
-struct PairFit {
+// One row per (source, target): the target's FitView, the source range, where its distances go in d2, and the row-major
+// 3x4 transform the source is moved by (a single call's staged pose, or a pair's final transformation in its control
+// block on the device).  Grid row y = row y.
+struct FitRow {
     FitView f;
     const float4* src;
     int n;
+    int64_t d2_off;
+    const float* T;
 };
-__global__ void __launch_bounds__(256) k_ndt_fitness_pairs(const PairFit* __restrict__ pf, const Ctl* __restrict__ ctls, const int64_t* __restrict__ d2_off,
-                                                           double* __restrict__ d2_out) {
+__global__ void __launch_bounds__(256) k_ndt_fitness(const FitRow* __restrict__ rows, double* __restrict__ d2_out) {
     __shared__ float M[12];
-    if (threadIdx.x < 12) M[threadIdx.x] = ctls[blockIdx.y].final_T[threadIdx.x];
+    const FitRow& R = rows[blockIdx.y];
+    if (threadIdx.x < 12) M[threadIdx.x] = R.T[threadIdx.x];
     __syncthreads();
-    const PairFit& P = pf[blockIdx.y];
     const int lane = threadIdx.x & 31;
     const int q = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (q >= P.n) return;
-    const float4 p = __ldg(P.src + q);
+    if (q >= R.n) return;
+    const float4 p = __ldg(R.src + q);
     float x, y, z;
     xform(M, p.x, p.y, p.z, x, y, z);
-    const float best = fitness_nn(P.f, x, y, z, lane);
-    if (lane == 0) d2_out[d2_off[blockIdx.y] + q] = (double)best;
+    const float best = fitness_nn(R.f, x, y, z, lane);
+    if (lane == 0) d2_out[R.d2_off + q] = (double)best;
 }
 
-// one block, fixed order: deterministic, and the same for a pair as for the single-target path
-__device__ __forceinline__ void fitness_reduce_block(const double* __restrict__ d2, int n, double max_range, double* __restrict__ out /*sum, count*/) {
+// block y = row y: its distances -> out[2y] = sum, out[2y + 1] = count of those within max_range.  One block in a fixed
+// order, so a pair's fitness has the bits of a single call at the same transform.
+__global__ void k_ndt_fitness_reduce(const FitRow* __restrict__ rows, const double* __restrict__ d2_all, double max_range, double* __restrict__ out) {
     __shared__ double ssum[256];
     __shared__ double scnt[256];
+    const FitRow& R = rows[blockIdx.x];
+    const double* d2 = d2_all + R.d2_off;
+    const int n = R.n;
     double s = 0.0, c = 0.0;
     const int per = (n + blockDim.x - 1) / blockDim.x;
     const int b = threadIdx.x * per, e = min(n, b + per);
@@ -1325,17 +1298,9 @@ __device__ __forceinline__ void fitness_reduce_block(const double* __restrict__ 
     if (threadIdx.x == 0) {
         double S = 0.0, C = 0.0;
         for (int i = 0; i < (int)blockDim.x; ++i) { S += ssum[i]; C += scnt[i]; }
-        out[0] = S;
-        out[1] = C;
+        out[2 * blockIdx.x] = S;
+        out[2 * blockIdx.x + 1] = C;
     }
-}
-__global__ void k_ndt_fitness_reduce(const double* __restrict__ d2, int n, double max_range, double* __restrict__ out) {
-    fitness_reduce_block(d2, n, max_range, out);
-}
-// block y = pair y: d2[d2_off[y] .. d2_off[y + 1]) -> out[2y], out[2y + 1]
-__global__ void k_ndt_fitness_reduce_pairs(const double* __restrict__ d2, const int64_t* __restrict__ d2_off, double max_range, double* __restrict__ out) {
-    const int64_t b = d2_off[blockIdx.x], e = d2_off[blockIdx.x + 1];
-    fitness_reduce_block(d2 + b, (int)(e - b), max_range, out + 2 * blockIdx.x);
 }
 
 // ------------------------------------------------------------------ host object
@@ -1364,6 +1329,9 @@ struct Ndt {
     DevBuf<int32_t> y_vals_in, y_vals_out;
     DevBuf<uint8_t> s_tmp;
     DevBuf<double> d_fit;
+    struct FitCall { FitRow row; float T[12]; };  // a single fitness call: its row and the pose it points to
+    DevBuf<FitCall> d_fitcall;
+    PinnedBuf<FitCall> h_fitcall;
     bool have_fitness_index = false;
     int64_t n_tgt = 0;
     DevBuf<int32_t> d_cell2leaf, d_nbr7;
@@ -1376,8 +1344,17 @@ struct Ndt {
     DevBuf<int32_t> d_npts, d_vals_in, d_vals_out, d_run_cnt, d_run_off, d_small;
     DevBuf<uint32_t> d_keys_in, d_keys_out, d_uniq;
     DevBuf<uint8_t> d_valid, cub_tmp;
+    // segments of a target build: offsets into d_tgt (the pairs append their source offsets), min / max, grids
+    DevBuf<int64_t> d_off;
+    PinnedBuf<int64_t> h_off;
+    DevBuf<int32_t> d_mm;
+    PinnedBuf<int32_t> h_mm;
+    DevBuf<PairGrid> d_pg;
+    PinnedBuf<PairGrid> h_pg;
     PinnedBuf<float4> h_stage;
     PinnedBuf<int32_t> h_small;
+    // d_small: scalars the device hands the host (read back through h_small[0]) and the cooperative barrier's generation
+    enum SmallSlot : int { SMALL_NRUNS = 0, SMALL_NVALID, SMALL_LEFT, SMALL_GEN, SMALL_SLOTS };
     int n_src = 0;
     bool have_target = false, have_nbr7 = false;
     // align
@@ -1408,6 +1385,10 @@ struct Ndt {
     int32_t upload(const float* xyz, int64_t n, int64_t stride, DevBuf<float4>& dst);
     int32_t set_target(const float* xyz, int64_t n, int64_t stride);
     int32_t build_target(int64_t n);
+    int32_t target_minmax(int64_t np, unsigned gx);
+    int32_t build_leaves(int64_t np, unsigned gx, int64_t n, int64_t cells);
+    int32_t build_fitness_index(int64_t n, int64_t cells);
+    FitView fit_view(const GridDims& g, uint32_t cell_base) const;
     int32_t set_source(const float* xyz, int64_t n, int64_t stride);
     int32_t run(int h, const float* d_guesses, const double* d_p, int phase);
     template <class Launch>
@@ -1434,8 +1415,8 @@ int32_t Ndt::init(const b200_ndt_params* p, int dev) {
     CUDA_TRY(cudaEventCreate(&ev1));
     CUDA_TRY(cudaEventCreate(&evs0));
     CUDA_TRY(cudaEventCreate(&evs1));
-    CUDA_TRY(d_small.reserve(16));
-    CUDA_TRY(h_small.reserve(16));
+    CUDA_TRY(d_small.reserve(SMALL_SLOTS));
+    CUDA_TRY(h_small.reserve(SMALL_SLOTS));
     CUDA_TRY(d_best.reserve(4));
     CUDA_TRY(h_best.reserve(4));
     gauss();
@@ -1446,9 +1427,10 @@ void Ndt::destroy() {
     cudaSetDevice(device);
     if (stream) cudaStreamSynchronize(stream);
     d_tgt.release(); d_src.release(); d_src_raw.release(); d_tgt_sorted.release(); s_keys_in.release(); s_keys_out.release();
-    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_sA.release(); d_sB.release(); d_sC.release(); d_cov.release(); d_sums.release(); d_centroid.release();
+    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_fitcall.release(); h_fitcall.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_sA.release(); d_sB.release(); d_sC.release(); d_cov.release(); d_sums.release(); d_centroid.release();
     d_npts.release(); d_vals_in.release(); d_vals_out.release(); d_run_cnt.release(); d_run_off.release(); d_small.release();
     d_keys_in.release(); d_keys_out.release(); d_uniq.release(); d_valid.release(); cub_tmp.release();
+    d_off.release(); h_off.release(); d_mm.release(); h_mm.release(); d_pg.release(); h_pg.release();
     h_stage.release(); h_small.release(); d_ctl.release(); d_partials.release(); d_p_in.release(); d_scores.release(); d_poses.release();
     h_ctl.release(); h_scores.release(); h_poses.release(); d_best.release(); d_bar.release(); h_best.release();
     if (ev0) cudaEventDestroy(ev0);
@@ -1589,29 +1571,32 @@ static int32_t grid_from_minmax(const int* mm6, float resolution, GridDims& gd, 
     return B200_OK;
 }
 
-int32_t Ndt::build_target(int64_t n) {
-    have_target = false;
-    have_fitness_index = false;
-    n_tgt = n;
-    CUDA_TRY(cudaEventRecord(ev0, stream));
-    int* mm = d_small.p;
-    k_ndt_minmax_init<<<1, 32, 0, stream>>>(mm);
-    k_ndt_minmax<<<sm_count * 8, 256, 0, stream>>>(d_tgt.p, n, mm);
-    CUDA_TRY(cudaMemcpyAsync(h_small.p, mm, 6 * sizeof(int), cudaMemcpyDeviceToHost, stream));
+// Min / max of the finite points of segments 0 .. np-1 of d_tgt (offsets in d_off) into h_mm[6 np]; gx blocks per segment.
+int32_t Ndt::target_minmax(int64_t np, unsigned gx) {
+    CUDA_TRY(d_mm.reserve(6 * (size_t)np));
+    CUDA_TRY(h_mm.reserve(6 * (size_t)np));
+    k_ndt_minmax_init<<<(unsigned)((6 * np + 255) / 256), 256, 0, stream>>>(d_mm.p, (int)np);
+    k_ndt_minmax<<<dim3(gx, (unsigned)np), 256, 0, stream>>>(d_tgt.p, d_off.p, d_mm.p);
+    LAUNCH_COUNT(2);
+    CUDA_TRY(cudaMemcpyAsync(h_mm.p, d_mm.p, 6 * np * sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
-    const int32_t grc = grid_from_minmax(h_small.p, prm.resolution, gd, ncells);
-    if (grc) return grc;
-    CUDA_TRY(d_cell2leaf.reserve((size_t)ncells));
-    CUDA_TRY(cudaMemsetAsync(d_cell2leaf.p, 0xFF, (size_t)ncells * sizeof(int32_t), stream));
+    return B200_OK;
+}
+
+// The leaves of segments 0 .. np-1 (grids in h_pg, the first n points of d_tgt), whose cell tables fill keys [0, cells):
+// leaf keys (non-finite points and segments that are not live take the sentinel key `cells`, which sorts last; gx blocks per
+// segment) -> one stable radix sort -> run-length encoding + scan -> k_ndt_accumulate -> k_ndt_finalize.  Sets nruns.
+int32_t Ndt::build_leaves(int64_t np, unsigned gx, int64_t n, int64_t cells) {
+    const uint32_t sentinel = (uint32_t)cells;
+    CUDA_TRY(d_pg.reserve((size_t)np));
+    CUDA_TRY(cudaMemcpyAsync(d_pg.p, h_pg.p, np * sizeof(PairGrid), cudaMemcpyHostToDevice, stream));
     CUDA_TRY(d_keys_in.reserve(n)); CUDA_TRY(d_keys_out.reserve(n)); CUDA_TRY(d_uniq.reserve(n));
     CUDA_TRY(d_vals_in.reserve(n)); CUDA_TRY(d_vals_out.reserve(n)); CUDA_TRY(d_run_cnt.reserve(n)); CUDA_TRY(d_run_off.reserve(n));
-    const int nb = (int)((n + 255) / 256);
-    const uint32_t sentinel = (uint32_t)ncells;  // key of non-finite points: one past the last leaf id, sorts last
-    k_ndt_keys<<<nb, 256, 0, stream>>>(d_tgt.p, (int)n, gd, sentinel, d_keys_in.p, d_vals_in.p);
+    k_ndt_keys<<<dim3(gx, (unsigned)np), 256, 0, stream>>>(d_tgt.p, d_off.p, d_pg.p, sentinel, d_keys_in.p, d_vals_in.p);
     int end_bit = 1;
-    while (end_bit < 32 && ((int64_t)1 << end_bit) <= ncells) ++end_bit;
+    while (end_bit < 32 && ((int64_t)1 << end_bit) <= cells) ++end_bit;
     size_t t1 = 0, t2 = 0, t3 = 0;
-    int32_t* d_nruns = d_small.p + 8;
+    int32_t* d_nruns = d_small.p + SMALL_NRUNS;
     cub::DeviceRadixSort::SortPairs(nullptr, t1, d_keys_in.p, d_keys_out.p, d_vals_in.p, d_vals_out.p, (int)n, 0, end_bit, stream);
     cub::DeviceRunLengthEncode::Encode(nullptr, t2, d_keys_out.p, d_uniq.p, d_run_cnt.p, d_nruns, (int)n, stream);
     cub::DeviceScan::ExclusiveSum(nullptr, t3, d_run_cnt.p, d_run_off.p, (int)n, stream);
@@ -1626,17 +1611,58 @@ int32_t Ndt::build_target(int64_t n) {
     CUDA_TRY(d_sums.reserve((size_t)nruns * 9));
     CUDA_TRY(d_centroid.reserve((size_t)nruns * 3 + 4));
     CUDA_TRY(d_leafF.reserve(nruns)); CUDA_TRY(d_leafD.reserve(nruns)); CUDA_TRY(d_cov.reserve((size_t)nruns * 9));
-    CUDA_TRY(d_sA.reserve(nruns)); CUDA_TRY(d_sB.reserve(nruns)); CUDA_TRY(d_sC.reserve(nruns));
     CUDA_TRY(d_npts.reserve(nruns)); CUDA_TRY(d_valid.reserve(nruns));
-    int32_t* d_nvalid = d_small.p + 9;
+    CUDA_TRY(d_cell2leaf.reserve((size_t)cells));
+    CUDA_TRY(cudaMemsetAsync(d_cell2leaf.p, 0xFF, (size_t)cells * sizeof(int32_t), stream));
+    int32_t* d_nvalid = d_small.p + SMALL_NVALID;
     CUDA_TRY(cudaMemsetAsync(d_nvalid, 0, sizeof(int32_t), stream));
     CUDA_TRY(cudaMemsetAsync(d_cov.p, 0, (size_t)nruns * 9 * sizeof(double), stream));
     const int acc_blocks = std::min((nruns + 7) / 8, sm_count * 8);
     k_ndt_accumulate<<<std::max(acc_blocks, 1), 256, 0, stream>>>(d_tgt.p, d_vals_out.p, d_uniq.p, d_run_off.p, d_run_cnt.p, d_nruns, sentinel, d_sums.p, d_centroid.p);
     k_ndt_finalize<<<(nruns + 127) / 128, 128, 0, stream>>>(d_uniq.p, d_run_cnt.p, d_nruns, sentinel, d_sums.p, prm.min_pts, prm.eig_ratio, d_leafF.p,
                                                             d_leafD.p, d_cov.p, d_npts.p, d_valid.p, d_cell2leaf.p, d_nvalid);
+    LAUNCH_COUNT(3);
+    return B200_OK;
+}
+
+// getFitnessScore's index over the last build_leaves: the n target points in cell order and the cell -> run table
+int32_t Ndt::build_fitness_index(int64_t n, int64_t cells) {
+    CUDA_TRY(d_tgt_sorted.reserve((size_t)n));
+    CUDA_TRY(d_cell2run.reserve((size_t)cells));
+    CUDA_TRY(cudaMemsetAsync(d_cell2run.p, 0xFF, (size_t)cells * sizeof(int32_t), stream));
+    k_ndt_gather<<<(unsigned)((n + 255) / 256), 256, 0, stream>>>(d_tgt.p, d_vals_out.p, (int)n, d_tgt_sorted.p);
+    k_ndt_cell_runs<<<(nruns + 255) / 256, 256, 0, stream>>>(d_uniq.p, d_small.p + SMALL_NRUNS, (uint32_t)cells, d_cell2run.p);
+    LAUNCH_COUNT(2);
+    return B200_OK;
+}
+
+FitView Ndt::fit_view(const GridDims& g, uint32_t cell_base) const {
+    FitView f;
+    f.pts = d_tgt_sorted.p; f.cell2run = d_cell2run.p + cell_base; f.run_off = d_run_off.p; f.run_cnt = d_run_cnt.p;
+    for (int k = 0; k < 3; ++k) { f.min_b[k] = g.min_b[k]; f.div_b[k] = g.div_b[k]; }
+    f.leaf = prm.resolution; f.inv_leaf = g.inv_leaf;
+    return f;
+}
+
+int32_t Ndt::build_target(int64_t n) {
+    have_target = false;
+    have_fitness_index = false;
+    n_tgt = n;
+    CUDA_TRY(d_off.reserve(2)); CUDA_TRY(h_off.reserve(2)); CUDA_TRY(h_pg.reserve(1));
+    h_off.p[0] = 0;
+    h_off.p[1] = n;
+    CUDA_TRY(cudaEventRecord(ev0, stream));
+    CUDA_TRY(cudaMemcpyAsync(d_off.p, h_off.p, 2 * sizeof(int64_t), cudaMemcpyHostToDevice, stream));
+    int32_t rc = target_minmax(1, (unsigned)sm_count * 8);
+    if (rc) return rc;
+    rc = grid_from_minmax(h_mm.p, prm.resolution, gd, ncells);
+    if (rc) return rc;
+    h_pg.p[0] = PairGrid{gd, 0, 1};
+    rc = build_leaves(1, (unsigned)((n + 255) / 256), n, ncells);
+    if (rc) return rc;
+    CUDA_TRY(d_sA.reserve(nruns)); CUDA_TRY(d_sB.reserve(nruns)); CUDA_TRY(d_sC.reserve(nruns));
     k_ndt_score_store<<<(nruns + 127) / 128, 128, 0, stream>>>(d_leafD.p, d_valid.p, nruns, d_sA.p, d_sB.p, d_sC.p);
-    LAUNCH_COUNT(6);
+    LAUNCH_COUNT(1);
     have_nbr7 = prm.search == 7 && ncells <= ((int64_t)1 << 26);  // 32 B per cell: at most 2 GB
     if (have_nbr7) {
         CUDA_TRY(d_nbr7.reserve((size_t)ncells * 8));
@@ -1645,7 +1671,7 @@ int32_t Ndt::build_target(int64_t n) {
     }
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaEventRecord(ev1, stream));
-    CUDA_TRY(cudaMemcpyAsync(h_small.p, d_nvalid, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
+    CUDA_TRY(cudaMemcpyAsync(h_small.p, d_small.p + SMALL_NVALID, sizeof(int32_t), cudaMemcpyDeviceToHost, stream));
     CUDA_TRY(cudaStreamSynchronize(stream));
     n_valid = h_small.p[0];
     cudaEventElapsedTime(&last_ms, ev0, ev1);
@@ -1693,7 +1719,7 @@ int32_t Ndt::set_source(const float* xyz, int64_t n, int64_t stride) {
 // polls of the done count.
 template <class Launch>
 int32_t Ndt::until_done(int h, int max_launches, int& launches, Launch launch) {
-    int* d_left = d_small.p + 10;
+    int* d_left = d_small.p + SMALL_LEFT;
     while (launches - 1 < max_launches) {
         // first poll after 12 evaluations: a typical relocalization align (8 iterations, 9-10 evaluations) then ends with one
         // poll and two or three no-op launches instead of two polls and seven no-ops
@@ -1736,7 +1762,7 @@ int32_t Ndt::run(int h, const float* d_guesses, const double* d_p, int phase) {
     const int max_launches = single ? 1 : (prm.max_iter + 3) * 12 + 1;
     static const bool persistent_ok = !(getenv("B200_NDT_LOOP") && atoi(getenv("B200_NDT_LOOP")) == 0);
     if (!single && h == 1 && persistent_ok && coop_launch) {  // one alignment: the whole Newton / line-search loop in one launch
-        unsigned int* d_gen = (unsigned int*)(d_small.p + 11);
+        unsigned int* d_gen = (unsigned int*)(d_small.p + SMALL_GEN);
         CUDA_TRY(cudaMemsetAsync(d_gen, 0, sizeof(unsigned int), stream));
         Ctl* ctls = d_ctl.p;
         double* parts = d_partials.p;
@@ -1845,28 +1871,23 @@ int32_t Ndt::score_batch_device(const float* d_poses16, int64_t h, double* d_out
 int32_t Ndt::fitness(const float* T16, double max_range, double* score, int64_t* nr) {
     if (!have_target) B200_FAIL(B200_ERR_ARG, "no target set");
     if (n_src < 1) B200_FAIL(B200_ERR_ARG, "no source set");
-    if (!have_fitness_index) {  // built on first use: target points in cell order + cell -> run table
-        CUDA_TRY(d_tgt_sorted.reserve((size_t)n_tgt));
-        CUDA_TRY(d_cell2run.reserve((size_t)ncells));
-        CUDA_TRY(cudaMemsetAsync(d_cell2run.p, 0xFF, (size_t)ncells * sizeof(int32_t), stream));
-        k_ndt_gather<<<(unsigned)((n_tgt + 255) / 256), 256, 0, stream>>>(d_tgt.p, d_vals_out.p, (int)n_tgt, d_tgt_sorted.p);
-        k_ndt_cell_runs<<<(nruns + 255) / 256, 256, 0, stream>>>(d_uniq.p, d_small.p + 8, (uint32_t)ncells, d_cell2run.p);
-        LAUNCH_COUNT(2);
+    if (!have_fitness_index) {  // built on first use
+        const int32_t rc = build_fitness_index(n_tgt, ncells);
+        if (rc) return rc;
         have_fitness_index = true;
     }
     CUDA_TRY(d_fit.reserve((size_t)n_src + 2));
-    CUDA_TRY(d_poses.reserve(16)); CUDA_TRY(h_poses.reserve(16)); CUDA_TRY(h_scores.reserve(8));
+    CUDA_TRY(d_fitcall.reserve(1)); CUDA_TRY(h_fitcall.reserve(1)); CUDA_TRY(h_scores.reserve(8));
+    FitCall& fc = *h_fitcall.p;
+    fc.row = FitRow{fit_view(gd, 0), d_src.p, n_src, 0, d_fitcall.p->T};
     for (int i = 0; i < 3; ++i)
-        for (int j = 0; j < 4; ++j) h_poses.p[i * 4 + j] = T16[j * 4 + i];
-    CUDA_TRY(cudaMemcpyAsync(d_poses.p, h_poses.p, 12 * sizeof(float), cudaMemcpyHostToDevice, stream));
-    FitView f;
-    f.pts = d_tgt_sorted.p; f.cell2run = d_cell2run.p; f.run_off = d_run_off.p; f.run_cnt = d_run_cnt.p;
-    for (int k = 0; k < 3; ++k) { f.min_b[k] = gd.min_b[k]; f.div_b[k] = gd.div_b[k]; }
-    f.leaf = prm.resolution; f.inv_leaf = gd.inv_leaf;
+        for (int j = 0; j < 4; ++j) fc.T[i * 4 + j] = T16[j * 4 + i];
+    CUDA_TRY(cudaMemcpyAsync(d_fitcall.p, h_fitcall.p, sizeof(FitCall), cudaMemcpyHostToDevice, stream));
+    const FitRow* row = &d_fitcall.p->row;
     CUDA_TRY(cudaEventRecord(ev0, stream));
     // the fitness is defined on the source in its original order; any order gives the same set of distances
-    k_ndt_fitness<<<(unsigned)(((size_t)n_src * 32 + 255) / 256), 256, 0, stream>>>(f, d_src.p, n_src, d_poses.p, d_fit.p);
-    k_ndt_fitness_reduce<<<1, 256, 0, stream>>>(d_fit.p, n_src, max_range, d_fit.p + n_src);
+    k_ndt_fitness<<<(unsigned)(((size_t)n_src * 32 + 255) / 256), 256, 0, stream>>>(row, d_fit.p);
+    k_ndt_fitness_reduce<<<1, 256, 0, stream>>>(row, d_fit.p, max_range, d_fit.p + n_src);
     LAUNCH_COUNT(2);
     CUDA_TRY(cudaEventRecord(ev1, stream));
     CUDA_TRY(cudaMemcpyAsync(h_scores.p, d_fit.p + n_src, 2 * sizeof(double), cudaMemcpyDeviceToHost, stream));
@@ -1940,16 +1961,10 @@ void pack_ranges(const float* xyz, int64_t stride, const int64_t* off, const int
 struct b200_ndt_pairs {
     Ndt k;  // parameters, stream, events, staging and the target / source / alignment buffers, reused by every chunk
     DevBuf<uint64_t> d_skeys_in, d_skeys_out;
-    DevBuf<int64_t> d_off, d_d2off;
-    PinnedBuf<int64_t> h_off;
-    DevBuf<int32_t> d_mm;
-    PinnedBuf<int32_t> h_mm;
-    DevBuf<ndt::PairGrid> d_pg;
-    PinnedBuf<ndt::PairGrid> h_pg;
     DevBuf<ndt::PairEval> d_pe;
     PinnedBuf<ndt::PairEval> h_pe;
-    DevBuf<ndt::PairFit> d_pf;
-    PinnedBuf<ndt::PairFit> h_pf;
+    DevBuf<ndt::FitRow> d_pf;
+    PinnedBuf<ndt::FitRow> h_pf;
     DevBuf<double> d_fitsum;
     PinnedBuf<double> h_fitsum;
     DevBuf<uint8_t> d_xchg;
@@ -1974,8 +1989,8 @@ struct b200_ndt_pairs {
     void destroy() {
         cudaSetDevice(k.device);
         if (k.stream) cudaStreamSynchronize(k.stream);
-        d_skeys_in.release(); d_skeys_out.release(); d_off.release(); d_d2off.release(); h_off.release(); d_mm.release(); h_mm.release();
-        d_pg.release(); h_pg.release(); d_pe.release(); h_pe.release(); d_pf.release(); h_pf.release(); d_fitsum.release(); h_fitsum.release();
+        d_skeys_in.release(); d_skeys_out.release();
+        d_pe.release(); h_pe.release(); d_pf.release(); h_pf.release(); d_fitsum.release(); h_fitsum.release();
         d_xchg.release(); h_xchg.release();
         k.destroy();
     }
@@ -2005,31 +2020,24 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     CUDA_TRY(K.d_src_raw.reserve((size_t)ns));
     CUDA_TRY(cudaMemcpyAsync(K.d_tgt.p, K.h_stage.p, (size_t)nt * sizeof(float4), cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(K.d_src_raw.p, K.h_stage.p + nt, (size_t)ns * sizeof(float4), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(h_off.reserve(2 * (size_t)(np + 1)));
-    CUDA_TRY(d_off.reserve(2 * (size_t)(np + 1)));
-    memcpy(h_off.p, toff.data(), (np + 1) * sizeof(int64_t));
-    memcpy(h_off.p + np + 1, soff.data(), (np + 1) * sizeof(int64_t));
-    CUDA_TRY(cudaMemcpyAsync(d_off.p, h_off.p, 2 * (np + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    const int64_t* d_toff = d_off.p;
-    const int64_t* d_soff = d_off.p + np + 1;
+    CUDA_TRY(K.h_off.reserve(2 * (size_t)(np + 1)));
+    CUDA_TRY(K.d_off.reserve(2 * (size_t)(np + 1)));
+    memcpy(K.h_off.p, toff.data(), (np + 1) * sizeof(int64_t));
+    memcpy(K.h_off.p + np + 1, soff.data(), (np + 1) * sizeof(int64_t));
+    CUDA_TRY(cudaMemcpyAsync(K.d_off.p, K.h_off.p, 2 * (np + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
+    const int64_t* d_soff = K.d_off.p + np + 1;
     // per-target min / max, read back once for the whole chunk
-    CUDA_TRY(d_mm.reserve(6 * (size_t)np));
-    CUDA_TRY(h_mm.reserve(6 * (size_t)np));
-    k_ndt_minmax_init_pairs<<<(unsigned)((6 * np + 255) / 256), 256, 0, s>>>(d_mm.p, (int)np);
-    k_ndt_minmax_pairs<<<dim3((unsigned)std::min<int64_t>((max_tn + 1023) / 1024, 256), (unsigned)np), 256, 0, s>>>(K.d_tgt.p, d_toff, d_mm.p);
-    CUDA_TRY(cudaMemcpyAsync(h_mm.p, d_mm.p, 6 * np * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    LAUNCH_COUNT(2);
+    int32_t rc = K.target_minmax(np, (unsigned)std::min<int64_t>((max_tn + 1023) / 1024, 256));
+    if (rc) return rc;
     // every target's grid, as Ndt::build_target derives it; the dense tables end to end
-    CUDA_TRY(h_pg.reserve((size_t)np));
-    CUDA_TRY(d_pg.reserve((size_t)np));
+    CUDA_TRY(K.h_pg.reserve((size_t)np));
     int64_t cells = 0, n_live = 0;
     used = np;
     for (int64_t j = 0; j < np; ++j) {
-        PairGrid& g = h_pg.p[j];
+        PairGrid& g = K.h_pg.p[j];
         memset(&g, 0, sizeof g);
         int64_t nc = 0;
-        const int32_t st = grid_from_minmax(h_mm.p + 6 * j, K.prm.resolution, g.gd, nc);
+        const int32_t st = grid_from_minmax(K.h_mm.p + 6 * j, K.prm.resolution, g.gd, nc);
         if (st) {
             memset(&g, 0, sizeof g);
             c.results[ids[j]].status = st;
@@ -2047,7 +2055,7 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     last_ncells.resize(np);
     last_live.resize(np);
     for (int64_t j = 0; j < np; ++j) {
-        const PairGrid& g = h_pg.p[j];
+        const PairGrid& g = K.h_pg.p[j];
         last_base[j] = g.cell_base;
         last_ncells[j] = g.live ? (int64_t)g.gd.div_b[0] * g.gd.div_b[1] * g.gd.div_b[2] : 0;
         last_live[j] = g.live;
@@ -2055,49 +2063,11 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     last_nruns = 0;
     if (!n_live) return B200_OK;
     const int64_t nt_u = toff[np], ns_u = soff[np];
-    CUDA_TRY(cudaMemcpyAsync(d_pg.p, h_pg.p, np * sizeof(PairGrid), cudaMemcpyHostToDevice, s));
-    // segmented target build: one stable sort of (cell_base + leaf id) over every target, then the single-target kernels
-    const uint32_t sentinel = (uint32_t)cells;
-    CUDA_TRY(K.d_keys_in.reserve(nt_u)); CUDA_TRY(K.d_keys_out.reserve(nt_u)); CUDA_TRY(K.d_uniq.reserve(nt_u));
-    CUDA_TRY(K.d_vals_in.reserve(nt_u)); CUDA_TRY(K.d_vals_out.reserve(nt_u)); CUDA_TRY(K.d_run_cnt.reserve(nt_u)); CUDA_TRY(K.d_run_off.reserve(nt_u));
-    k_ndt_keys_pairs<<<dim3((unsigned)std::min<int64_t>((max_tn + 255) / 256, 1024), (unsigned)np), 256, 0, s>>>(K.d_tgt.p, d_toff, d_pg.p, sentinel,
-                                                                                                           K.d_keys_in.p, K.d_vals_in.p);
-    int end_bit = 1;
-    while (end_bit < 32 && ((int64_t)1 << end_bit) <= cells) ++end_bit;
-    int32_t* d_nruns = K.d_small.p + 8;
-    size_t t1 = 0, t2 = 0, t3 = 0;
-    cub::DeviceRadixSort::SortPairs(nullptr, t1, K.d_keys_in.p, K.d_keys_out.p, K.d_vals_in.p, K.d_vals_out.p, (int)nt_u, 0, end_bit, s);
-    cub::DeviceRunLengthEncode::Encode(nullptr, t2, K.d_keys_out.p, K.d_uniq.p, K.d_run_cnt.p, d_nruns, (int)nt_u, s);
-    cub::DeviceScan::ExclusiveSum(nullptr, t3, K.d_run_cnt.p, K.d_run_off.p, (int)nt_u, s);
-    size_t tmp = std::max(t1, std::max(t2, t3));
-    CUDA_TRY(K.cub_tmp.reserve(tmp));
-    CUDA_TRY(cub::DeviceRadixSort::SortPairs(K.cub_tmp.p, tmp, K.d_keys_in.p, K.d_keys_out.p, K.d_vals_in.p, K.d_vals_out.p, (int)nt_u, 0, end_bit, s));
-    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(K.cub_tmp.p, tmp, K.d_keys_out.p, K.d_uniq.p, K.d_run_cnt.p, d_nruns, (int)nt_u, s));
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(K.cub_tmp.p, tmp, K.d_run_cnt.p, K.d_run_off.p, (int)nt_u, s));
-    CUDA_TRY(cudaMemcpyAsync(K.h_small.p, d_nruns, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-    CUDA_TRY(cudaStreamSynchronize(s));
-    const int nruns = K.h_small.p[0];
-    CUDA_TRY(K.d_sums.reserve((size_t)nruns * 9));
-    CUDA_TRY(K.d_centroid.reserve((size_t)nruns * 3 + 4));
-    CUDA_TRY(K.d_leafF.reserve(nruns)); CUDA_TRY(K.d_leafD.reserve(nruns)); CUDA_TRY(K.d_cov.reserve((size_t)nruns * 9));
-    CUDA_TRY(K.d_npts.reserve(nruns)); CUDA_TRY(K.d_valid.reserve(nruns));
-    CUDA_TRY(K.d_cell2leaf.reserve((size_t)cells));
-    CUDA_TRY(K.d_cell2run.reserve((size_t)cells));
-    CUDA_TRY(cudaMemsetAsync(K.d_cell2leaf.p, 0xFF, (size_t)cells * sizeof(int32_t), s));
-    CUDA_TRY(cudaMemsetAsync(K.d_cell2run.p, 0xFF, (size_t)cells * sizeof(int32_t), s));
-    int32_t* d_nvalid = K.d_small.p + 9;
-    CUDA_TRY(cudaMemsetAsync(d_nvalid, 0, sizeof(int32_t), s));
-    CUDA_TRY(cudaMemsetAsync(K.d_cov.p, 0, (size_t)nruns * 9 * sizeof(double), s));
-    const int acc_blocks = std::min((nruns + 7) / 8, K.sm_count * 8);
-    k_ndt_accumulate<<<std::max(acc_blocks, 1), 256, 0, s>>>(K.d_tgt.p, K.d_vals_out.p, K.d_uniq.p, K.d_run_off.p, K.d_run_cnt.p, d_nruns, sentinel,
-                                                             K.d_sums.p, K.d_centroid.p);
-    k_ndt_finalize<<<(nruns + 127) / 128, 128, 0, s>>>(K.d_uniq.p, K.d_run_cnt.p, d_nruns, sentinel, K.d_sums.p, K.prm.min_pts, K.prm.eig_ratio,
-                                                       K.d_leafF.p, K.d_leafD.p, K.d_cov.p, K.d_npts.p, K.d_valid.p, K.d_cell2leaf.p, d_nvalid);
-    // fitness index: target points in cell order, cell -> run
-    CUDA_TRY(K.d_tgt_sorted.reserve((size_t)nt_u));
-    k_ndt_gather<<<(unsigned)((nt_u + 255) / 256), 256, 0, s>>>(K.d_tgt.p, K.d_vals_out.p, (int)nt_u, K.d_tgt_sorted.p);
-    k_ndt_cell_runs<<<(nruns + 255) / 256, 256, 0, s>>>(K.d_uniq.p, d_nruns, sentinel, K.d_cell2run.p);
-    last_nruns = nruns;
+    rc = K.build_leaves(np, (unsigned)std::min<int64_t>((max_tn + 255) / 256, 1024), nt_u, cells);
+    if (rc) return rc;
+    rc = K.build_fitness_index(nt_u, cells);
+    if (rc) return rc;
+    last_nruns = K.nruns;
     // sources: one stable sort by (pair, Morton key), so every pair is ordered as set_source orders it alone
     CUDA_TRY(d_skeys_in.reserve(ns_u)); CUDA_TRY(d_skeys_out.reserve(ns_u));
     CUDA_TRY(K.s_vals_in.reserve(ns_u)); CUDA_TRY(K.s_vals_out.reserve(ns_u)); CUDA_TRY(K.d_src.reserve((size_t)ns_u));
@@ -2105,24 +2075,26 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
         K.d_src_raw.p, d_soff, 1.0f / K.prm.resolution, d_skeys_in.p, K.s_vals_in.p);
     int s_end = 33;
     while (s_end < 64 && ((int64_t)1 << (s_end - 32)) < np) ++s_end;
-    tmp = 0;
+    size_t tmp = 0;
     CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp, d_skeys_in.p, d_skeys_out.p, K.s_vals_in.p, K.s_vals_out.p, (int)ns_u, 0, s_end, s));
     CUDA_TRY(K.s_tmp.reserve(tmp));
     CUDA_TRY(cub::DeviceRadixSort::SortPairs(K.s_tmp.p, tmp, d_skeys_in.p, d_skeys_out.p, K.s_vals_in.p, K.s_vals_out.p, (int)ns_u, 0, s_end, s));
     k_ndt_gather<<<(unsigned)((ns_u + 255) / 256), 256, 0, s>>>(K.d_src_raw.p, K.s_vals_out.p, (int)ns_u, K.d_src.p);
-    LAUNCH_COUNT(7);
-    // alignment: one control block and one view per built pair
+    LAUNCH_COUNT(2);
+    // alignment: one control block and one view per built pair; fitness: one row per built pair, moved by the final
+    // transformation in its control block
     K.gauss();  // recomputed at every computeTransformation (ndt_omp_impl.hpp:77-81)
     View base = K.view();
     base.nbr7 = nullptr;
     CUDA_TRY(h_pe.reserve((size_t)n_live)); CUDA_TRY(d_pe.reserve((size_t)n_live));
     CUDA_TRY(h_pf.reserve((size_t)n_live)); CUDA_TRY(d_pf.reserve((size_t)n_live));
     CUDA_TRY(K.h_poses.reserve((size_t)n_live * 16)); CUDA_TRY(K.d_poses.reserve((size_t)n_live * 16));
-    std::vector<int64_t> live(n_live), d2off(n_live + 1, 0);
+    CUDA_TRY(K.d_ctl.reserve(n_live)); CUDA_TRY(K.h_ctl.reserve(n_live));
+    std::vector<int64_t> live(n_live);
     int max_nbx = 1;
-    int64_t max_live_sn = 1;
+    int64_t max_live_sn = 1, n_d2 = 0;
     for (int64_t j = 0, a = 0; j < np; ++j) {
-        const PairGrid& g = h_pg.p[j];
+        const PairGrid& g = K.h_pg.p[j];
         if (!g.live) continue;
         live[a] = j;
         const int64_t sn = soff[j + 1] - soff[j];
@@ -2135,13 +2107,8 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
         const int64_t items = sn * K.nst();
         e.nbx = (int)std::max<int64_t>(1, (items + EVAL_THREADS * kPairMaxItemsPerThread - 1) / (EVAL_THREADS * kPairMaxItemsPerThread));
         max_nbx = std::max(max_nbx, e.nbx);
-        PairFit& f = h_pf.p[a];
-        f.f.pts = K.d_tgt_sorted.p; f.f.cell2run = K.d_cell2run.p + g.cell_base; f.f.run_off = K.d_run_off.p; f.f.run_cnt = K.d_run_cnt.p;
-        for (int q = 0; q < 3; ++q) { f.f.min_b[q] = g.gd.min_b[q]; f.f.div_b[q] = g.gd.div_b[q]; }
-        f.f.leaf = K.prm.resolution; f.f.inv_leaf = g.gd.inv_leaf;
-        f.src = e.v.src;
-        f.n = (int)sn;
-        d2off[a + 1] = d2off[a] + sn;
+        h_pf.p[a] = FitRow{K.fit_view(g.gd, g.cell_base), e.v.src, (int)sn, n_d2, K.d_ctl.p[a].final_T};
+        n_d2 += sn;
         max_live_sn = std::max(max_live_sn, sn);
         float* G = K.h_poses.p + a * 16;
         if (c.guesses16) memcpy(G, c.guesses16 + ids[j] * 16, 16 * sizeof(float));
@@ -2149,30 +2116,25 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
         ++a;
     }
     CUDA_TRY(cudaMemcpyAsync(d_pe.p, h_pe.p, n_live * sizeof(PairEval), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(cudaMemcpyAsync(d_pf.p, h_pf.p, n_live * sizeof(PairFit), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(d_pf.p, h_pf.p, n_live * sizeof(FitRow), cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(K.d_poses.p, K.h_poses.p, n_live * 16 * sizeof(float), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(K.d_ctl.reserve(n_live)); CUDA_TRY(K.h_ctl.reserve(n_live));
     const int part_stride = NACC * max_nbx;
     CUDA_TRY(K.d_partials.reserve((size_t)n_live * part_stride));
     AlignConsts kc{K.prm.step_size, K.prm.trans_eps, K.prm.max_iter, 0};
     k_ndt_init<<<(unsigned)((n_live + 63) / 64), 64, 0, s>>>(K.d_ctl.p, (int)n_live, K.d_poses.p, nullptr, PH_INIT);
     int launches = 1;
     const int max_launches = (K.prm.max_iter + 3) * 12 + 1;
-    int32_t rc = K.until_done((int)n_live, max_launches, launches, [&]() {
+    rc = K.until_done((int)n_live, max_launches, launches, [&]() {
         k_ndt_eval<false, true><<<dim3(max_nbx, (unsigned)n_live), EVAL_THREADS, 0, s>>>(View{}, K.d_ctl.p, kc, K.d_partials.p, nullptr, 1, d_pe.p,
                                                                                             part_stride);
     });
     LAUNCH_COUNT(launches);
     if (rc) return rc;
-    // getFitnessScore(max_range) of every pair at its final transformation, read from its control block on the device
-    CUDA_TRY(d_d2off.reserve((size_t)n_live + 1));
-    CUDA_TRY(h_off.reserve((size_t)n_live + 1));
-    memcpy(h_off.p, d2off.data(), (n_live + 1) * sizeof(int64_t));  // h_off's chunk offsets reached the device before the last poll
-    CUDA_TRY(cudaMemcpyAsync(d_d2off.p, h_off.p, (n_live + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
-    CUDA_TRY(K.d_fit.reserve((size_t)d2off[n_live]));
+    // getFitnessScore(max_range) of every pair at its final transformation
+    CUDA_TRY(K.d_fit.reserve((size_t)n_d2));
     CUDA_TRY(d_fitsum.reserve(2 * (size_t)n_live)); CUDA_TRY(h_fitsum.reserve(2 * (size_t)n_live));
-    k_ndt_fitness_pairs<<<dim3((unsigned)((max_live_sn * 32 + 255) / 256), (unsigned)n_live), 256, 0, s>>>(d_pf.p, K.d_ctl.p, d_d2off.p, K.d_fit.p);
-    k_ndt_fitness_reduce_pairs<<<(unsigned)n_live, 256, 0, s>>>(K.d_fit.p, d_d2off.p, c.max_range, d_fitsum.p);
+    k_ndt_fitness<<<dim3((unsigned)((max_live_sn * 32 + 255) / 256), (unsigned)n_live), 256, 0, s>>>(d_pf.p, K.d_fit.p);
+    k_ndt_fitness_reduce<<<(unsigned)n_live, 256, 0, s>>>(d_pf.p, K.d_fit.p, c.max_range, d_fitsum.p);
     LAUNCH_COUNT(3);
     CUDA_TRY(cudaMemcpyAsync(K.h_ctl.p, K.d_ctl.p, n_live * sizeof(Ctl), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(h_fitsum.p, d_fitsum.p, 2 * n_live * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -2226,13 +2188,49 @@ int32_t b200_ndt_pairs::local(const Call& c, int64_t P, int64_t first, int64_t s
     return B200_OK;
 }
 
+// The valid leaves of the last target build whose key lies in [lo, hi), in key order, reported with leaf id = key - lo
+// (the parity probe of b200_ndt_leaves / b200_ndt_pairs_leaves): how many there are; the first `max` are written.
+static int64_t read_leaves(Ndt& k, int nr, uint64_t lo, uint64_t hi, int64_t max, int64_t* ids, int32_t* npts, double* mean3, double* cov9,
+                           double* icov9) {
+    cudaSetDevice(k.device);
+    std::vector<uint8_t> valid(nr);
+    std::vector<uint32_t> uniq(nr);
+    std::vector<int32_t> np(nr);
+    std::vector<ndt::LeafD> L(nr);
+    std::vector<double> cov((size_t)nr * 9);
+    cudaStreamSynchronize(k.stream);
+    cudaMemcpy(valid.data(), k.d_valid.p, nr, cudaMemcpyDeviceToHost);
+    cudaMemcpy(uniq.data(), k.d_uniq.p, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(np.data(), k.d_npts.p, nr * sizeof(int32_t), cudaMemcpyDeviceToHost);
+    cudaMemcpy(L.data(), k.d_leafD.p, nr * sizeof(ndt::LeafD), cudaMemcpyDeviceToHost);
+    cudaMemcpy(cov.data(), k.d_cov.p, (size_t)nr * 9 * sizeof(double), cudaMemcpyDeviceToHost);
+    int64_t cnt = 0;
+    for (int r = 0; r < nr; ++r) {  // runs are sorted by key
+        if (!valid[r] || uniq[r] < lo || uniq[r] >= hi) continue;
+        if (cnt < max) {
+            if (ids) ids[cnt] = (int64_t)(uniq[r] - lo);
+            if (npts) npts[cnt] = np[r];
+            if (mean3) memcpy(mean3 + cnt * 3, L[r].mean, 24);
+            if (cov9) memcpy(cov9 + cnt * 9, &cov[(size_t)r * 9], 72);
+            if (icov9) memcpy(icov9 + cnt * 9, L[r].icov, 72);
+        }
+        ++cnt;
+    }
+    return cnt;
+}
+
+static int32_t check_device(int32_t device) {
+    int ndev = 0;
+    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) B200_FAIL(B200_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
+    if (device < 0 || device >= ndev) B200_FAIL(B200_ERR_ARG, "bad device ordinal");
+    return B200_OK;
+}
+
 extern "C" {
 
 int32_t b200_ndt_create(const b200_ndt_params* params, int32_t device, b200_ndt** out) {
     if (!params || !out) B200_FAIL(B200_ERR_ARG, "null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) B200_FAIL(B200_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) B200_FAIL(B200_ERR_ARG, "bad device ordinal");
+    if (const int32_t rc = check_device(device)) return rc;
     b200_ndt* h = new b200_ndt();
     int32_t rc = h->k.init(params, device);
     if (rc != B200_OK) { h->k.destroy(); delete h; return rc; }
@@ -2306,33 +2304,7 @@ int32_t b200_ndt_debug_cycles(b200_ndt* n, int64_t* step_cycles, int64_t* solve_
 
 int64_t b200_ndt_leaves(b200_ndt* n, int64_t max, int64_t* ids, int32_t* npts, double* mean3, double* cov9, double* icov9) {
     if (!n || !n->k.have_target) return 0;
-    Ndt& k = n->k;
-    cudaSetDevice(k.device);
-    const int nr = k.nruns;
-    std::vector<uint8_t> valid(nr);
-    std::vector<uint32_t> uniq(nr);
-    std::vector<int32_t> np(nr);
-    std::vector<ndt::LeafD> L(nr);
-    std::vector<double> cov((size_t)nr * 9);
-    cudaStreamSynchronize(k.stream);
-    cudaMemcpy(valid.data(), k.d_valid.p, nr, cudaMemcpyDeviceToHost);
-    cudaMemcpy(uniq.data(), k.d_uniq.p, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
-    cudaMemcpy(np.data(), k.d_npts.p, nr * sizeof(int32_t), cudaMemcpyDeviceToHost);
-    cudaMemcpy(L.data(), k.d_leafD.p, nr * sizeof(ndt::LeafD), cudaMemcpyDeviceToHost);
-    cudaMemcpy(cov.data(), k.d_cov.p, (size_t)nr * 9 * sizeof(double), cudaMemcpyDeviceToHost);
-    int64_t cnt = 0;
-    for (int r = 0; r < nr; ++r) {  // runs are sorted by leaf id
-        if (!valid[r]) continue;
-        if (cnt < max) {
-            if (ids) ids[cnt] = (int64_t)uniq[r];
-            if (npts) npts[cnt] = np[r];
-            if (mean3) memcpy(mean3 + cnt * 3, L[r].mean, 24);
-            if (cov9) memcpy(cov9 + cnt * 9, &cov[(size_t)r * 9], 72);
-            if (icov9) memcpy(icov9 + cnt * 9, L[r].icov, 72);
-        }
-        ++cnt;
-    }
-    return cnt;
+    return read_leaves(n->k, n->k.nruns, 0, (uint64_t)n->k.ncells, max, ids, npts, mean3, cov9, icov9);
 }
 
 int32_t b200_ndt_grid(b200_ndt* n, int32_t* min_b3, int32_t* div_b3) {
@@ -2498,17 +2470,17 @@ int64_t b200_ndt_nbhd_total(b200_ndt* n, const double* p6) {
             for (int j = 0; j < 3; ++j) T1[i * 3 + j] = (Rx[i * 3] * Ry[j] + Rx[i * 3 + 1] * Ry[3 + j]) + Rx[i * 3 + 2] * Ry[6 + j];
         for (int i = 0; i < 3; ++i)
             for (int j = 0; j < 3; ++j) T2[i * 3 + j] = (T1[i * 3] * Rz[j] + T1[i * 3 + 1] * Rz[3 + j]) + T1[i * 3 + 2] * Rz[6 + j];
-        for (int i = 0; i < 3; ++i) {
-            for (int j = 0; j < 3; ++j) M[i * 4 + j] = T2[i * 3 + j];
-            M[i * 4 + 3] = (float)p6[i];
+        for (int i = 0; i < 3; ++i) {  // column-major
+            for (int j = 0; j < 3; ++j) M[j * 4 + i] = T2[i * 3 + j];
+            M[12 + i] = (float)p6[i];
         }
-        M[12] = M[13] = M[14] = 0.f; M[15] = 1.f;
+        M[3] = M[7] = M[11] = 0.f; M[15] = 1.f;
     }
     if (k.d_poses.reserve(16) != cudaSuccess || k.h_poses.reserve(16) != cudaSuccess) return -1;
     memcpy(k.h_poses.p, M, sizeof M);
     cudaMemcpyAsync(k.d_poses.p, k.h_poses.p, sizeof M, cudaMemcpyHostToDevice, k.stream);
     cudaMemsetAsync(k.d_best.p, 0, sizeof(unsigned long long), k.stream);
-    ndt::k_ndt_nbhd_total<<<k.sm_count, 256, 0, k.stream>>>(k.view(), k.d_poses.p, k.d_best.p);
+    ndt::k_ndt_pairs_batch<<<dim3(k.sm_count, 1), 256, 0, k.stream>>>(k.view(), k.d_poses.p, k.d_best.p);
     cudaMemcpyAsync(k.h_best.p, k.d_best.p, sizeof(unsigned long long), cudaMemcpyDeviceToHost, k.stream);
     cudaStreamSynchronize(k.stream);
     return (int64_t)k.h_best.p[0];
@@ -2619,9 +2591,7 @@ int32_t b200_reloc_argmin_strided(b200_comm* comm, b200_ndt* n, const float* pos
 
 int32_t b200_ndt_pairs_create(const b200_ndt_params* params, int32_t device, b200_ndt_pairs** out) {
     if (!params || !out) B200_FAIL(B200_ERR_ARG, "null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) B200_FAIL(B200_ERR_CUDA, "no CUDA device (there is no CPU fallback)");
-    if (device < 0 || device >= ndev) B200_FAIL(B200_ERR_ARG, "bad device ordinal");
+    if (const int32_t rc = check_device(device)) return rc;
     b200_ndt_pairs* h = new b200_ndt_pairs();
     const int32_t rc = h->k.init(params, device);
     if (rc != B200_OK) { h->destroy(); delete h; return rc; }
@@ -2701,34 +2671,8 @@ int64_t b200_ndt_pairs_leaves(b200_ndt_pairs* h, int64_t p, int64_t max, int64_t
     size_t j = 0;
     while (j < h->last_ids.size() && h->last_ids[j] != p) ++j;
     if (j == h->last_ids.size() || !h->last_live[j]) return -1;
-    Ndt& k = h->k;
-    cudaSetDevice(k.device);
-    const int nr = h->last_nruns;
-    std::vector<uint8_t> valid(nr);
-    std::vector<uint32_t> uniq(nr);
-    std::vector<int32_t> np(nr);
-    std::vector<ndt::LeafD> L(nr);
-    std::vector<double> cov((size_t)nr * 9);
-    cudaStreamSynchronize(k.stream);
-    cudaMemcpy(valid.data(), k.d_valid.p, nr, cudaMemcpyDeviceToHost);
-    cudaMemcpy(uniq.data(), k.d_uniq.p, nr * sizeof(uint32_t), cudaMemcpyDeviceToHost);
-    cudaMemcpy(np.data(), k.d_npts.p, nr * sizeof(int32_t), cudaMemcpyDeviceToHost);
-    cudaMemcpy(L.data(), k.d_leafD.p, nr * sizeof(ndt::LeafD), cudaMemcpyDeviceToHost);
-    cudaMemcpy(cov.data(), k.d_cov.p, (size_t)nr * 9 * sizeof(double), cudaMemcpyDeviceToHost);
-    const uint64_t lo = h->last_base[j], hi = lo + (uint64_t)h->last_ncells[j];
-    int64_t cnt = 0;
-    for (int r = 0; r < nr; ++r) {  // runs are sorted by key = cell_base + leaf id
-        if (!valid[r] || uniq[r] < lo || uniq[r] >= hi) continue;
-        if (cnt < max) {
-            if (ids) ids[cnt] = (int64_t)(uniq[r] - lo);
-            if (npts) npts[cnt] = np[r];
-            if (mean3) memcpy(mean3 + cnt * 3, L[r].mean, 24);
-            if (cov9) memcpy(cov9 + cnt * 9, &cov[(size_t)r * 9], 72);
-            if (icov9) memcpy(icov9 + cnt * 9, L[r].icov, 72);
-        }
-        ++cnt;
-    }
-    return cnt;
+    const uint64_t lo = h->last_base[j];
+    return read_leaves(h->k, h->last_nruns, lo, lo + (uint64_t)h->last_ncells[j], max, ids, npts, mean3, cov9, icov9);
 }
 
 }  // extern "C"
