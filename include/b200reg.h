@@ -305,6 +305,29 @@ int32_t b200_reloc_argmin(b200_comm* comm, b200_ndt* ndt, const float* poses16, 
 /* same with an interleaved slice: local hypothesis i = global hypothesis h_begin + i * h_stride (rank r of N: h_begin r, stride N) */
 int32_t b200_reloc_argmin_strided(b200_comm* comm, b200_ndt* ndt, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride,
                                   int64_t* best, double* best_score, float* gpu_ms);
+/* Global relocalization with NDT refinement: score -> global top-K -> align() of every candidate -> getFitnessScore -> winner.
+ * Slices as for b200_reloc_argmin_strided (comm may be NULL).  The candidates are the top_k hypotheses of highest
+ * calculateScore over all ranks (NaN scores and poses with a non-finite entry never qualify), ordered by score descending,
+ * then global index ascending; *n_cands = how many there are (fewer than top_k when fewer hypotheses have a finite score).
+ * Candidate j is aligned on rank j mod N from its hypothesis pose with computeTransformation against the handle's target and
+ * source, then getFitnessScore(max_range) runs at its final transformation.  cands[0 .. top_k) receives the candidates in that
+ * order (slots past *n_cands: hypothesis -1, everything else zero); refined.ndt.gpu_ms is 0 - the device time of the whole
+ * call is *gpu_ms (may be NULL, as may n_cands).  A candidate's record depends only on its pose, the handle's target and
+ * source and the parameters: it is bit-identical for any top_k, slicing and number of ranks.
+ * *best = the hypothesis of the converged candidate (refined.status == B200_OK) with the highest trans_probability, ties to
+ * the lower hypothesis, and the call returns B200_OK; with no converged candidate, the highest trans_probability among all of
+ * them and B200_NOT_CONVERGED; with no candidate at all, -1 and B200_NO_EFFECTIVE_POINTS.
+ * With a communicator every rank passes the same top_k and max_range (they set the sizes of the two ncclAllGathers), and every
+ * rank returns the same code, *best and cands: a rank whose own part fails (a malformed slice, no target or source, a CUDA
+ * error) still takes part in both collectives and its error is returned everywhere.  A NULL ndt or a top_k outside
+ * 1 .. 65535 is B200_ERR_ARG at once, before any collective. */
+typedef struct {
+    int64_t hypothesis;           /* global index h_begin + i * h_stride on the rank that scored it; -1 = empty slot */
+    double initial_score;         /* calculateScore at the hypothesis pose: the bits b200_ndt_score_batch returns */
+    b200_ndt_pair_result refined; /* status (B200_OK / B200_NOT_CONVERGED), align result, fitness at the final pose, final16 */
+} b200_reloc_candidate;
+int32_t b200_reloc_refine(b200_comm* comm, b200_ndt* ndt, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride,
+                          int64_t top_k, double max_range, int64_t* best, b200_reloc_candidate* cands, int64_t* n_cands, float* gpu_ms);
 
 /* measurement aids (bench.py): device time of the score kernel of the last score / relocalization call; the number of
  * (source point, occupied neighbourhood voxel) pairs over h poses (algorithmic bytes of the roofline); a device-side

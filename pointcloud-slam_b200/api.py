@@ -58,6 +58,11 @@ class NdtPairResult(C.Structure):
                 ("final16", C.c_float * 16)]
 
 
+class RelocCandidate(C.Structure):
+    """b200_reloc_candidate (include/b200reg.h)."""
+    _fields_ = [("hypothesis", C.c_int64), ("initial_score", C.c_double), ("refined", NdtPairResult)]
+
+
 class GicpParams(C.Structure):
     _fields_ = [("k_correspondences", C.c_int32), ("gicp_epsilon", C.c_double), ("rotation_epsilon", C.c_double),
                 ("transformation_epsilon", C.c_double), ("corr_dist_threshold", C.c_double), ("max_iterations", C.c_int32),
@@ -169,6 +174,9 @@ def lib():
         L.b200_ndt_last_score_kernel_ms.argtypes = [vp]
         L.b200_ndt_score_pairs.argtypes = [vp, vp, i64, vp]
         L.b200_ndt_stream_barrier.argtypes = [vp, vp]
+    if hasattr(L, "b200_reloc_refine"):  # absent from builds older than the refined relocalization (B200REG_LIB A/B timing)
+        L.b200_reloc_refine.argtypes = [vp, vp, vp, i64, i64, i64, i64, C.c_double, vp, vp, vp, vp]
+        L.b200_ndt_last_polls.argtypes = [vp]
     if hasattr(L, "b200_ndt_pairs_create"):  # absent from builds older than the batched pair registration (B200REG_LIB A/B timing)
         L.b200_ndt_pairs_create.argtypes = [C.POINTER(NdtParams), i32, C.POINTER(vp)]
         L.b200_ndt_pairs_destroy.argtypes = [vp]
@@ -882,6 +890,96 @@ def relocalize(ndt: "NormalDistributionsTransform", poses_cm16, comm: Communicat
                                          poses.shape[0], h_begin, h_stride, C.byref(best), C.byref(score), C.byref(ms))
     _check(rc)
     return best.value, score.value, ms.value
+
+
+def relocalize_refine(ndt: "NormalDistributionsTransform", poses_slice, comm: Communicator | None = None, h_begin=0, h_stride=1, top_k=16,
+                      max_range=1.7976931348623157e308):
+    """Global relocalization with NDT refinement (b200_reloc_refine): the top_k hypotheses of highest calculateScore over all
+    ranks are aligned from their poses (candidate j on rank j mod N) and the converged one with the highest transformation
+    probability wins.  Slices as for relocalize(); top_k and max_range must be equal on every rank.  Returns
+    (best, candidates, gpu_ms) - identical on every rank; candidates = the RelocCandidate records in candidate order (score
+    descending, index ascending), as many as have a finite score.  B200_NOT_CONVERGED (no candidate converged; best is then the
+    candidate of highest probability) and B200_NO_EFFECTIVE_POINTS (no candidate; best = -1) are not errors: the code is in
+    `.status` of the returned list."""
+    poses = np.ascontiguousarray(poses_slice, dtype=np.float32).reshape(-1, 16)
+    res = (RelocCandidate * int(top_k))()
+    best, nc, ms = C.c_int64(-1), C.c_int64(0), C.c_float(0)
+    rc = lib().b200_reloc_refine(comm.h if comm is not None else None, ndt._handle(), _p(poses) if len(poses) else None, poses.shape[0],
+                                 h_begin, h_stride, int(top_k), max_range, C.byref(best), res, C.byref(nc), C.byref(ms))
+    _check(rc)
+    cands = RelocCandidates(res[:nc.value])
+    cands.status = rc
+    cands.records = res
+    return best.value, cands, ms.value
+
+
+class RelocCandidates(list):
+    """The candidates of relocalize_refine(); .status = the call's return code, .records = all top_k ctypes slots."""
+    status = 0
+    records = None
+
+
+def _reloc_record_words(key, hyp, pose16):
+    """One 80-byte entry of exchange 1 as 10 int64 words: key (shifted into int64 order), hypothesis, pose (16 float32)."""
+    return [key - (1 << 63), hyp] + np.asarray(pose16, np.float32).reshape(16).view(np.int64).tolist()
+
+
+def reloc_refine_protocol_host(scores, poses, h_begin, h_stride, top_k, nranks, rank, all_gather, refine, status=0):
+    """Host mirror of b200_reloc_refine's two exchanges (used by the CPU gloo test).  scores / poses = this rank's slice (local
+    hypothesis i = global h_begin + i * h_stride); all_gather(int64 tensor) returns the tensors of all ranks stacked ([R, ...]);
+    refine(pose16) -> (status, trans_probability, fitness) aligns one candidate; status != 0 = this rank's own failure.
+    Exchange 1: a header and this rank's top_k entries sorted by (score key desc, index asc), empty entries last.  Global order:
+    the same over the gathered lists (ties across ranks cannot occur: indices are distinct).  Candidate j is refined on rank
+    j mod nranks.  Exchange 2: a header and one record per row (j = rank + row * nranks).  Returns a dict: status, best,
+    candidates [(hypothesis, key)], dealt (the j this rank refined), refined [(hypothesis, status, trans_probability, fitness)]."""
+    import torch
+    K = int(top_k)
+    rows = (K + nranks - 1) // nranks
+    keys = []
+    for i, s in enumerate(scores):
+        finite = bool(np.isfinite(np.asarray(poses[i], np.float32)).all())
+        keys.append(score_key(float(s)) if finite else 0)
+    order = sorted(range(len(keys)), key=lambda i: (-keys[i], i))
+    send = [int(status)]
+    for r in range(K):
+        if status == 0 and r < len(order) and keys[order[r]] != 0:
+            i = order[r]
+            send += _reloc_record_words(keys[i], h_begin + i * h_stride, poses[i])
+        else:
+            send += _reloc_record_words(0, -1, np.zeros(16, np.float32))
+    got = all_gather(torch.tensor(send, dtype=torch.int64)).numpy().reshape(nranks, 1 + 10 * K)
+    headers1 = got[:, 0].tolist()
+    entries = []
+    for q in range(nranks):
+        rec = got[q, 1:].reshape(K, 10)
+        for i in range(K):
+            key = int(rec[i, 0]) + (1 << 63)
+            if key:
+                entries.append((key, int(rec[i, 1]), q, rec[i, 2:].copy().view(np.float32)))
+    entries.sort(key=lambda e: (-e[0], e[1], e[2]))
+    cand = entries[:K]
+    dealt = [j for j in range(len(cand)) if j % nranks == rank] if status == 0 else []
+    send2 = [int(status)] + [-1, 0, 0, 0] * rows
+    for j in dealt:
+        st, tp, fit = refine(cand[j][3])
+        row = j // nranks
+        send2[1 + 4 * row: 5 + 4 * row] = [cand[j][1], int(st), int(np.float64(tp).view(np.int64)), int(np.float64(fit).view(np.int64))]
+    got2 = all_gather(torch.tensor(send2, dtype=torch.int64)).numpy().reshape(nranks, 1 + 4 * rows)
+    refined = []
+    for j in range(len(cand)):
+        hyp, st, tp, fit = got2[j % nranks, 1 + 4 * (j // nranks): 5 + 4 * (j // nranks)].tolist()
+        refined.append((hyp, st, float(np.int64(tp).view(np.float64)), float(np.int64(fit).view(np.float64))))
+    bad = [h for h in headers1 + got2[:, 0].tolist() if h]
+    out = dict(candidates=[(e[1], e[0]) for e in cand], dealt=dealt, refined=refined)
+    if bad:
+        return dict(out, status=bad[0], best=-1)
+    if not refined:
+        return dict(out, status=1, best=-1)  # B200_NO_EFFECTIVE_POINTS
+    tkey = lambda r: (-score_key(r[2]), r[0])
+    ok = [r for r in refined if r[1] == 0]
+    if ok:
+        return dict(out, status=0, best=min(ok, key=tkey)[0])
+    return dict(out, status=2, best=min(refined, key=tkey)[0])  # B200_NOT_CONVERGED
 
 
 class VoxelGrid:

@@ -1303,6 +1303,193 @@ __global__ void k_ndt_fitness_reduce(const FitRow* __restrict__ rows, const doub
     }
 }
 
+// ------------------------------------------------------------------ relocalization with refinement (b200_reloc_refine)
+// score -> this rank's top K -> exchange 1 (every rank's sorted top K) -> global top K -> align of the candidates dealt to
+// this rank (candidate j on rank j mod N, row j / N) -> fitness -> exchange 2 (every rank's refined rows) -> winner.  Every
+// exchange slot starts with an 8-byte header holding the sender's status, so that all ranks agree on the outcome.
+struct TopRec {  // one entry of a rank's top K on the wire of exchange 1
+    unsigned long long key;  // dbl_key(score); 0 = empty (NaN score, non-finite pose, or fewer than K hypotheses)
+    long long hyp;           // global hypothesis index, -1 = empty
+    float pose[16];          // column-major
+};
+static_assert(sizeof(TopRec) == 80, "exchange-1 record");
+struct RowTab {  // the candidate on one of this rank's rows
+    long long j;             // global candidate position, -1 = the row is empty
+    unsigned long long key;
+    long long hyp;
+};
+__device__ __forceinline__ double key_dbl(unsigned long long k) {  // inverse of dbl_key for k != 0
+    return __longlong_as_double((long long)((k >> 63) ? (k & 0x7FFFFFFFFFFFFFFFull) : ~k));
+}
+
+// Ranking key of local hypothesis i (a pose with a non-finite entry never qualifies) and its local index
+__global__ void k_reloc_keys(const double* __restrict__ scores, const float* __restrict__ poses, int h, unsigned long long* __restrict__ keys,
+                             int32_t* __restrict__ vals) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= h) return;
+    bool finite = true;
+#pragma unroll
+    for (int q = 0; q < 16; ++q) finite = finite && isfinite(poses[(size_t)i * 16 + q]);
+    keys[i] = finite ? dbl_key(scores[i]) : 0ull;
+    vals[i] = i;
+}
+
+// This rank's send slot of exchange 1: header = status, then the first K entries of its slice sorted by (key desc, local
+// index asc) - the local index ascends with the global one, so that is (key desc, global index asc).  h = 0: K empty entries.
+__global__ void k_reloc_topk(const unsigned long long* __restrict__ skeys, const int32_t* __restrict__ svals, int h, const float* __restrict__ poses,
+                             long long h_begin, long long h_stride, int K, int status, uint8_t* __restrict__ slot) {
+    const int r = blockIdx.x * blockDim.x + threadIdx.x;
+    if (r == 0) *reinterpret_cast<long long*>(slot) = status;
+    if (r >= K) return;
+    TopRec t;
+    t.key = 0ull;
+    t.hyp = -1;
+    for (int q = 0; q < 16; ++q) t.pose[q] = 0.f;
+    if (r < h && skeys[r] != 0ull) {
+        const int i = svals[r];
+        t.key = skeys[r];
+        t.hyp = h_begin + (long long)i * h_stride;
+        for (int q = 0; q < 16; ++q) t.pose[q] = poses[(size_t)i * 16 + q];
+    }
+    reinterpret_cast<TopRec*>(slot + 8)[r] = t;
+}
+
+// a comes before b in the global order: key descending, hypothesis ascending (then rank, should two slices overlap)
+__device__ __forceinline__ bool reloc_before(unsigned long long ka, long long ha, int ra, unsigned long long kb, long long hb, int rb) {
+    return ka > kb || (ka == kb && (ha < hb || (ha == hb && ra < rb)));
+}
+// Global top K from the N gathered lists (each sorted, empties last): the position of entry (r, i) is i plus the number of
+// entries of every other list that come before it (a binary search per list).  Positions j < K with j mod N == me land on
+// row j / N of this rank: its guess goes straight into guesses, its identity into tab.  Every rank computes the same order.
+__global__ void k_reloc_merge(const uint8_t* __restrict__ gathered, long long slot_bytes, int N, int K, int me, float* __restrict__ guesses,
+                              RowTab* __restrict__ tab) {
+    const int total = N * K;
+    for (int e = blockIdx.x * blockDim.x + threadIdx.x; e < total; e += gridDim.x * blockDim.x) {
+        const int r = e / K, i = e - r * K;
+        const TopRec* L = reinterpret_cast<const TopRec*>(gathered + (size_t)r * slot_bytes + 8);
+        const unsigned long long key = L[i].key;
+        if (key == 0ull) continue;
+        const long long hyp = L[i].hyp;
+        long long pos = i;
+        for (int q = 0; q < N; ++q) {
+            if (q == r) continue;
+            const TopRec* Q = reinterpret_cast<const TopRec*>(gathered + (size_t)q * slot_bytes + 8);
+            int lo = 0, hi = K;
+            while (lo < hi) {
+                const int mid = (lo + hi) >> 1;
+                if (reloc_before(Q[mid].key, Q[mid].hyp, q, key, hyp, r)) lo = mid + 1;
+                else hi = mid;
+            }
+            pos += lo;
+        }
+        if (pos >= K || pos % N != me) continue;
+        const int row = (int)(pos / N);
+        for (int q = 0; q < 16; ++q) guesses[(size_t)row * 16 + q] = L[i].pose[q];
+        tab[row] = RowTab{pos, key, hyp};
+    }
+}
+
+// After k_ndt_init: rows that received no candidate are done before they start and have no fitness points
+__global__ void k_reloc_rows(const RowTab* __restrict__ tab, int rows, Ctl* __restrict__ ctls, FitRow* __restrict__ fit) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    if (a >= rows || tab[a].j >= 0) return;
+    ctls[a].done = 1;
+    fit[a].n = 0;
+}
+
+// This rank's send slot of exchange 2: header = status, then one b200_reloc_candidate per row (hypothesis -1 when empty).
+// gpu_ms stays 0 and the padding is zero, so the records of a candidate are byte-identical wherever it was refined.
+__global__ void k_reloc_pack(const RowTab* __restrict__ tab, int rows, const Ctl* __restrict__ ctls, const double* __restrict__ fitsum, int status,
+                             uint8_t* __restrict__ slot) {
+    const int a = blockIdx.x * blockDim.x + threadIdx.x;
+    if (a == 0) *reinterpret_cast<long long*>(slot) = status;
+    if (a >= rows) return;
+    b200_reloc_candidate c;
+    memset(&c, 0, sizeof c);
+    c.hypothesis = -1;
+    const RowTab t = tab[a];
+    if (t.j >= 0) {
+        const Ctl& ct = ctls[a];
+        c.hypothesis = t.hyp;
+        c.initial_score = key_dbl(t.key);
+        b200_ndt_pair_result& r = c.refined;
+        r.status = !ct.done ? B200_ERR_CUDA : ct.converged ? B200_OK : B200_NOT_CONVERGED;
+        for (int i = 0; i < 4; ++i)
+            for (int j = 0; j < 4; ++j) r.final16[j * 4 + i] = ct.final_T[i * 4 + j];
+        r.ndt.converged = ct.converged;
+        r.ndt.iters = ct.nr_iterations;
+        r.ndt.evals = ct.evals;
+        r.ndt.hess_evals = ct.hess_evals;
+        r.ndt.trans_probability = ct.trans_probability;
+        for (int q = 0; q < 36; ++q) r.ndt.hessian[q] = ct.H[q];
+        r.ndt.score = ct.score;
+        for (int q = 0; q < 6; ++q) r.ndt.p_final[q] = ct.p[q];
+        const double S = fitsum[2 * a], Cn = fitsum[2 * a + 1];
+        r.n_in_range = (int64_t)Cn;
+        r.fitness = Cn > 0 ? S / Cn : 1.7976931348623157e308;  // as Ndt::fitness (PCL returns DBL_MAX when nothing is in range)
+    }
+    memcpy(slot + 8 + (size_t)a * sizeof(b200_reloc_candidate), &c, sizeof c);
+}
+
+// One block over the gathered exchange-2 slots: the K records in candidate order (candidate j = slot j mod N, row j / N) and
+// the agreed outcome.  out[0] status (the first failing rank's code, exchange 1 before exchange 2), out[1] best, out[2] the
+// number of candidates, out[3] the failing rank or -1, then the K records.
+constexpr int WINNER_THREADS = 256;
+__global__ void __launch_bounds__(WINNER_THREADS) k_reloc_winner(const uint8_t* __restrict__ g1, long long slot1, const uint8_t* __restrict__ g2,
+                                                                 long long slot2, int N, int K, long long* __restrict__ out) {
+    constexpr int W = sizeof(b200_reloc_candidate) / 8;
+    static_assert(sizeof(b200_reloc_candidate) % 8 == 0, "records are copied in 8-byte words");
+    __shared__ unsigned long long s_ok_k[WINNER_THREADS], s_any_k[WINNER_THREADS];
+    __shared__ long long s_ok_h[WINNER_THREADS], s_any_h[WINNER_THREADS], s_cnt[WINNER_THREADS];
+    const int tid = threadIdx.x;
+    const long long none = 0x7FFFFFFFFFFFFFFFll;
+    unsigned long long ok_k = 0, any_k = 0;
+    long long ok_h = none, any_h = none, cnt = 0;
+    unsigned long long* dst = reinterpret_cast<unsigned long long*>(out + 4);
+    for (int j = tid; j < K; j += WINNER_THREADS) {
+        const uint8_t* rec = g2 + (size_t)(j % N) * slot2 + 8 + (size_t)(j / N) * sizeof(b200_reloc_candidate);
+        const unsigned long long* w = reinterpret_cast<const unsigned long long*>(rec);
+        for (int q = 0; q < W; ++q) dst[(size_t)j * W + q] = w[q];
+        const b200_reloc_candidate* c = reinterpret_cast<const b200_reloc_candidate*>(rec);
+        const long long hyp = c->hypothesis;
+        if (hyp < 0) continue;
+        ++cnt;
+        const unsigned long long tk = dbl_key(c->refined.ndt.trans_probability);
+        if (any_h == none || tk > any_k || (tk == any_k && hyp < any_h)) { any_k = tk; any_h = hyp; }
+        if (c->refined.status == B200_OK && (ok_h == none || tk > ok_k || (tk == ok_k && hyp < ok_h))) { ok_k = tk; ok_h = hyp; }
+    }
+    s_ok_k[tid] = ok_k; s_ok_h[tid] = ok_h; s_any_k[tid] = any_k; s_any_h[tid] = any_h; s_cnt[tid] = cnt;
+    __syncthreads();
+    for (int o = WINNER_THREADS / 2; o > 0; o >>= 1) {
+        if (tid < o) {
+            const int u = tid + o;
+            if (s_ok_h[u] != none && (s_ok_h[tid] == none || s_ok_k[u] > s_ok_k[tid] || (s_ok_k[u] == s_ok_k[tid] && s_ok_h[u] < s_ok_h[tid]))) {
+                s_ok_k[tid] = s_ok_k[u]; s_ok_h[tid] = s_ok_h[u];
+            }
+            if (s_any_h[u] != none && (s_any_h[tid] == none || s_any_k[u] > s_any_k[tid] || (s_any_k[u] == s_any_k[tid] && s_any_h[u] < s_any_h[tid]))) {
+                s_any_k[tid] = s_any_k[u]; s_any_h[tid] = s_any_h[u];
+            }
+            s_cnt[tid] += s_cnt[u];
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {
+        long long st = 0, bad = -1;
+        for (int x = 0; x < 2 && !st; ++x)
+            for (int q = 0; q < N; ++q) {
+                const long long hq = *reinterpret_cast<const long long*>((x == 0 ? g1 + (size_t)q * slot1 : g2 + (size_t)q * slot2));
+                if (hq) { st = hq; bad = q; break; }
+            }
+        long long b = -1;
+        if (!st) {
+            if (s_cnt[0] == 0) st = B200_NO_EFFECTIVE_POINTS;
+            else if (s_ok_h[0] != none) { st = B200_OK; b = s_ok_h[0]; }
+            else { st = B200_NOT_CONVERGED; b = s_any_h[0]; }
+        }
+        out[0] = st; out[1] = b; out[2] = s_cnt[0]; out[3] = bad;
+    }
+}
+
 // ------------------------------------------------------------------ host object
 struct Ndt {
     b200_ndt_params prm;
@@ -1900,6 +2087,28 @@ int32_t Ndt::fitness(const float* T16, double max_range, double* score, int64_t*
     return B200_OK;
 }
 
+// b200_reloc_refine's buffers (the control blocks are the handle's d_ctl, which Ndt::until_done polls)
+struct RelocRefine {
+    DevBuf<unsigned long long> d_keys_in, d_keys_out;
+    DevBuf<int32_t> d_vals_in, d_vals_out;
+    DevBuf<uint8_t> d_sort_tmp, d_x1, d_x2;
+    DevBuf<float> d_guess;
+    DevBuf<RowTab> d_tab;
+    DevBuf<double> d_partials, d_fit, d_fitsum;
+    DevBuf<PairEval> d_pe;
+    PinnedBuf<PairEval> h_pe;
+    DevBuf<FitRow> d_pf;
+    PinnedBuf<FitRow> h_pf;
+    DevBuf<long long> d_out;
+    PinnedBuf<long long> h_out;
+    int last_polls = 0;  // host synchronisations of the last call
+    void release() {
+        d_keys_in.release(); d_keys_out.release(); d_vals_in.release(); d_vals_out.release(); d_sort_tmp.release(); d_x1.release(); d_x2.release();
+        d_guess.release(); d_tab.release(); d_partials.release(); d_fit.release(); d_fitsum.release(); d_pe.release(); h_pe.release();
+        d_pf.release(); h_pf.release(); d_out.release(); h_out.release();
+    }
+};
+
 }  // namespace ndt
 }  // namespace b200
 
@@ -1909,7 +2118,10 @@ int32_t Ndt::fitness(const float* T16, double max_range, double* score, int64_t*
 // ------------------------------------------------------------------ C ABI (B3)
 using namespace b200;
 using b200::ndt::Ndt;
-struct b200_ndt { Ndt k; };
+struct b200_ndt {
+    Ndt k;
+    ndt::RelocRefine rr;  // b200_reloc_refine
+};
 
 static void fill_result(const ndt::Ctl& c, float* final16, b200_ndt_result* r, float ms) {
     if (final16)
@@ -2240,6 +2452,7 @@ int32_t b200_ndt_create(const b200_ndt_params* params, int32_t device, b200_ndt*
 int32_t b200_ndt_destroy(b200_ndt* n) {
     if (!n) return B200_OK;
     n->k.destroy();
+    n->rr.release();
     delete n;
     return B200_OK;
 }
@@ -2587,6 +2800,143 @@ int32_t b200_reloc_argmin_strided(b200_comm* comm, b200_ndt* n, const float* pos
                                   double* best_score, float* gpu_ms) {
     return reloc_argmin_impl(comm, n, poses16, h, h_begin, h_stride, best, best_score, gpu_ms);
 }
+
+/* Relocalization with NDT refinement (include/b200reg.h).  One stream; the host reads nothing back before the final copy except
+ * the done polls of the alignments.  Rows: rank r refines candidates j = r, r + N, ... on rows j / N; a row's evaluation
+ * view is the handle's own and its block count is fixed by the source size (the rule of the loop-closure pairs), so a
+ * candidate's record never depends on the other rows, on top_k, on the slicing or on the ranks. */
+int32_t b200_reloc_refine(b200_comm* comm, b200_ndt* n, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride, int64_t top_k,
+                          double max_range, int64_t* best, b200_reloc_candidate* cands, int64_t* n_cands, float* gpu_ms) {
+    using namespace ndt;
+    if (!n || top_k < 1 || top_k > 65535) B200_FAIL(B200_ERR_ARG, "bad argument");
+    Ndt& k = n->k;
+    RelocRefine& rr = n->rr;
+    CUDA_SET_DEVICE(k.device);
+    cudaStream_t s = k.stream;
+    const int R = comm && comm->nranks > 1 ? comm->nranks : 1, me = R > 1 ? comm->rank : 0;
+    const int K = (int)top_k, rows = (K + R - 1) / R;
+    const size_t slot1 = 8 + (size_t)K * sizeof(TopRec), slot2 = 8 + (size_t)rows * sizeof(b200_reloc_candidate);
+    const size_t out_words = 4 + (size_t)K * (sizeof(b200_reloc_candidate) / 8);
+    // before any work: past this point every rank reaches both collectives
+    CUDA_TRY(rr.d_x1.reserve(slot1 * (R + 1))); CUDA_TRY(rr.d_x2.reserve(slot2 * (R + 1)));
+    CUDA_TRY(rr.d_tab.reserve(rows));
+    CUDA_TRY(rr.d_out.reserve(out_words)); CUDA_TRY(rr.h_out.reserve(out_words));
+    int64_t launches0 = g_kernel_launches.load();
+    int polls = 0;
+    // ---- local step 1: this rank's scores, sorted
+    auto step1 = [&]() -> int32_t {
+        if (h < 0 || (h > 0 && !poses16) || h_begin < 0 || h_stride < 1 || !best || !cands) B200_FAIL(B200_ERR_ARG, "bad argument");
+        if (h > 65535) B200_FAIL(B200_ERR_ARG, "at most 65535 hypotheses per call");
+        if (!k.have_target) B200_FAIL(B200_ERR_ARG, "no target set");
+        if (k.n_src < 1) B200_FAIL(B200_ERR_ARG, "no source set");
+        if (!h) return B200_OK;
+        CUDA_TRY(k.d_poses.reserve((size_t)h * 16)); CUDA_TRY(k.h_poses.reserve((size_t)h * 16)); CUDA_TRY(k.d_scores.reserve(h));
+        CUDA_TRY(rr.d_keys_in.reserve(h)); CUDA_TRY(rr.d_keys_out.reserve(h)); CUDA_TRY(rr.d_vals_in.reserve(h)); CUDA_TRY(rr.d_vals_out.reserve(h));
+        memcpy(k.h_poses.p, poses16, (size_t)h * 16 * sizeof(float));
+        CUDA_TRY(cudaMemcpyAsync(k.d_poses.p, k.h_poses.p, (size_t)h * 16 * sizeof(float), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaEventRecord(k.ev0, s));
+        const int yaw_built = k.yaw_built;
+        int32_t rc = k.score_batch_device(k.d_poses.p, h, k.d_scores.p);
+        if (rc) return rc;
+        if (k.yaw_built != yaw_built) ++polls;  // the first orderings of a source read back the bins they need
+        k_reloc_keys<<<(unsigned)((h + 255) / 256), 256, 0, s>>>(k.d_scores.p, k.d_poses.p, (int)h, rr.d_keys_in.p, rr.d_vals_in.p);
+        size_t tmp = 0;
+        CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(nullptr, tmp, rr.d_keys_in.p, rr.d_keys_out.p, rr.d_vals_in.p, rr.d_vals_out.p, (int)h, 0, 64, s));
+        CUDA_TRY(rr.d_sort_tmp.reserve(tmp));
+        // stable: equal keys keep ascending local (hence global) index
+        CUDA_TRY(cub::DeviceRadixSort::SortPairsDescending(rr.d_sort_tmp.p, tmp, rr.d_keys_in.p, rr.d_keys_out.p, rr.d_vals_in.p, rr.d_vals_out.p, (int)h, 0, 64, s));
+        LAUNCH_COUNT(2);
+        return B200_OK;
+    };
+    const int32_t rc1 = step1();
+    if (R == 1 && rc1) return rc1;
+    const std::string err1 = rc1 ? g_last_error : std::string();
+    if (rc1 || !h) CUDA_TRY(cudaEventRecord(k.ev0, s));
+    k_reloc_topk<<<(unsigned)((K + 255) / 256), 256, 0, s>>>(rr.d_keys_out.p, rr.d_vals_out.p, rc1 ? 0 : (int)h, k.d_poses.p, h_begin, h_stride, K, rc1,
+                                                           rr.d_x1.p);
+    LAUNCH_COUNT(1);
+    // ---- exchange 1: every rank's sorted top K and status
+    if (R > 1) NCCL_TRY(comm, comm->AllGather(rr.d_x1.p, rr.d_x1.p + slot1, slot1, ncclChar, comm->comm, s));
+    else CUDA_TRY(cudaMemcpyAsync(rr.d_x1.p + slot1, rr.d_x1.p, slot1, cudaMemcpyDeviceToDevice, s));
+    CUDA_TRY(cudaMemsetAsync(rr.d_tab.p, 0xFF, (size_t)rows * sizeof(RowTab), s));  // j = -1: empty row
+    // ---- local step 2: merge, align and fitness of this rank's rows
+    auto step2 = [&]() -> int32_t {
+        if (!k.have_fitness_index) {  // built on first use, as b200_ndt_fitness_score does
+            const int32_t rc = k.build_fitness_index(k.n_tgt, k.ncells);
+            if (rc) return rc;
+            k.have_fitness_index = true;
+        }
+        const int64_t ns = k.n_src;
+        const int nbx = (int)std::max<int64_t>(1, (ns * k.nst() + EVAL_THREADS * kPairMaxItemsPerThread - 1) / (EVAL_THREADS * kPairMaxItemsPerThread));
+        const int part_stride = NACC * nbx;
+        CUDA_TRY(k.d_ctl.reserve(rows)); CUDA_TRY(rr.d_guess.reserve((size_t)rows * 16));
+        CUDA_TRY(rr.d_pe.reserve(rows)); CUDA_TRY(rr.h_pe.reserve(rows)); CUDA_TRY(rr.d_pf.reserve(rows)); CUDA_TRY(rr.h_pf.reserve(rows));
+        CUDA_TRY(rr.d_partials.reserve((size_t)rows * part_stride));
+        CUDA_TRY(rr.d_fit.reserve((size_t)rows * ns)); CUDA_TRY(rr.d_fitsum.reserve(2 * (size_t)rows));
+        k.gauss();  // recomputed at every computeTransformation (ndt_omp_impl.hpp:77-81)
+        const View v = k.view();
+        const FitView fv = k.fit_view(k.gd, 0);
+        for (int a = 0; a < rows; ++a) {  // the rows do not depend on which candidates land on them
+            rr.h_pe.p[a] = PairEval{v, nbx};
+            rr.h_pf.p[a] = FitRow{fv, k.d_src.p, (int)ns, (int64_t)a * ns, k.d_ctl.p[a].final_T};
+        }
+        CUDA_TRY(cudaMemcpyAsync(rr.d_pe.p, rr.h_pe.p, rows * sizeof(PairEval), cudaMemcpyHostToDevice, s));
+        CUDA_TRY(cudaMemcpyAsync(rr.d_pf.p, rr.h_pf.p, rows * sizeof(FitRow), cudaMemcpyHostToDevice, s));
+        k_reloc_merge<<<(unsigned)std::min<int64_t>(((int64_t)R * K + 255) / 256, 1024), 256, 0, s>>>(rr.d_x1.p + slot1, (long long)slot1, R, K, me,
+                                                                                                   rr.d_guess.p, rr.d_tab.p);
+        k_ndt_init<<<(unsigned)((rows + 63) / 64), 64, 0, s>>>(k.d_ctl.p, rows, rr.d_guess.p, nullptr, PH_INIT);
+        k_reloc_rows<<<(unsigned)((rows + 255) / 256), 256, 0, s>>>(rr.d_tab.p, rows, k.d_ctl.p, rr.d_pf.p);
+        LAUNCH_COUNT(3);
+        AlignConsts kc{k.prm.step_size, k.prm.trans_eps, k.prm.max_iter, 0};
+        int launches = 1, evals = 0;
+        const int max_launches = (k.prm.max_iter + 3) * 12 + 1;
+        int32_t rc = k.until_done(rows, max_launches, launches, [&]() {
+            k_ndt_eval<false, true><<<dim3(nbx, (unsigned)rows), EVAL_THREADS, 0, s>>>(View{}, k.d_ctl.p, kc, rr.d_partials.p, nullptr, 1, rr.d_pe.p,
+                                                                                      part_stride);
+            ++evals;
+        });
+        LAUNCH_COUNT(launches - 1);
+        // until_done polls after LAUNCH_BATCH + 4 evaluations, then after every LAUNCH_BATCH
+        polls += evals ? 1 + (evals - (LAUNCH_BATCH + 4)) / LAUNCH_BATCH : 0;
+        if (rc) return rc;
+        k_ndt_fitness<<<dim3((unsigned)((ns * 32 + 255) / 256), (unsigned)rows), 256, 0, s>>>(rr.d_pf.p, rr.d_fit.p);
+        k_ndt_fitness_reduce<<<(unsigned)rows, 256, 0, s>>>(rr.d_pf.p, rr.d_fit.p, max_range, rr.d_fitsum.p);
+        LAUNCH_COUNT(2);
+        CUDA_TRY(cudaGetLastError());
+        return B200_OK;
+    };
+    int32_t rc2 = rc1;
+    if (!rc1) rc2 = step2();
+    const std::string err2 = rc1 ? err1 : rc2 ? g_last_error : std::string();
+    if (rc2 && !rc1) CUDA_TRY(cudaMemsetAsync(rr.d_tab.p, 0xFF, (size_t)rows * sizeof(RowTab), s));  // send empty rows
+    k_reloc_pack<<<(unsigned)((rows + 127) / 128), 128, 0, s>>>(rr.d_tab.p, rows, k.d_ctl.p, rr.d_fitsum.p, rc2, rr.d_x2.p);
+    LAUNCH_COUNT(1);
+    // ---- exchange 2: every rank's refined rows and status; the same winner everywhere
+    if (R > 1) NCCL_TRY(comm, comm->AllGather(rr.d_x2.p, rr.d_x2.p + slot2, slot2, ncclChar, comm->comm, s));
+    else CUDA_TRY(cudaMemcpyAsync(rr.d_x2.p + slot2, rr.d_x2.p, slot2, cudaMemcpyDeviceToDevice, s));
+    k_reloc_winner<<<1, WINNER_THREADS, 0, s>>>(rr.d_x1.p + slot1, (long long)slot1, rr.d_x2.p + slot2, (long long)slot2, R, K, rr.d_out.p);
+    LAUNCH_COUNT(1);
+    CUDA_TRY(cudaEventRecord(k.ev1, s));
+    CUDA_TRY(cudaMemcpyAsync(rr.h_out.p, rr.d_out.p, out_words * sizeof(long long), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    CUDA_TRY(cudaGetLastError());
+    rr.last_polls = polls + 1;
+    k.last_launches = (int)(g_kernel_launches.load() - launches0);
+    cudaEventElapsedTime(&k.last_ms, k.ev0, k.ev1);
+    if (gpu_ms) *gpu_ms = k.last_ms;
+    const long long* o = rr.h_out.p;
+    if (best) *best = o[1];
+    if (n_cands) *n_cands = o[2];
+    if (cands) memcpy(cands, o + 4, (size_t)K * sizeof(b200_reloc_candidate));
+    const int32_t st = (int32_t)o[0];
+    if (st < 0) {
+        if (o[3] == me) g_last_error = err2;
+        else fail(st, ("relocalization refinement failed on rank " + std::to_string(o[3])).c_str(), __FILE__, __LINE__);
+    }
+    return st;
+}
+/* measurement aid: host synchronisations (done polls, a first-use yaw read-back, the final copy) of the last b200_reloc_refine */
+int32_t b200_ndt_last_polls(b200_ndt* n) { return n ? n->rr.last_polls : 0; }
 
 
 int32_t b200_ndt_pairs_create(const b200_ndt_params* params, int32_t device, b200_ndt_pairs** out) {

@@ -80,6 +80,24 @@ class NormalDistributionsTransform {
         sync();
         check(b200_ndt_score_batch(ndt_, poses16, h, scores), "b200_ndt_score_batch");
     }
+    /// Global relocalization with refinement (b200_reloc_refine): the top_k hypotheses of highest calculateScore (poses16 =
+    /// this rank's slice, h x 16 column-major; local i = global h_begin + i * h_stride) are aligned from their poses and the
+    /// converged one with the highest transformation probability wins.  comm may be NULL; with one, every rank passes the
+    /// same top_k and max_range.  Returns the winning hypothesis (-1: none had a finite score) and fills the candidates in
+    /// order (score descending, index ascending); `converged` = false when no candidate converged.  Errors throw.
+    int64_t relocalizeRefine(b200_comm* comm, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride, int64_t top_k,
+                             std::vector<b200_reloc_candidate>& candidates, bool* converged = nullptr,
+                             double max_range = 1.7976931348623157e308) {
+        sync();
+        candidates.assign(top_k > 0 ? (size_t)top_k : 0, b200_reloc_candidate{});
+        int64_t best = -1, n = 0;
+        const int32_t rc = b200_reloc_refine(comm, ndt_, poses16, h, h_begin, h_stride, top_k, max_range, &best,
+                                             candidates.empty() ? nullptr : candidates.data(), &n, nullptr);
+        check(rc, "b200_reloc_refine");
+        candidates.resize((size_t)n);
+        if (converged) *converged = rc == B200_OK;
+        return best;
+    }
     b200_ndt* handle() { sync(); return ndt_; }
 
    private:
