@@ -234,6 +234,57 @@ int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* sr
  * the pair), when pair p was built in the last chunk of that call; -1 otherwise */
 int64_t b200_ndt_pairs_leaves(b200_ndt_pairs* h, int64_t p, int64_t max, int64_t* ids, int32_t* npts, double* mean3, double* cov9, double* icov9);
 
+/* Loop closure from a device keyframe store: the front half of performLoopClosure (LIO-SAM mapOptmization.cpp, from which
+ * jueying_slam derives) - detectLoopClosureDistance and loopFindNearKeyframes - on the device, feeding the pair registration
+ * above.  A keyframe is ONE cloud in the lidar frame, x y z intensity: LIO-SAM keeps a corner and a surf cloud per keyframe
+ * and loopFindNearKeyframes appends corner then surf, so pass them concatenated in that order (the order of the points sets
+ * the order of VoxelGrid's fp32 sums).  Poses are PointTypePose {x, y, z, roll, pitch, yaw} (float), moved into the world
+ * by pcl::getTransformation; times are seconds (double). */
+typedef struct b200_keyframes b200_keyframes;
+int32_t b200_keyframes_create(int32_t device, b200_keyframes** out);
+int32_t b200_keyframes_destroy(b200_keyframes* h);
+/* cornerCloudKeyFrames / surfCloudKeyFrames.push_back + cloudKeyPoses3D / cloudKeyPoses6D.push_back (saveKeyFramesAndFactor):
+ * records x y z[ intensity] at stride_bytes (>= 16 carries the intensity, 12 stores 0); *key = the keyframe's index (may be NULL) */
+int32_t b200_keyframes_add(b200_keyframes* h, const float* xyzi, int64_t n, int64_t stride_bytes, const float* pose6, double time, int64_t* key);
+/* correctPoses(): poses of keyframes first .. first+count-1 replaced by poses6 (count x 6 floats); clouds untouched */
+int32_t b200_keyframes_set_poses(b200_keyframes* h, int64_t first, int64_t count, const float* poses6);
+int64_t b200_keyframes_count(b200_keyframes* h); /* -1 for a NULL handle */
+
+typedef struct {
+    float search_radius;      /* historyKeyframeSearchRadius */
+    double time_gap;          /* historyKeyframeSearchTimeDiff */
+    int32_t search_num;       /* historyKeyframeSearchNum */
+    float leaf;               /* downSizeFilterICP leaf size */
+    int32_t min_source_points; /* 300: cureKeyframeCloud->size() below it is not registered */
+    int32_t min_target_points; /* 1000: prevKeyframeCloud->size() below it is not registered */
+    double max_range;         /* getFitnessScore argument */
+} b200_loop_params;
+typedef struct {
+    int64_t cur, pre;         /* pre = -1: no candidate */
+    float pre_sqdist;         /* squared distance of the detected candidate; 0 when pre was given or is -1 */
+    int32_t n_source, n_target; /* sizes after the downsample; 0 when not assembled */
+    b200_ndt_pair_result reg; /* B200_OK / B200_NOT_CONVERGED; B200_NO_EFFECTIVE_POINTS = no candidate or under a size gate (not
+                                 registered); otherwise the status b200_ndt_pairs_align reports for these clouds */
+} b200_loop_result;
+
+/* detectLoopClosureDistance for Q queries (cur[q] = the keyframe that was the newest): the keyframe j < cur[q] nearest to it
+ * (squared distance summed x, y, z in fp32, strictly below search_radius^2 = (float)((double)r * r)) with
+ * |time_j - time_cur| > time_gap; ties to the lower index; pre[q] = -1 (sqdist 0) without one.  The loopIndexContainer check
+ * stays with the caller: detect, filter, then b200_loop_close with explicit pre. */
+int32_t b200_loop_detect(b200_keyframes* h, const int64_t* cur, int64_t Q, const b200_loop_params* prm, int64_t* pre, float* sqdist);
+/* parity probe: loopFindNearKeyframes(key, search_num) = keyframes key-search_num .. key+search_num (clipped) moved by their
+ * poses, appended in index order, VoxelGrid(leaf), min points 0: out_xyzi 4 floats per point in ascending leaf order (at most
+ * max_out written, may be NULL), *n_out = points */
+int32_t b200_loop_submap(b200_keyframes* h, int64_t key, int32_t search_num, float leaf, float* out_xyzi, int64_t max_out, int64_t* n_out);
+/* performLoopClosure up to the fitness gate for Q queries: pre NULL = detect by distance (b200_loop_detect), otherwise pre[q]
+ * is query q's partner (detectLoopClosureExternal; -1 = none).  Source = loopFindNearKeyframes(cur, 0), target =
+ * loopFindNearKeyframes(pre, search_num), size gates, then align(identity) and getFitnessScore(max_range): reg is the record
+ * b200_ndt_pairs_align gives the same two clouds.  comm may be NULL; with a communicator every rank holds the same store and
+ * passes the same arguments, rank r assembles and registers the queries q = r (mod N) and every rank returns all Q results.
+ * The store and the pairs handle must be on the same device. */
+int32_t b200_loop_close(b200_comm* comm, b200_ndt_pairs* ndt, b200_keyframes* h, const int64_t* cur, const int64_t* pre, int64_t Q,
+                        const b200_loop_params* prm, b200_loop_result* results);
+
 /* ------------------------------------------------------------------------- *
  * B3 (alternative) — Generalized ICP.  Replaces pclomp::GeneralizedIterativeClosestPoint<PointT, PointT>
  * (pointcloud_match/ndt_omp/include/pclomp/gicp_omp.h:60-135, gicp_omp_impl.hpp), the registration object

@@ -63,6 +63,19 @@ class RelocCandidate(C.Structure):
     _fields_ = [("hypothesis", C.c_int64), ("initial_score", C.c_double), ("refined", NdtPairResult)]
 
 
+class LoopParams(C.Structure):
+    """b200_loop_params: performLoopClosure's settings (historyKeyframeSearchRadius / TimeDiff / Num, downSizeFilterICP leaf,
+    the 300 / 1000 size gates, getFitnessScore's max_range)."""
+    _fields_ = [("search_radius", C.c_float), ("time_gap", C.c_double), ("search_num", C.c_int32), ("leaf", C.c_float),
+                ("min_source_points", C.c_int32), ("min_target_points", C.c_int32), ("max_range", C.c_double)]
+
+
+class LoopResult(C.Structure):
+    """b200_loop_result: the query, its partner (-1 = none), the downsampled sizes and the pair record."""
+    _fields_ = [("cur", C.c_int64), ("pre", C.c_int64), ("pre_sqdist", C.c_float), ("n_source", C.c_int32), ("n_target", C.c_int32),
+                ("reg", NdtPairResult)]
+
+
 class GicpParams(C.Structure):
     _fields_ = [("k_correspondences", C.c_int32), ("gicp_epsilon", C.c_double), ("rotation_epsilon", C.c_double),
                 ("transformation_epsilon", C.c_double), ("corr_dist_threshold", C.c_double), ("max_iterations", C.c_int32),
@@ -183,6 +196,16 @@ def lib():
         L.b200_ndt_pairs_align.argtypes = [vp, vp, vp, vp, vp, vp, i64, i64, vp, C.c_double, vp]
         L.b200_ndt_pairs_leaves.restype = i64
         L.b200_ndt_pairs_leaves.argtypes = [vp, i64, i64, vp, vp, vp, vp, vp]
+    if hasattr(L, "b200_keyframes_create"):  # absent from builds older than the device keyframe store (B200REG_LIB A/B timing)
+        L.b200_keyframes_create.argtypes = [i32, C.POINTER(vp)]
+        L.b200_keyframes_destroy.argtypes = [vp]
+        L.b200_keyframes_add.argtypes = [vp, vp, i64, i64, vp, C.c_double, vp]
+        L.b200_keyframes_set_poses.argtypes = [vp, i64, i64, vp]
+        L.b200_keyframes_count.restype = i64
+        L.b200_keyframes_count.argtypes = [vp]
+        L.b200_loop_detect.argtypes = [vp, vp, i64, C.POINTER(LoopParams), vp, vp]
+        L.b200_loop_submap.argtypes = [vp, i64, i32, C.c_float, vp, i64, vp]
+        L.b200_loop_close.argtypes = [vp, vp, vp, vp, vp, i64, C.POINTER(LoopParams), vp]
     L.b200_downsampler_create.argtypes = [i32, C.POINTER(vp)]
     L.b200_downsampler_destroy.argtypes = [vp]
     L.b200_voxel_downsample.argtypes = [vp, vp, i64, i64, C.c_float, i32, vp, vp, i64, vp]
@@ -772,6 +795,100 @@ class NdtPairBatch:
         icov = np.empty((n, 3, 3))
         lib().b200_ndt_pairs_leaves(self.h, p, n, _p(ids), _p(npts), _p(mean), _p(cov), _p(icov))
         return dict(ids=ids, npts=npts, mean=mean, cov=cov, icov=icov)
+
+
+    def close_loops(self, store: "KeyframeStore", cur, pre=None, comm=None, **loop):
+        """performLoopClosure up to the fitness gate for the query keyframes `cur` (b200_loop_close): pre None = detect the
+        partners by distance, otherwise pre[q] is query q's partner (-1 = none).  Keyword arguments are the LoopParams fields
+        (KeyframeStore.params).  Returns the align() dict of the pair records plus cur, pre, pre_sqdist, n_source, n_target
+        and the raw LoopResult records under "loop_records"."""
+        cur = np.ascontiguousarray(cur, dtype=np.int64).reshape(-1)
+        Q = len(cur)
+        prm = KeyframeStore.params(**loop)
+        pv = None if pre is None else np.ascontiguousarray(pre, dtype=np.int64).reshape(-1)
+        if pv is not None and len(pv) != Q:
+            raise ValueError("one partner per query")
+        res = (LoopResult * max(Q, 1))()
+        _check(lib().b200_loop_close(comm.h if comm is not None else None, self.h, store.h, _p(cur), None if pv is None else _p(pv), Q,
+                                     C.byref(prm), res))
+        regs = (NdtPairResult * max(Q, 1))()
+        for q in range(Q):
+            regs[q] = res[q].reg
+        out = self.unpack(regs, Q)
+        out["loop_records"] = res
+        out["cur"] = np.array([r.cur for r in res[:Q]], np.int64)
+        out["pre"] = np.array([r.pre for r in res[:Q]], np.int64)
+        out["pre_sqdist"] = np.array([r.pre_sqdist for r in res[:Q]], np.float32)
+        out["n_source"] = np.array([r.n_source for r in res[:Q]], np.int32)
+        out["n_target"] = np.array([r.n_target for r in res[:Q]], np.int32)
+        return out
+
+
+class KeyframeStore:
+    """The keyframes of a session on the device (b200_keyframes_*): one cloud per keyframe in the lidar frame (x, y, z,
+    intensity; LIO-SAM's corner cloud followed by its surf cloud), its pose (x, y, z, roll, pitch, yaw) and its time (s).
+    Loop candidates are detected and submaps assembled from it without the clouds crossing PCIe again."""
+
+    _DEFAULTS = dict(search_radius=15.0, time_gap=30.0, search_num=25, leaf=0.4, min_source_points=300, min_target_points=1000,
+                     max_range=1.7976931348623157e308)
+
+    def __init__(self, device=0):
+        self.device = device
+        self.h = C.c_void_p()
+        _check(lib().b200_keyframes_create(device, C.byref(self.h)))
+
+    def close(self):
+        if getattr(self, "h", None):
+            try:
+                lib().b200_keyframes_destroy(self.h)
+            except TypeError:  # interpreter shutdown: module globals are already torn down
+                pass
+            self.h = None
+
+    __del__ = close
+
+    @classmethod
+    def params(cls, **kw) -> LoopParams:
+        unknown = set(kw) - set(cls._DEFAULTS)
+        if unknown:
+            raise TypeError(f"unknown loop parameter(s): {sorted(unknown)}")
+        v = dict(cls._DEFAULTS, **kw)
+        return LoopParams(v["search_radius"], v["time_gap"], v["search_num"], v["leaf"], v["min_source_points"], v["min_target_points"],
+                          v["max_range"])
+
+    def __len__(self):
+        return int(lib().b200_keyframes_count(self.h))
+
+    def add(self, cloud_xyzi, pose6, time) -> int:
+        """Appends a keyframe ([n, 3] or [n, 4] float32, lidar frame); returns its index."""
+        c = np.asarray(cloud_xyzi, dtype=np.float32)
+        c = np.ascontiguousarray(c.reshape(-1, c.shape[-1] if c.ndim == 2 else 4))
+        pose = np.ascontiguousarray(pose6, dtype=np.float32).reshape(6)
+        key = C.c_int64()
+        _check(lib().b200_keyframes_add(self.h, _p(c) if len(c) else None, len(c), c.strides[0] if c.ndim == 2 else 16, _p(pose),
+                                        float(time), C.byref(key)))
+        return key.value
+
+    def set_poses(self, first, poses6):
+        """correctPoses(): the poses of keyframes first .. first + len(poses6) - 1."""
+        p = np.ascontiguousarray(poses6, dtype=np.float32).reshape(-1, 6)
+        _check(lib().b200_keyframes_set_poses(self.h, first, len(p), _p(p)))
+
+    def detect(self, cur, **loop):
+        """detectLoopClosureDistance for the query keyframes `cur`: (pre int64 [Q], squared distance float32 [Q])."""
+        cur = np.ascontiguousarray(cur, dtype=np.int64).reshape(-1)
+        pre = np.empty(len(cur), np.int64)
+        d2 = np.empty(len(cur), np.float32)
+        _check(lib().b200_loop_detect(self.h, _p(cur), len(cur), C.byref(self.params(**loop)), _p(pre), _p(d2)))
+        return pre, d2
+
+    def submap(self, key, search_num, leaf) -> "np.ndarray":
+        """loopFindNearKeyframes(key, search_num) downsampled with leaf: float32 [m, 4] (x, y, z, intensity)."""
+        n = C.c_int64()
+        _check(lib().b200_loop_submap(self.h, key, search_num, leaf, None, 0, C.byref(n)))
+        out = np.empty((max(n.value, 1), 4), np.float32)
+        _check(lib().b200_loop_submap(self.h, key, search_num, leaf, _p(out), n.value, C.byref(n)))
+        return out[: n.value]
 
 
 class Communicator:

@@ -1,0 +1,48 @@
+// b200reg — the keyframe store's side of the loop closure (loop.cu), as the pair registration (ndt.cu) drives it.
+#pragma once
+#include "common.cuh"
+
+#include <vector>
+
+namespace b200 {
+namespace ndt {
+// Min / max of the finite points of segments: segment y = off[y] .. off[y+1]-1 of pts, into mm[6 y .. 6 y + 6) (ordered ints:
+// min x y z, max x y z).  Defined in ndt.cu (the NDT target build); the submaps' VoxelGrid uses them too.
+__global__ void k_ndt_minmax_init(int* mm, int np);
+__global__ void k_ndt_minmax(const float4* __restrict__ pts, const int64_t* __restrict__ off, int* __restrict__ mm);
+}  // namespace ndt
+
+namespace loop {
+
+struct Seg {  // loopFindNearKeyframes(key, num)
+    int64_t key;
+    int32_t num;
+};
+struct GatherEntry {  // gather(): count points from pts[src ..) to dst[which][dst ..)
+    int64_t src, count, dst;
+    int64_t which;
+};
+struct Submaps {
+    const float4* pts = nullptr;       // device: the downsampled points of every segment, segment after segment
+    std::vector<int64_t> first, count; // per segment: its points are pts[first .. first + count)
+    std::vector<int32_t> status;       // per segment: B200_OK, or the code b200_voxel_downsample returns for this cloud
+    int64_t done = 0;                  // segments assembled: a prefix of whole groups
+};
+
+int32_t check_params(const b200_loop_params* prm);
+// keys[0 .. n) in [0, count); with allow_none, -1 too
+int32_t check_keys(const b200_keyframes* h, const int64_t* keys, int64_t n, bool allow_none);
+int32_t device_of(const b200_keyframes* h);
+// points of loopFindNearKeyframes(key, num) before the downsample
+int64_t raw_size(const b200_keyframes* h, int64_t key, int32_t num);
+// detectLoopClosureDistance for Q queries on stream s (one read-back)
+int32_t detect(b200_keyframes* h, cudaStream_t s, const int64_t* cur, int64_t Q, const b200_loop_params& prm, int64_t* pre, float* sqdist);
+// Assembles and VoxelGrid-downsamples segs[0 .. nseg) on stream s (two read-backs: min / max, run ranges).  Segments come in
+// groups of `group`; the call ends after the last whole group whose leaves still fit the 64-bit sort key (at least one group).
+// Out-of-range raw sizes are the caller's: the raw points of all segments must stay below 2^31.
+int32_t submaps(b200_keyframes* h, cudaStream_t s, const Seg* segs, int64_t nseg, int64_t group, float leaf, Submaps& out);
+// e[0 .. n) from pts into dst0 / dst1 as (x, y, z, 0) records, one launch on stream s
+int32_t gather(b200_keyframes* h, cudaStream_t s, const float4* pts, const GatherEntry* e, int64_t n, float4* dst0, float4* dst1);
+
+}  // namespace loop
+}  // namespace b200

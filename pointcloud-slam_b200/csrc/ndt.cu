@@ -16,6 +16,7 @@
 //             + computeStepLengthMT) by one evaluation.  The host only polls a done flag every few launches.
 //             gridDim.y indexes independent alignments (hypotheses), each with its own control block.
 #include "ndt.cuh"
+#include "loop.cuh"
 
 #include <cub/cub.cuh>
 
@@ -2197,7 +2198,11 @@ struct b200_ndt_pairs {
         b200_ndt_pair_result* results;
     };
     int32_t chunk(const Call& c, const int64_t* ids, int64_t np, int64_t cell_limit, int64_t& used);
+    int32_t build(const int64_t* ids, int64_t np, const int64_t* toff, const int64_t* soff, const float* guesses16, double max_range,
+                  b200_ndt_pair_result* results, int64_t cell_limit, int64_t& used);
     int32_t local(const Call& c, int64_t P, int64_t first, int64_t step);
+    int32_t close_local(b200_keyframes* kf, const int64_t* cur, const int64_t* pre, int64_t Q, const b200_loop_params& prm,
+                        b200_loop_result* results, int64_t first, int64_t step);
     void destroy() {
         cudaSetDevice(k.device);
         if (k.stream) cudaStreamSynchronize(k.stream);
@@ -2208,23 +2213,16 @@ struct b200_ndt_pairs {
     }
 };
 
-// Builds, aligns and scores pairs ids[0 .. np-1] (all with a non-empty source and target); `used` = how many of them fit the
-// 32-bit key space / memory bound and were done (at least one).
+// Fills the chunk of pairs ids[0 .. np-1] from the caller's host clouds (one upload of every cloud) and builds it.
 int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int64_t cell_limit, int64_t& used) {
-    using namespace ndt;
     Ndt& K = k;
     cudaStream_t s = K.stream;
     std::vector<int64_t> toff(np + 1, 0), soff(np + 1, 0);
-    int64_t max_tn = 1, max_sn = 1;
     for (int64_t j = 0; j < np; ++j) {
-        const int64_t tn = c.tgt_off[ids[j] + 1] - c.tgt_off[ids[j]], sn = c.src_off[ids[j] + 1] - c.src_off[ids[j]];
-        toff[j + 1] = toff[j] + tn;
-        soff[j + 1] = soff[j] + sn;
-        max_tn = std::max(max_tn, tn);
-        max_sn = std::max(max_sn, sn);
+        toff[j + 1] = toff[j] + (c.tgt_off[ids[j] + 1] - c.tgt_off[ids[j]]);
+        soff[j + 1] = soff[j] + (c.src_off[ids[j] + 1] - c.src_off[ids[j]]);
     }
     const int64_t nt = toff[np], ns = soff[np];
-    // one upload of every cloud of the chunk
     CUDA_TRY(K.h_stage.reserve((size_t)(nt + ns)));
     pack_ranges(c.tgt_xyz, c.stride, c.tgt_off, ids, np, toff.data(), K.h_stage.p);
     pack_ranges(c.src_xyz, c.stride, c.src_off, ids, np, soff.data(), K.h_stage.p + nt);
@@ -2232,10 +2230,27 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     CUDA_TRY(K.d_src_raw.reserve((size_t)ns));
     CUDA_TRY(cudaMemcpyAsync(K.d_tgt.p, K.h_stage.p, (size_t)nt * sizeof(float4), cudaMemcpyHostToDevice, s));
     CUDA_TRY(cudaMemcpyAsync(K.d_src_raw.p, K.h_stage.p + nt, (size_t)ns * sizeof(float4), cudaMemcpyHostToDevice, s));
+    return build(ids, np, toff.data(), soff.data(), c.guesses16, c.max_range, c.results, cell_limit, used);
+}
+
+// Builds, aligns and scores pairs ids[0 .. np-1], whose clouds are already in d_tgt / d_src_raw (x, y, z, 0) at the
+// chunk-local offsets toff / soff (all non-empty; filled from host clouds by chunk() or on the device by the loop closure).
+// Pair j's guess is guesses16[16 ids[j]] (NULL = identity), its record results[ids[j]].  `used` = how many of them fit the
+// 32-bit key space / memory bound and were done (at least one).
+int32_t b200_ndt_pairs::build(const int64_t* ids, int64_t np, const int64_t* toff, const int64_t* soff, const float* guesses16, double max_range,
+                              b200_ndt_pair_result* results, int64_t cell_limit, int64_t& used) {
+    using namespace ndt;
+    Ndt& K = k;
+    cudaStream_t s = K.stream;
+    int64_t max_tn = 1, max_sn = 1;
+    for (int64_t j = 0; j < np; ++j) {
+        max_tn = std::max(max_tn, toff[j + 1] - toff[j]);
+        max_sn = std::max(max_sn, soff[j + 1] - soff[j]);
+    }
     CUDA_TRY(K.h_off.reserve(2 * (size_t)(np + 1)));
     CUDA_TRY(K.d_off.reserve(2 * (size_t)(np + 1)));
-    memcpy(K.h_off.p, toff.data(), (np + 1) * sizeof(int64_t));
-    memcpy(K.h_off.p + np + 1, soff.data(), (np + 1) * sizeof(int64_t));
+    memcpy(K.h_off.p, toff, (np + 1) * sizeof(int64_t));
+    memcpy(K.h_off.p + np + 1, soff, (np + 1) * sizeof(int64_t));
     CUDA_TRY(cudaMemcpyAsync(K.d_off.p, K.h_off.p, 2 * (np + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, s));
     const int64_t* d_soff = K.d_off.p + np + 1;
     // per-target min / max, read back once for the whole chunk
@@ -2252,7 +2267,7 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
         const int32_t st = grid_from_minmax(K.h_mm.p + 6 * j, K.prm.resolution, g.gd, nc);
         if (st) {
             memset(&g, 0, sizeof g);
-            c.results[ids[j]].status = st;
+            results[ids[j]].status = st;
             continue;
         }
         if (cells + nc > cell_limit && j > 0) { used = j; break; }
@@ -2323,7 +2338,7 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
         n_d2 += sn;
         max_live_sn = std::max(max_live_sn, sn);
         float* G = K.h_poses.p + a * 16;
-        if (c.guesses16) memcpy(G, c.guesses16 + ids[j] * 16, 16 * sizeof(float));
+        if (guesses16) memcpy(G, guesses16 + ids[j] * 16, 16 * sizeof(float));
         else for (int q = 0; q < 16; ++q) G[q] = (q % 5 == 0) ? 1.f : 0.f;
         ++a;
     }
@@ -2346,7 +2361,7 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     CUDA_TRY(K.d_fit.reserve((size_t)n_d2));
     CUDA_TRY(d_fitsum.reserve(2 * (size_t)n_live)); CUDA_TRY(h_fitsum.reserve(2 * (size_t)n_live));
     k_ndt_fitness<<<dim3((unsigned)((max_live_sn * 32 + 255) / 256), (unsigned)n_live), 256, 0, s>>>(d_pf.p, K.d_fit.p);
-    k_ndt_fitness_reduce<<<(unsigned)n_live, 256, 0, s>>>(d_pf.p, K.d_fit.p, c.max_range, d_fitsum.p);
+    k_ndt_fitness_reduce<<<(unsigned)n_live, 256, 0, s>>>(d_pf.p, K.d_fit.p, max_range, d_fitsum.p);
     LAUNCH_COUNT(3);
     CUDA_TRY(cudaMemcpyAsync(K.h_ctl.p, K.d_ctl.p, n_live * sizeof(Ctl), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaMemcpyAsync(h_fitsum.p, d_fitsum.p, 2 * n_live * sizeof(double), cudaMemcpyDeviceToHost, s));
@@ -2354,7 +2369,7 @@ int32_t b200_ndt_pairs::chunk(const Call& c, const int64_t* ids, int64_t np, int
     CUDA_TRY(cudaGetLastError());
     for (int64_t a = 0; a < n_live; ++a) {
         const Ctl& ct = K.h_ctl.p[a];
-        b200_ndt_pair_result& r = c.results[ids[live[a]]];
+        b200_ndt_pair_result& r = results[ids[live[a]]];
         fill_result(ct, r.final16, &r.ndt, 0.f);
         r.status = !ct.done ? B200_ERR_CUDA : ct.converged ? B200_OK : B200_NOT_CONVERGED;
         const double S = h_fitsum.p[2 * a], Cn = h_fitsum.p[2 * a + 1];
@@ -2397,6 +2412,98 @@ int32_t b200_ndt_pairs::local(const Call& c, int64_t P, int64_t first, int64_t s
         if (rc) return rc;
         i += (size_t)std::max<int64_t>(used, 1);
     }
+    return B200_OK;
+}
+
+// The loop queries first, first + step, ... < Q: partners (one read-back when detected), then chunks of the queries that
+// have one, budgeted by their raw submap sizes.
+int32_t b200_ndt_pairs::close_local(b200_keyframes* kf, const int64_t* cur, const int64_t* pre, int64_t Q, const b200_loop_params& prm,
+                                    b200_loop_result* results, int64_t first, int64_t step) {
+    constexpr int64_t kLoopRawBytes = 80;  // device bytes per raw submap point (assembled cloud, sort keys and indices, runs, centroids)
+    Ndt& K = k;
+    std::vector<int64_t> pv(Q);
+    std::vector<float> d2(Q, 0.f);
+    if (pre) memcpy(pv.data(), pre, Q * sizeof(int64_t));
+    else if (const int32_t rc = loop::detect(kf, K.stream, cur, Q, prm, pv.data(), d2.data())) return rc;
+    std::vector<b200_ndt_pair_result> reg(Q);
+    std::vector<int64_t> cand;
+    for (int64_t q = first; q < Q; q += step) {
+        b200_loop_result& r = results[q];
+        memset(&r, 0, sizeof r);
+        r.cur = cur[q];
+        r.pre = pv[q];
+        r.pre_sqdist = d2[q];
+        memset(&reg[q], 0, sizeof reg[q]);
+        reg[q].status = B200_NO_EFFECTIVE_POINTS;
+        if (pv[q] >= 0) cand.push_back(q);
+    }
+    size_t free_b = 0, total_b = 0;
+    CUDA_TRY(cudaMemGetInfo(&free_b, &total_b));
+    const int64_t budget = (int64_t)(0.6 * (double)free_b);
+    const int64_t cell_limit = std::min<int64_t>(((int64_t)1 << 32) - 2, std::max<int64_t>(budget / 4 / 8, (int64_t)1 << 30));
+    const int64_t max_q = std::min<int64_t>(pairs_chunk_max(), 32767);  // two segments per query in one launch row each
+    std::vector<loop::Seg> segs;
+    std::vector<loop::GatherEntry> ge;
+    std::vector<int64_t> kept, ids, toff, soff;
+    for (size_t i = 0; i < cand.size();) {
+        size_t e = i;
+        int64_t bytes = 0, nraw = 0;
+        while (e < cand.size() && (int64_t)(e - i) < max_q) {
+            const int64_t q = cand[e];
+            const int64_t tn = loop::raw_size(kf, pv[q], prm.search_num), sn = loop::raw_size(kf, cur[q], 0);
+            const int64_t add = (tn + sn) * kLoopRawBytes + tn * kPairTgtBytes + sn * kPairSrcBytes;
+            if (e > i && (bytes + add > budget * 3 / 4 || nraw + tn + sn > (int64_t)0x7fffff00)) break;
+            if (tn + sn > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_RANGE, "loop submap larger than 2^31 points");
+            bytes += add; nraw += tn + sn;
+            ++e;
+        }
+        segs.clear();
+        for (size_t j = i; j < e; ++j) {
+            segs.push_back(loop::Seg{pv[cand[j]], prm.search_num});
+            segs.push_back(loop::Seg{cur[cand[j]], 0});
+        }
+        loop::Submaps sm;
+        int32_t rc = loop::submaps(kf, K.stream, segs.data(), (int64_t)segs.size(), 2, prm.leaf, sm);
+        if (rc) return rc;
+        const int64_t nq = sm.done / 2;
+        // the size gates of performLoopClosure, then the checks b200_ndt_pairs_align makes of a pair's clouds
+        kept.clear();
+        for (int64_t j = 0; j < nq; ++j) {
+            const int64_t q = cand[i + j];
+            b200_loop_result& r = results[q];
+            r.n_target = (int32_t)sm.count[2 * j];
+            r.n_source = (int32_t)sm.count[2 * j + 1];
+            if (sm.status[2 * j] || sm.status[2 * j + 1]) reg[q].status = sm.status[2 * j] ? sm.status[2 * j] : sm.status[2 * j + 1];
+            else if (r.n_source < prm.min_source_points || r.n_target < prm.min_target_points) continue;
+            else if (r.n_target < 1 || r.n_source < 1) reg[q].status = B200_ERR_ARG;
+            else kept.push_back(j);
+        }
+        while (!kept.empty()) {
+            const int64_t np = (int64_t)kept.size();
+            ids.resize(np);
+            toff.assign(np + 1, 0);
+            soff.assign(np + 1, 0);
+            ge.clear();
+            for (int64_t a = 0; a < np; ++a) {
+                const int64_t j = kept[a];
+                ids[a] = cand[i + j];
+                ge.push_back(loop::GatherEntry{sm.first[2 * j], sm.count[2 * j], toff[a], 0});
+                ge.push_back(loop::GatherEntry{sm.first[2 * j + 1], sm.count[2 * j + 1], soff[a], 1});
+                toff[a + 1] = toff[a] + sm.count[2 * j];
+                soff[a + 1] = soff[a] + sm.count[2 * j + 1];
+            }
+            CUDA_TRY(K.d_tgt.reserve((size_t)toff[np]));
+            CUDA_TRY(K.d_src_raw.reserve((size_t)soff[np]));
+            rc = loop::gather(kf, K.stream, sm.pts, ge.data(), (int64_t)ge.size(), K.d_tgt.p, K.d_src_raw.p);
+            if (rc) return rc;
+            int64_t used = 0;
+            rc = build(ids.data(), np, toff.data(), soff.data(), nullptr, prm.max_range, reg.data(), cell_limit, used);
+            if (rc) return rc;
+            kept.erase(kept.begin(), kept.begin() + std::max<int64_t>(used, 1));
+        }
+        i += (size_t)nq;
+    }
+    for (int64_t q = first; q < Q; q += step) results[q].reg = reg[q];
     return B200_OK;
 }
 
@@ -2955,10 +3062,45 @@ int32_t b200_ndt_pairs_destroy(b200_ndt_pairs* h) {
     return B200_OK;
 }
 
+// The records of a sharded pair call travel in ONE ncclAllGather of fixed-size slots: rank r fills the records p = r (mod R)
+// of its slot (ceil(P / R) of `rec` bytes each) behind its call status, so all ranks return the same code and the same P
+// records, and a rank that failed locally still takes part in the collective.  The int32 status of a record sits at
+// status_off; a failed rank's records carry its code there.
+static int32_t pairs_exchange(b200_comm* comm, b200_ndt_pairs* h, int32_t rc_local, const std::string& err_local, int64_t P, uint8_t* records,
+                              size_t rec, size_t status_off) {
+    Ndt& K = h->k;
+    const int R = comm->nranks, me = comm->rank;
+    const int64_t per = (P + R - 1) / R;
+    const size_t slot = 8 + (size_t)per * rec;
+    uint8_t* hs = h->h_xchg.p;
+    memset(hs, 0, 8);
+    memcpy(hs, &rc_local, sizeof(int32_t));
+    for (int64_t i = 0, p = me; p < P; ++i, p += R) memcpy(hs + 8 + i * rec, records + p * rec, rec);
+    CUDA_TRY(cudaMemcpyAsync(h->d_xchg.p, hs, slot, cudaMemcpyHostToDevice, K.stream));
+    NCCL_TRY(comm, comm->AllGather(h->d_xchg.p, h->d_xchg.p + slot, slot, ncclChar, comm->comm, K.stream));
+    CUDA_TRY(cudaMemcpyAsync(hs + slot, h->d_xchg.p + slot, slot * R, cudaMemcpyDeviceToHost, K.stream));
+    CUDA_TRY(cudaStreamSynchronize(K.stream));
+    int32_t rc = B200_OK;
+    int bad = -1;
+    for (int q = 0; q < R; ++q) {
+        const uint8_t* b = hs + slot * (q + 1);
+        int32_t sq;
+        memcpy(&sq, b, sizeof sq);
+        if (sq && rc == B200_OK) { rc = sq; bad = q; }
+        for (int64_t i = 0, p = q; p < P; ++i, p += R) {
+            memcpy(records + p * rec, b + 8 + i * rec, rec);
+            if (sq) memcpy(records + p * rec + status_off, &sq, sizeof sq);
+        }
+    }
+    if (rc) {
+        if (bad == me) g_last_error = err_local;
+        else fail(rc, ("NDT pair registration failed on rank " + std::to_string(bad)).c_str(), __FILE__, __LINE__);
+    }
+    return rc;
+}
+
 /* P independent registrations (loop-closure candidates): see include/b200reg.h.  With a communicator of N ranks, rank r
- * registers the pairs p = r (mod N); the results and every rank's call status travel in ONE ncclAllGather of fixed-size
- * slots (ceil(P / N) records each), so all ranks return the same code and the same P results, and a rank that failed
- * locally still takes part in the collective. */
+ * registers the pairs p = r (mod N); the results and every rank's call status travel in one ncclAllGather (pairs_exchange). */
 int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* src_xyz, const int64_t* src_off, const float* tgt_xyz,
                              const int64_t* tgt_off, int64_t stride_bytes, int64_t P, const float* guesses16, double max_range,
                              b200_ndt_pair_result* results) {
@@ -2981,31 +3123,8 @@ int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* sr
     const std::string err_local = rc_local ? g_last_error : std::string();
     if (R == 1 && rc_local) return rc_local;
     if (R > 1) {
-        uint8_t* hs = h->h_xchg.p;
-        memset(hs, 0, 8);
-        memcpy(hs, &rc_local, sizeof(int32_t));
-        for (int64_t i = 0, p = me; p < P; ++i, p += R) memcpy(hs + 8 + i * rec, &results[p], rec);
-        CUDA_TRY(cudaMemcpyAsync(h->d_xchg.p, hs, slot, cudaMemcpyHostToDevice, K.stream));
-        NCCL_TRY(comm, comm->AllGather(h->d_xchg.p, h->d_xchg.p + slot, slot, ncclChar, comm->comm, K.stream));
-        CUDA_TRY(cudaMemcpyAsync(hs + slot, h->d_xchg.p + slot, slot * R, cudaMemcpyDeviceToHost, K.stream));
-        CUDA_TRY(cudaStreamSynchronize(K.stream));
-        int32_t rc = B200_OK;
-        int bad = -1;
-        for (int q = 0; q < R; ++q) {
-            const uint8_t* b = hs + slot * (q + 1);
-            int32_t sq;
-            memcpy(&sq, b, sizeof sq);
-            if (sq && rc == B200_OK) { rc = sq; bad = q; }
-            for (int64_t i = 0, p = q; p < P; ++i, p += R) {
-                memcpy(&results[p], b + 8 + i * rec, rec);
-                if (sq) results[p].status = sq;
-            }
-        }
-        if (rc) {
-            if (bad == me) g_last_error = err_local;
-            else fail(rc, ("NDT pair registration failed on rank " + std::to_string(bad)).c_str(), __FILE__, __LINE__);
-            return rc;
-        }
+        const int32_t rc = pairs_exchange(comm, h, rc_local, err_local, P, (uint8_t*)results, rec, offsetof(b200_ndt_pair_result, status));
+        if (rc) return rc;
     }
     CUDA_TRY(cudaEventRecord(K.ev1, K.stream));
     CUDA_TRY(cudaEventSynchronize(K.ev1));
@@ -3013,6 +3132,44 @@ int32_t b200_ndt_pairs_align(b200_comm* comm, b200_ndt_pairs* h, const float* sr
     cudaEventElapsedTime(&ms, K.ev0, K.ev1);
     K.last_ms = ms;
     for (int64_t p = 0; p < P; ++p) results[p].ndt.gpu_ms = ms;
+    return B200_OK;
+}
+
+/* performLoopClosure up to the fitness gate (see include/b200reg.h).  Rank r takes the queries q = r (mod N) that have a
+ * partner; per chunk of them: their submaps assembled and downsampled on the device (loop.cu), the size gates on the
+ * downsampled sizes, the survivors gathered into the pair buffers and registered by b200_ndt_pairs::build - so a record is
+ * the one b200_ndt_pairs_align gives the same clouds.  The records travel in one ncclAllGather (pairs_exchange). */
+int32_t b200_loop_close(b200_comm* comm, b200_ndt_pairs* ndt, b200_keyframes* kf, const int64_t* cur, const int64_t* pre, int64_t Q,
+                        const b200_loop_params* prm, b200_loop_result* results) {
+    if (!ndt || !kf || !cur || !prm || !results || Q < 1 || Q > (int64_t)1 << 26) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (const int32_t rc = loop::check_params(prm)) return rc;
+    if (const int32_t rc = loop::check_keys(kf, cur, Q, false)) return rc;
+    if (pre)
+        if (const int32_t rc = loop::check_keys(kf, pre, Q, true)) return rc;
+    Ndt& K = ndt->k;
+    if (loop::device_of(kf) != K.device) B200_FAIL(B200_ERR_ARG, "keyframe store and pairs handle are on different devices");
+    CUDA_SET_DEVICE(K.device);
+    const int R = comm && comm->nranks > 1 ? comm->nranks : 1, me = R > 1 ? comm->rank : 0;
+    const int64_t per = (Q + R - 1) / R;
+    const size_t rec = sizeof(b200_loop_result), slot = 8 + (size_t)per * rec;
+    if (R > 1) {  // before any work: past this point every rank reaches the collective
+        CUDA_TRY(ndt->h_xchg.reserve(slot * (R + 1)));
+        CUDA_TRY(ndt->d_xchg.reserve(slot * (R + 1)));
+    }
+    CUDA_TRY(cudaEventRecord(K.ev0, K.stream));
+    const int32_t rc_local = ndt->close_local(kf, cur, pre, Q, *prm, results, me, R);
+    const std::string err_local = rc_local ? g_last_error : std::string();
+    if (R == 1 && rc_local) return rc_local;
+    if (R > 1) {
+        const int32_t rc = pairs_exchange(comm, ndt, rc_local, err_local, Q, (uint8_t*)results, rec, offsetof(b200_loop_result, reg.status));
+        if (rc) return rc;
+    }
+    CUDA_TRY(cudaEventRecord(K.ev1, K.stream));
+    CUDA_TRY(cudaEventSynchronize(K.ev1));
+    float ms = 0.f;
+    cudaEventElapsedTime(&ms, K.ev0, K.ev1);
+    K.last_ms = ms;
+    for (int64_t q = 0; q < Q; ++q) results[q].reg.ndt.gpu_ms = ms;
     return B200_OK;
 }
 

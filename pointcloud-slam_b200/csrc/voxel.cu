@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "comm.cuh"
+#include "voxel.cuh"
 
 namespace b200 {
 namespace vox {
@@ -63,11 +64,6 @@ __global__ void k_minmax(const float4* __restrict__ pts, int64_t n, int* __restr
     }
 }
 
-struct Grid {
-    long long min_b[3], div_b[3];
-    float inv_leaf;
-};
-
 // leaf index of every point (voxel_grid_large.cpp:163-168), 64-bit; non-finite points get the sentinel and sort last
 __global__ void k_keys(const float4* __restrict__ pts, int n, Grid g, unsigned long long sentinel, unsigned long long* __restrict__ keys,
                        int32_t* __restrict__ vals) {
@@ -85,7 +81,6 @@ __global__ void k_keys(const float4* __restrict__ pts, int n, Grid g, unsigned l
     vals[i] = i;
 }
 
-// one thread per leaf: fp32 sums in input order, divided by the count (pcl::CentroidPoint); compacts on min_points
 __global__ void k_centroids(const float4* __restrict__ pts, const int32_t* __restrict__ sorted_idx, const unsigned long long* __restrict__ uniq,
                             const int32_t* __restrict__ run_off, const int32_t* __restrict__ run_cnt, const int32_t* __restrict__ nruns,
                             unsigned long long sentinel, int min_points, float4* __restrict__ out, int32_t* __restrict__ out_cnt,
@@ -587,6 +582,33 @@ struct b200_downsampler {
     int64_t n_staged = 0;  // undistorted points waiting in d_in
 };
 
+int32_t vox::grid_from_minmax(const int* mm6, float leaf, Grid& g, unsigned long long& cells) {
+    float mn[3], mx[3];
+    for (int k = 0; k < 3; ++k) {
+        int a = mm6[k], b = mm6[3 + k];
+        a = a >= 0 ? a : a ^ 0x7fffffff;
+        b = b >= 0 ? b : b ^ 0x7fffffff;
+        memcpy(&mn[k], &a, 4);
+        memcpy(&mx[k], &b, 4);
+    }
+    cells = 0;
+    if (!(mn[0] <= mx[0])) return B200_OK;
+    g.inv_leaf = 1.0f / leaf;
+    // The product of the extents is taken in integers: the last leaf index is cells - 1 and the sentinel is cells, so a
+    // product rounded in double (above 2^53) can make the max-corner leaf equal the sentinel and drop it.
+    unsigned long long c = 1;
+    for (int k = 0; k < 3; ++k) {
+        const float lo = std::floor(mn[k] * g.inv_leaf), hi = std::floor(mx[k] * g.inv_leaf);
+        if (!(std::fabs(lo) < 4.0e18f && std::fabs(hi) < 4.0e18f)) B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
+        g.min_b[k] = (long long)lo;
+        g.div_b[k] = (long long)hi - g.min_b[k] + 1;
+        if (__builtin_mul_overflow(c, (unsigned long long)g.div_b[k], &c) || c > 9000000000000000000ull)
+            B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
+    }
+    cells = c;
+    return B200_OK;
+}
+
 static int32_t downsample_run(b200_downsampler* d, int64_t n, float leaf, int32_t min_points) {
     using namespace vox;
     cudaStream_t s = d->stream;
@@ -597,29 +619,11 @@ static int32_t downsample_run(b200_downsampler* d, int64_t n, float leaf, int32_
     CUDA_TRY(cudaGetLastError());
     CUDA_TRY(cudaMemcpyAsync(d->h_small.p, mm, 6 * sizeof(int), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
-    float mn[3], mx[3];
-    for (int k = 0; k < 3; ++k) {
-        int a = d->h_small.p[k], b = d->h_small.p[3 + k];
-        a = a >= 0 ? a : a ^ 0x7fffffff;
-        b = b >= 0 ? b : b ^ 0x7fffffff;
-        memcpy(&mn[k], &a, 4);
-        memcpy(&mx[k], &b, 4);
-    }
     d->n_out = 0;
-    if (!(mn[0] <= mx[0])) return B200_OK;  // no finite point: empty output
     Grid g;
-    g.inv_leaf = 1.0f / leaf;
-    // The product of the extents is taken in integers: the last leaf index is cells - 1 and the sentinel is cells, so a
-    // product rounded in double (above 2^53) can make the max-corner leaf equal the sentinel and drop it.
-    unsigned long long cells = 1;
-    for (int k = 0; k < 3; ++k) {
-        const float lo = std::floor(mn[k] * g.inv_leaf), hi = std::floor(mx[k] * g.inv_leaf);
-        if (!(std::fabs(lo) < 4.0e18f && std::fabs(hi) < 4.0e18f)) B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
-        g.min_b[k] = (long long)lo;
-        g.div_b[k] = (long long)hi - g.min_b[k] + 1;
-        if (__builtin_mul_overflow(cells, (unsigned long long)g.div_b[k], &cells) || cells > 9000000000000000000ull)
-            B200_FAIL(B200_ERR_RANGE, "leaf size too small for the cloud extent");
-    }
+    unsigned long long cells = 0;
+    if (const int32_t rc = grid_from_minmax(d->h_small.p, leaf, g, cells)) return rc;
+    if (!cells) return B200_OK;  // no finite point: empty output
     const unsigned long long sentinel = cells;
     int end_bit = 1;
     while (end_bit < 64 && (1ull << end_bit) <= cells) ++end_bit;

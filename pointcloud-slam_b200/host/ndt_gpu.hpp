@@ -163,12 +163,7 @@ class NdtPairBatch {
     void align(const std::vector<const CloudT*>& sources, const std::vector<const CloudT*>& targets, const float* guesses16 = nullptr,
                double max_range = 1.7976931348623157e308) {
         if (sources.size() != targets.size() || sources.empty()) throw std::runtime_error("NdtPairBatch::align: one target per source, at least one pair");
-        if (!h_ || dirty_) {
-            if (h_) b200_ndt_pairs_destroy(h_);
-            h_ = nullptr;
-            check(b200_ndt_pairs_create(&prm_, device_, &h_), "b200_ndt_pairs_create");
-            dirty_ = false;
-        }
+        ensure();
         const size_t P = sources.size();
         std::vector<int64_t> soff(P + 1, 0), toff(P + 1, 0);
         for (size_t p = 0; p < P; ++p) {
@@ -187,6 +182,22 @@ class NdtPairBatch {
         check(b200_ndt_pairs_align(nullptr, h_, src_.data(), soff.data(), tgt_.data(), toff.data(), 12, (int64_t)P, guesses16, max_range, res_.data()),
               "b200_ndt_pairs_align");
     }
+    /// performLoopClosure up to the fitness gate for the query keyframes cur (mapOptmization.cpp: detectLoopClosureDistance or
+    /// detectLoopClosureExternal, loopFindNearKeyframes for both sides, the 300 / 1000 size gates, align(identity),
+    /// getFitnessScore(max_range)), all on the device: pre empty = detect by distance, otherwise pre[q] is query q's partner
+    /// (-1 = none).  Query q's record is then result(q) / hasConverged(q) / getFitnessScore(q) / getFinalTransformation(q);
+    /// loopResult(q) adds the partner and the downsampled sizes.  status(q) == B200_NO_EFFECTIVE_POINTS: not registered.
+    template <class KeyframesT>
+    void closeLoops(KeyframesT& store, const std::vector<int64_t>& cur, const std::vector<int64_t>& pre, const b200_loop_params& prm) {
+        if (cur.empty() || (!pre.empty() && pre.size() != cur.size())) throw std::runtime_error("NdtPairBatch::closeLoops: one partner per query, at least one query");
+        ensure();
+        loop_.assign(cur.size(), b200_loop_result{});
+        check(b200_loop_close(nullptr, h_, store.handle(), cur.data(), pre.empty() ? nullptr : pre.data(), (int64_t)cur.size(), &prm, loop_.data()),
+              "b200_loop_close");
+        res_.resize(cur.size());
+        for (size_t q = 0; q < cur.size(); ++q) res_[q] = loop_[q].reg;
+    }
+    const b200_loop_result& loopResult(size_t q) const { return loop_.at(q); }
     size_t size() const { return res_.size(); }
     int status(size_t p) const { return res_.at(p).status; }
     bool hasConverged(size_t p) const { return res_.at(p).status == B200_OK && res_[p].ndt.converged != 0; }
@@ -197,12 +208,55 @@ class NdtPairBatch {
     const b200_ndt_pair_result& result(size_t p) const { return res_.at(p); }
 
    private:
+    void ensure() {
+        if (!h_ || dirty_) {
+            if (h_) b200_ndt_pairs_destroy(h_);
+            h_ = nullptr;
+            check(b200_ndt_pairs_create(&prm_, device_, &h_), "b200_ndt_pairs_create");
+            dirty_ = false;
+        }
+    }
     int device_;
     b200_ndt_params prm_{};
     b200_ndt_pairs* h_ = nullptr;
     bool dirty_ = true;
     std::vector<float> src_, tgt_;
     std::vector<b200_ndt_pair_result> res_;
+    std::vector<b200_loop_result> loop_;
+};
+
+/// The keyframes of a session on the device: cornerCloudKeyFrames / surfCloudKeyFrames / cloudKeyPoses6D of mapOptmization.cpp.
+/// add() stores the corner cloud followed by the surf cloud (the order loopFindNearKeyframes appends them in) with the
+/// keyframe's pose {x, y, z, roll, pitch, yaw} and time; setPoses() is correctPoses() after a graph optimisation.
+template <class CloudT>
+class KeyframeStore {
+   public:
+    explicit KeyframeStore(int device = 0) { check(b200_keyframes_create(device, &h_), "b200_keyframes_create"); }
+    ~KeyframeStore() { b200_keyframes_destroy(h_); }
+    KeyframeStore(const KeyframeStore&) = delete;
+    KeyframeStore& operator=(const KeyframeStore&) = delete;
+
+    int64_t add(const CloudT& corner, const CloudT& surf, const float pose6[6], double time) {
+        xyzi_.clear();
+        for (const CloudT* c : {&corner, &surf})
+            for (const auto& q : c->points) { xyzi_.push_back(q.x); xyzi_.push_back(q.y); xyzi_.push_back(q.z); xyzi_.push_back(q.intensity); }
+        int64_t key = -1;
+        check(b200_keyframes_add(h_, xyzi_.empty() ? nullptr : xyzi_.data(), (int64_t)xyzi_.size() / 4, 16, pose6, time, &key), "b200_keyframes_add");
+        return key;
+    }
+    void setPoses(int64_t first, int64_t count, const float* poses6) { check(b200_keyframes_set_poses(h_, first, count, poses6), "b200_keyframes_set_poses"); }
+    int64_t size() const { return b200_keyframes_count(h_); }
+    /// detectLoopClosureDistance for the query keyframes cur: pre[q] = -1 without a candidate
+    std::vector<int64_t> detect(const std::vector<int64_t>& cur, const b200_loop_params& prm) {
+        std::vector<int64_t> pre(cur.size(), -1);
+        if (!cur.empty()) check(b200_loop_detect(h_, cur.data(), (int64_t)cur.size(), &prm, pre.data(), nullptr), "b200_loop_detect");
+        return pre;
+    }
+    b200_keyframes* handle() { return h_; }
+
+   private:
+    b200_keyframes* h_ = nullptr;
+    std::vector<float> xyzi_;
 };
 
 }  // namespace b200host

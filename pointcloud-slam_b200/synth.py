@@ -337,3 +337,55 @@ def loam_scene(n_surf_map=60_000, seed: int = SEED, t_true=(0.01, -0.02, 0.6, 3.
     nearc = np.linalg.norm(corner_map - t, axis=1) < 30
     corner = to_body(corner_map[nearc][::corner_stride])
     return dict(corner_map=corner_map, surf_map=surf_map, corner=np.ascontiguousarray(corner), surf=np.ascontiguousarray(surf), t_true=t_true)
+
+
+# ---- loop-closure session: keyframes of a trajectory that revisits its places, stored with accumulated drift ----
+def pose6_matrix(p6) -> np.ndarray:
+    """PointTypePose (x, y, z, roll, pitch, yaw) -> 4x4 fp64, the matrix pcl::getTransformation writes down."""
+    R, t = pcl_transform([p6[3], p6[4], p6[5], p6[0], p6[1], p6[2]])
+    M = np.eye(4)
+    M[:3, :3], M[:3, 3] = R, t
+    return M
+
+
+def _loop_cloud(job):
+    k, pose6, n_points, seed = job
+    Tt = pose6_matrix(pose6)
+    dirs = livox_dirs(int(n_points * 1.3) + 32, seed + 5000 + k)
+    hits = raycast(Tt[:3, 3], Tt[:3, :3], dirs, make_world(seed, beams=True), seed=seed + 5000 + k)[:n_points]
+    inten = np.floor(np.linalg.norm(hits, axis=1) * 7.0) % 256
+    return np.ascontiguousarray(np.concatenate([hits, inten[:, None].astype(np.float32)], 1), dtype=np.float32)
+
+
+def loop_session(K=2000, n_points=1000, laps=2, radius=18.0, drift=(0.3, 1.0), seed: int = SEED, workers: int = 1):
+    """A seeded session for the loop closure: K keyframes on a circle of `radius` m around the warehouse centre driven `laps`
+    times, 1 s apart.  Keyframe k is a raycast of about n_points points from its TRUE pose (lidar frame, x y z intensity), stored
+    with a DRIFTED pose: the drift grows linearly to drift[0] m (in x / y) and drift[1] degrees (in yaw) per lap.  Returns
+    dict(clouds, poses (K x 6 float32, drifted: x y z roll pitch yaw), poses_true, times, T_true / T_drift (K x 4 x 4)).  The
+    correction that registers keyframe c against the submap of keyframe p is D_p D_c^-1 with D_k = T_drift[k] T_true[k]^-1.
+    workers > 1 raycasts the keyframes in that many processes (same result)."""
+    rng = np.random.default_rng(seed + 31)
+    per_lap = K / laps
+    ang = 2 * np.pi * np.arange(K) / per_lap
+    true6 = np.zeros((K, 6))
+    true6[:, 0], true6[:, 1] = radius * np.cos(ang), radius * np.sin(ang)
+    true6[:, 2] = 1.5 + 0.05 * np.sin(3 * ang)
+    true6[:, 3] = np.deg2rad(1.0) * np.sin(ang)
+    true6[:, 4] = np.deg2rad(0.5) * np.cos(2 * ang)
+    true6[:, 5] = np.arctan2(np.sin(ang + np.pi / 2), np.cos(ang + np.pi / 2))
+    lap = np.arange(K) / per_lap
+    a = rng.uniform(-np.pi, np.pi)
+    drift6 = true6.copy()
+    drift6[:, 0] += drift[0] * lap * np.cos(a)
+    drift6[:, 1] += drift[0] * lap * np.sin(a)
+    drift6[:, 5] += np.deg2rad(drift[1]) * lap
+    true6, drift6 = true6.astype(np.float32), drift6.astype(np.float32)
+    jobs = [(k, true6[k], n_points, seed) for k in range(K)]
+    if workers > 1:
+        import multiprocessing as mp
+        with mp.get_context("fork").Pool(workers) as pool:
+            clouds = pool.map(_loop_cloud, jobs, chunksize=max(1, K // (8 * workers)))
+    else:
+        clouds = [_loop_cloud(j) for j in jobs]
+    return dict(clouds=clouds, poses=drift6, poses_true=true6, times=np.arange(K, dtype=np.float64),
+                T_true=np.array([pose6_matrix(p) for p in true6]), T_drift=np.array([pose6_matrix(p) for p in drift6]))
