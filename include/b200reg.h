@@ -356,6 +356,13 @@ int32_t b200_reloc_argmin(b200_comm* comm, b200_ndt* ndt, const float* poses16, 
 /* same with an interleaved slice: local hypothesis i = global hypothesis h_begin + i * h_stride (rank r of N: h_begin r, stride N) */
 int32_t b200_reloc_argmin_strided(b200_comm* comm, b200_ndt* ndt, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride,
                                   int64_t* best, double* best_score, float* gpu_ms);
+/* How b200_reloc_argmin[_strided] scores (per handle; default on): on = every hypothesis is first scored in fp32 with a
+ * certified interval that contains its calculateScore value, and only those that can still be the winner are scored in
+ * fp64; off = all of them in fp64.  The winner, its score bits and the return code are the same either way. */
+int32_t b200_ndt_set_reloc_screen(b200_ndt* ndt, int32_t on);
+/* The certified intervals behind the screen: lo[i] <= calculateScore(pose i) <= hi[i] for h <= 65535 poses, with
+ * [-inf, +inf] where no finite bound holds (non-finite poses, a missing source ordering). */
+int32_t b200_ndt_score_screen(b200_ndt* ndt, const float* poses16, int64_t h, double* lo, double* hi);
 /* Global relocalization with NDT refinement: score -> global top-K -> align() of every candidate -> getFitnessScore -> winner.
  * Slices as for b200_reloc_argmin_strided (comm may be NULL).  The candidates are the top_k hypotheses of highest
  * calculateScore over all ranks (NaN scores and poses with a non-finite entry never qualify), ordered by score descending,
@@ -380,7 +387,8 @@ typedef struct {
 int32_t b200_reloc_refine(b200_comm* comm, b200_ndt* ndt, const float* poses16, int64_t h, int64_t h_begin, int64_t h_stride,
                           int64_t top_k, double max_range, int64_t* best, b200_reloc_candidate* cands, int64_t* n_cands, float* gpu_ms);
 
-/* measurement aids (bench.py): device time of the score kernel of the last score / relocalization call; the number of
+/* measurement aids (bench.py): device time of the scoring of the last score / relocalization call (the fp64 score kernel of
+ * a score call; screen, selection, rescore and finish of a screened relocalization); the number of
  * (source point, occupied neighbourhood voxel) pairs over h poses (algorithmic bytes of the roofline); a device-side
  * rendezvous of the ranks on the handle's stream, so that a timed step starts on all ranks together */
 float b200_ndt_last_score_kernel_ms(b200_ndt* ndt);

@@ -187,6 +187,9 @@ def lib():
         L.b200_ndt_last_score_kernel_ms.argtypes = [vp]
         L.b200_ndt_score_pairs.argtypes = [vp, vp, i64, vp]
         L.b200_ndt_stream_barrier.argtypes = [vp, vp]
+    if hasattr(L, "b200_ndt_score_screen"):  # absent from builds older than the relocalization screen (B200REG_LIB A/B timing)
+        L.b200_ndt_set_reloc_screen.argtypes = [vp, i32]
+        L.b200_ndt_score_screen.argtypes = [vp, vp, i64, vp, vp]
     if hasattr(L, "b200_reloc_refine"):  # absent from builds older than the refined relocalization (B200REG_LIB A/B timing)
         L.b200_reloc_refine.argtypes = [vp, vp, vp, i64, i64, i64, i64, C.c_double, vp, vp, vp, vp]
         L.b200_ndt_last_polls.argtypes = [vp]
@@ -657,6 +660,19 @@ class NormalDistributionsTransform:
         _check(lib().b200_ndt_score_batch(self._handle(), _p(poses), poses.shape[0], _p(s)))
         return s
 
+    def screenScore(self, poses_cm16):
+        """Certified intervals (lo, hi) with lo <= calculateScore <= hi for every pose ([h,16] column-major 4x4); [-inf, inf]
+        where no finite bound holds.  What relocalize screens with: a hypothesis with hi < max(lo) cannot be the winner."""
+        poses = np.ascontiguousarray(poses_cm16, dtype=np.float32).reshape(-1, 16)
+        lo = np.zeros(poses.shape[0])
+        hi = np.zeros(poses.shape[0])
+        _check(lib().b200_ndt_score_screen(self._handle(), _p(poses), poses.shape[0], _p(lo), _p(hi)))
+        return lo, hi
+
+    def setRelocScreen(self, on):
+        """relocalize through the certified fp32 screen (default) or with the fp64 score of every hypothesis; same results."""
+        _check(lib().b200_ndt_set_reloc_screen(self._handle(), int(bool(on))))
+
     def alignBatch(self, guesses_cm16):
         """align() from h independent initial guesses in one batch; returns (finals [h,4,4] row-major, results)."""
         g = np.ascontiguousarray(guesses_cm16, dtype=np.float32).reshape(-1, 16)
@@ -684,7 +700,8 @@ class NormalDistributionsTransform:
         return int(lib().b200_ndt_last_launches(self._handle()))
 
     def last_score_kernel_ms(self):
-        """Device time of the k_ndt_score_batch launch of the last calculateScore / relocalize call."""
+        """Device time of the scoring of the last calculateScore (its k_ndt_score_batch launch) or relocalize call (with the
+        screen on: screen, selection, rescore and finish)."""
         return float(lib().b200_ndt_last_score_kernel_ms(self._handle()))
 
     def score_pairs(self, poses_cm16):

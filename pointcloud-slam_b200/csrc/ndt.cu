@@ -240,25 +240,38 @@ __global__ void k_ndt_finalize(const uint32_t* __restrict__ uniq, const int32_t*
     atomicAdd(n_valid, 1);
 }
 
-// One thread per leaf: the score store (ndt.cuh) from leafD, indexed by the same leaf slot so cell2leaf and nbr7 address
-// it unchanged.  The off-diagonal pairs are stored summed: xt' C xt = xt' ((C + C') / 2) xt.  Leaves without a valid
-// Gaussian are never referenced by cell2leaf / nbr7 and get zeros.
-__global__ void k_ndt_score_store(const LeafD* __restrict__ leafD, const uint8_t* __restrict__ valid, int nruns, Dbl4* __restrict__ sA,
-                                  Dbl4* __restrict__ sB, double* __restrict__ sC) {
+// One thread per leaf: the score store and the fp32 screen store (ndt.cuh) from leafD, indexed by the same leaf slot so
+// cell2leaf and nbr7 address them unchanged.  The off-diagonal pairs are stored summed: xt' C xt = xt' ((C + C') / 2) xt.
+// The screen store holds the mean relative to the corner of the leaf's cell (uniq[r] = its cell id), so that x = (t - o) - m
+// subtracts numbers about a cell apart in fp32 however far the map lies from the origin.  Leaves without a valid Gaussian
+// are never referenced by cell2leaf / nbr7 and get zeros.
+__global__ void k_ndt_score_store(const LeafD* __restrict__ leafD, const uint8_t* __restrict__ valid, const uint32_t* __restrict__ uniq, int nruns,
+                                  GridDims gd, float leaf, Dbl4* __restrict__ sA, Dbl4* __restrict__ sB, double* __restrict__ sC,
+                                  float4* __restrict__ fA, float4* __restrict__ fB, float* __restrict__ fC) {
     const int r = blockIdx.x * blockDim.x + threadIdx.x;
     if (r >= nruns) return;
     Dbl4 a = {0.0, 0.0, 0.0, 0.0}, b = {0.0, 0.0, 0.0, 0.0};
     double c = 0.0;
+    float4 fa = make_float4(0.f, 0.f, 0.f, 0.f);
     if (valid[r]) {
         const LeafD L = leafD[r];
         const double* C = L.icov;
         a = {L.mean[0], L.mean[1], L.mean[2], C[0]};
         b = {C[1] + C[3], C[2] + C[6], C[4], C[5] + C[7]};
         c = C[8];
+        const uint64_t id = uniq[r];
+        const int i0 = (int)(id % (uint64_t)gd.div_b[0]) + gd.min_b[0];
+        const int i1 = (int)((id / (uint64_t)gd.div_b[0]) % (uint64_t)gd.div_b[1]) + gd.min_b[1];
+        const int i2 = (int)(id / ((uint64_t)gd.div_b[0] * (uint64_t)gd.div_b[1])) + gd.min_b[2];
+        fa = make_float4((float)(a.x - (double)cell_origin(i0, leaf)), (float)(a.y - (double)cell_origin(i1, leaf)),
+                         (float)(a.z - (double)cell_origin(i2, leaf)), (float)a.w);
     }
     sA[r] = a;
     sB[r] = b;
     sC[r] = c;
+    fA[r] = fa;
+    fB[r] = make_float4((float)b.x, (float)b.y, (float)b.z, (float)b.w);
+    fC[r] = (float)c;
 }
 
 // DIRECT7 neighbourhood table: one 32-byte record per grid cell = the leaf slots of the cell and its six face neighbours
@@ -1049,58 +1062,70 @@ __global__ void k_ndt_count_done(const Ctl* ctls, int h, int* out) {
 constexpr int SCORE_THREADS = 128;
 constexpr int SCORE_CHUNK = 1024;
 
+// The points of hypothesis h in the ordering of its yaw bin, or nullptr when that ordering is missing (one thread calls it)
+__device__ __forceinline__ const float4* score_src(const View& v, const float* poses, int h, const float4* src_yaw, const int32_t* yaw_slot,
+                                                   int yaw_bins) {
+    const float4* src = v.src;
+    if (yaw_bins) {  // Ndt::yaw_orderings() has built the bin of every pose of the batch; a missing one scores NaN
+        const int slot = yaw_slot[score_yaw_bin(poses[(size_t)h * 16], poses[(size_t)h * 16 + 1], yaw_bins)];
+        src = slot >= 0 ? src_yaw + (size_t)slot * v.n_src : nullptr;
+    }
+    return src;
+}
+
+// Neighbourhood of the transformed point (getNeighborhoodAtPoint): the leaf slot of each stencil cell (or -1) and how many
+// exist.  The fp64 score kernel and the screen share it, so both see exactly the same (point, leaf) pairs.
 template <int NST>
-__global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_batch(View v, const float* __restrict__ poses /*h x 16 col-major*/,
-                                                                   const float4* __restrict__ src_yaw, const int32_t* __restrict__ yaw_slot, int yaw_bins,
-                                                                   double* __restrict__ partial /*[h][nchunks]*/) {
-    __shared__ float M[12];
-    __shared__ double red[SCORE_THREADS / 32];
-    __shared__ const float4* src_s;
-    const int h = blockIdx.y, tid = threadIdx.x;
-    if (tid < 12) M[tid] = poses[(size_t)h * 16 + (tid & 3) * 4 + (tid >> 2)];
-    if (tid == 0) {
-        src_s = v.src;
-        if (yaw_bins) {  // Ndt::yaw_orderings() has built the bin of every pose of the batch; a missing one scores NaN
-            const int slot = yaw_slot[score_yaw_bin(poses[(size_t)h * 16], poses[(size_t)h * 16 + 1], yaw_bins)];
-            src_s = slot >= 0 ? src_yaw + (size_t)slot * v.n_src : nullptr;
+__device__ __forceinline__ int score_nbhd(const View& v, float tx, float ty, float tz, int (&lf)[NST]) {
+    int cnt = 0;
+    bool looked_up = false;
+    if (NST == 7 && v.nbr7) {  // the whole neighbourhood with one 256-bit load when the point's own cell is inside the grid
+        const int ix = (int)floorf(tx / v.leaf) - v.min_b[0], iy = (int)floorf(ty / v.leaf) - v.min_b[1], iz = (int)floorf(tz / v.leaf) - v.min_b[2];
+        if (ix >= 0 && iy >= 0 && iz >= 0 && ix <= v.max_b[0] - v.min_b[0] && iy <= v.max_b[1] - v.min_b[1] && iz <= v.max_b[2] - v.min_b[2]) {
+            const int* rec = v.nbr7 + ((size_t)ix * v.mul[0] + (size_t)iy * v.mul[1] + (size_t)iz * v.mul[2]) * 8;
+            int r[8];
+            asm volatile("ld.global.nc.v8.s32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+                         : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
+                         : "l"(rec));
+#pragma unroll
+            for (int s = 0; s < NST; ++s) lf[s] = r[s < 7 ? s : 0];
+            cnt = r[7];
+            looked_up = true;
         }
     }
+    if (!looked_up) {
+#pragma unroll
+        for (int s = 0; s < NST; ++s) {
+            lf[s] = nbr_leaf(v, tx, ty, tz, s);
+            cnt += lf[s] >= 0 ? 1 : 0;
+        }
+    }
+    return cnt;
+}
+
+// One block's partial sum of calculateScore: chunk `chunk` of the points of hypothesis h, fp64 throughout.  M, red and
+// src_s are the block's shared memory; the caller synchronises before reusing them.
+template <int NST>
+__device__ __forceinline__ void score_chunk(const View& v, const float* __restrict__ poses, const float4* __restrict__ src_yaw,
+                                            const int32_t* __restrict__ yaw_slot, int yaw_bins, int h, int chunk, int nchunks,
+                                            double* __restrict__ partial, float* M, double* red, const float4** src_s) {
+    const int tid = threadIdx.x;
+    if (tid < 12) M[tid] = poses[(size_t)h * 16 + (tid & 3) * 4 + (tid >> 2)];
+    if (tid == 0) *src_s = score_src(v, poses, h, src_yaw, yaw_slot, yaw_bins);
     __syncthreads();
-    const float4* __restrict__ src = src_s;
+    const float4* __restrict__ src = *src_s;
     if (!src) {
-        if (tid == 0) partial[(size_t)h * gridDim.x + blockIdx.x] = __longlong_as_double(0x7ff8000000000000ll);
+        if (tid == 0) partial[(size_t)h * nchunks + chunk] = __longlong_as_double(0x7ff8000000000000ll);
         return;
     }
     double acc = 0.0;
-    const int i_end = min(v.n_src, (int)(blockIdx.x + 1) * SCORE_CHUNK);
-    for (int i = blockIdx.x * SCORE_CHUNK + tid; i < i_end; i += SCORE_THREADS) {
+    const int i_end = min(v.n_src, (chunk + 1) * SCORE_CHUNK);
+    for (int i = chunk * SCORE_CHUNK + tid; i < i_end; i += SCORE_THREADS) {
         const float4 p = __ldg(src + i);
         float tx, ty, tz;
         xform(M, p.x, p.y, p.z, tx, ty, tz);
         int lf[NST];
-        int cnt = 0;
-        bool looked_up = false;
-        if (NST == 7 && v.nbr7) {  // the whole neighbourhood with one 256-bit load when the point's own cell is inside the grid
-            const int ix = (int)floorf(tx / v.leaf) - v.min_b[0], iy = (int)floorf(ty / v.leaf) - v.min_b[1], iz = (int)floorf(tz / v.leaf) - v.min_b[2];
-            if (ix >= 0 && iy >= 0 && iz >= 0 && ix <= v.max_b[0] - v.min_b[0] && iy <= v.max_b[1] - v.min_b[1] && iz <= v.max_b[2] - v.min_b[2]) {
-                const int* rec = v.nbr7 + ((size_t)ix * v.mul[0] + (size_t)iy * v.mul[1] + (size_t)iz * v.mul[2]) * 8;
-                int r[8];
-                asm volatile("ld.global.nc.v8.s32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                             : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                             : "l"(rec));
-#pragma unroll
-                for (int s = 0; s < NST; ++s) lf[s] = r[s < 7 ? s : 0];
-                cnt = r[7];
-                looked_up = true;
-            }
-        }
-        if (!looked_up) {
-#pragma unroll
-            for (int s = 0; s < NST; ++s) {
-                lf[s] = nbr_leaf(v, tx, ty, tz, s);
-                cnt += lf[s] >= 0 ? 1 : 0;
-            }
-        }
+        const int cnt = score_nbhd<NST>(v, tx, ty, tz, lf);
         // score_inc / neighborhood.size() (:876): the size is inverted once per point (<= 1 ulp per term, far inside the
         // 1e-12 score tolerance) - the fp64 division was 13 % of this kernel's instructions
         const double rcnt = cnt > 0 ? 1.0 / (double)cnt : 0.0;
@@ -1126,15 +1151,211 @@ __global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_batch(View v, const
         double a = red[0];
 #pragma unroll
         for (int w = 1; w < SCORE_THREADS / 32; ++w) a += red[w];
-        partial[(size_t)h * gridDim.x + blockIdx.x] = a;
+        partial[(size_t)h * nchunks + chunk] = a;
     }
+}
+
+template <int NST>
+__global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_batch(View v, const float* __restrict__ poses /*h x 16 col-major*/,
+                                                                   const float4* __restrict__ src_yaw, const int32_t* __restrict__ yaw_slot, int yaw_bins,
+                                                                   double* __restrict__ partial /*[h][nchunks]*/) {
+    __shared__ float M[12];
+    __shared__ double red[SCORE_THREADS / 32];
+    __shared__ const float4* src_s;
+    score_chunk<NST>(v, poses, src_yaw, yaw_slot, yaw_bins, blockIdx.y, blockIdx.x, gridDim.x, partial, M, red, &src_s);
+}
+__device__ __forceinline__ double score_finish_one(const double* __restrict__ partial, int nchunks, int64_t a, int n_src) {
+    double s = 0.0;
+    for (int c = 0; c < nchunks; ++c) s += partial[a * nchunks + c];
+    return s / (double)n_src;
 }
 __global__ void k_ndt_score_finish(const double* __restrict__ partial, int nchunks, int64_t h, int n_src, double* __restrict__ scores) {
     const int64_t a = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     if (a >= h) return;
-    double s = 0.0;
-    for (int c = 0; c < nchunks; ++c) s += partial[a * nchunks + c];
-    scores[a] = s / (double)n_src;
+    scores[a] = score_finish_one(partial, nchunks, a, n_src);
+}
+
+// ------------------------------------------------------------------ relocalization screen (DESIGN.md §5, "certified screen")
+// A relocalization needs the fp64 score of the winner only.  k_ndt_score_screen scores every hypothesis in fp32 from the
+// 36-byte screen store, over exactly the fp64 kernel's (point, leaf) pairs, together with a rigorous bound on the distance
+// to the fp64 score; k_ndt_screen_finish turns both into an interval [lo, hi] that contains the score k_ndt_score_batch
+// computes.  Only hypotheses whose hi reaches the best lo (ties included) are rescored with the unchanged fp64 arithmetic,
+// so the winner and its score bits are those of the full fp64 batch.
+constexpr float SCREEN_U = 5.9604644775390625e-8f;     // 2^-24: unit roundoff of fp32
+constexpr float SCREEN_EX2_ERR = 1.9073486328125e-6f;  // 2^-19 >= 2 x (1 + 2^-20) x ex2.approx's documented 2^-22 relative error
+constexpr float SCREEN_FTZ = 1.1754943508222875e-38f;  // 2^-126: what ex2.approx.ftz may flush to zero
+constexpr float SCREEN_PAIR_ABS = 1.7763568394002505e-15f;  // 2^-49 >= the fp64 path's own |exp error| per pair
+constexpr int SCREEN_CAP = 64;                          // rescore blocks per chunk (survivor i goes to block row i mod CAP)
+
+__device__ __forceinline__ float ex2_approx(float y) {
+    float r;
+    asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(y));
+    return r;
+}
+
+// grid = (point chunks, hypotheses) as k_ndt_score_batch.  kq = fp32(-d2 / 2 * log2(e)); kD = (d2 / 2) * 16 u, rounded up.
+// part[(h * nchunks + chunk) * 3 + {0, 1, 2}] = {sum of E_p / cnt_p, bound on its error, points with a neighbour}.
+template <int NST>
+__global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_screen(View v, const float* __restrict__ poses, const float4* __restrict__ src_yaw,
+                                                                    const int32_t* __restrict__ yaw_slot, int yaw_bins, const float4* __restrict__ fA,
+                                                                    const float4* __restrict__ fB, const float* __restrict__ fC, float kq, float kD,
+                                                                    double* __restrict__ part) {
+    __shared__ float M[12];
+    __shared__ double red[2][SCORE_THREADS / 32];
+    __shared__ int redn[SCORE_THREADS / 32];
+    __shared__ const float4* src_s;
+    const int tid = threadIdx.x, h = blockIdx.y;
+    double* out = part + ((size_t)h * gridDim.x + blockIdx.x) * 3;
+    if (tid < 12) M[tid] = poses[(size_t)h * 16 + (tid & 3) * 4 + (tid >> 2)];
+    if (tid == 0) src_s = score_src(v, poses, h, src_yaw, yaw_slot, yaw_bins);
+    __syncthreads();
+    const float4* __restrict__ src = src_s;
+    if (!src) {
+        if (tid == 0) { out[0] = __longlong_as_double(0x7ff8000000000000ll); out[1] = 0.0; out[2] = 0.0; }
+        return;
+    }
+    double accW = 0.0;
+    float accErr = 0.f;
+    int accN = 0;
+    const int i_end = min(v.n_src, (int)(blockIdx.x + 1) * SCORE_CHUNK);
+    for (int i = blockIdx.x * SCORE_CHUNK + tid; i < i_end; i += SCORE_THREADS) {
+        const float4 p = __ldg(src + i);
+        float tx, ty, tz;
+        xform(M, p.x, p.y, p.z, tx, ty, tz);
+        int lf[NST];
+        const int cnt = score_nbhd<NST>(v, tx, ty, tz, lf);
+        if (cnt == 0) continue;
+        const int cx = (int)floorf(tx / v.leaf), cy = (int)floorf(ty / v.leaf), cz = (int)floorf(tz / v.leaf);
+        float E = 0.f, errE = 0.f;
+#pragma unroll
+        for (int s = 0; s < NST; ++s) {
+            if (lf[s] < 0) continue;
+            int dx, dy, dz;
+            nbr_offset(NST == 27 ? 27 : 7, s, dx, dy, dz);
+            const float4 A = __ldg(fA + lf[s]);  // m, c00
+            const float4 B = __ldg(fB + lf[s]);  // s01, s02, c11, s12
+            const float c22 = __ldg(fC + lf[s]);
+            // x = (t - o) - m: both differences are between numbers about a cell apart
+            const float d0 = tx - cell_origin(cx + dx, v.leaf), d1 = ty - cell_origin(cy + dy, v.leaf), d2 = tz - cell_origin(cz + dz, v.leaf);
+            const float x0 = d0 - A.x, x1 = d1 - A.y, x2 = d2 - A.z;
+            const float b0 = fabsf(d0) + fabsf(A.x), b1 = fabsf(d1) + fabsf(A.y), b2 = fabsf(d2) + fabsf(A.z);
+            const float q = fmaf(x0, fmaf(B.y, x2, fmaf(B.x, x1, A.w * x0)), fmaf(x1, fmaf(B.w, x2, B.z * x1), x2 * (c22 * x2)));
+            // absolute companion: the same form over |coefficients| and b_i = |d_i| + |m_i| >= |x_i|
+            const float Q = fmaf(b0, fmaf(fabsf(B.y), b2, fmaf(fabsf(B.x), b1, fabsf(A.w) * b0)),
+                                 fmaf(b1, fmaf(fabsf(B.w), b2, fabsf(B.z) * b1), b2 * (fabsf(c22) * b2)));
+            const float e = ex2_approx(q * kq);
+            const float D = Q * kD;  // bound on |exponent error| (natural log units)
+            const float fac = D <= 0.015625f ? 1.03f * D : 1.03f * D * ex2_approx(1.5f * D);
+            E += e;
+            errE += (e + SCREEN_FTZ) * (SCREEN_EX2_ERR + fac) + SCREEN_PAIR_ABS;
+        }
+        const float rc = __frcp_rn((float)cnt);
+        accW += (double)(E * rc);
+        accErr += (errE + 36.f * SCREEN_U * E) * rc;
+        ++accN;
+    }
+    double err = (double)accErr;
+    for (int o = 16; o > 0; o >>= 1) {
+        accW += __shfl_xor_sync(0xffffffffu, accW, o);
+        err += __shfl_xor_sync(0xffffffffu, err, o);
+        accN += __shfl_xor_sync(0xffffffffu, accN, o);
+    }
+    if ((tid & 31) == 0) { red[0][tid >> 5] = accW; red[1][tid >> 5] = err; redn[tid >> 5] = accN; }
+    __syncthreads();
+    if (tid == 0) {
+        double w = red[0][0], e = red[1][0];
+        int n = redn[0];
+#pragma unroll
+        for (int k = 1; k < SCORE_THREADS / 32; ++k) { w += red[0][k]; e += red[1][k]; n += redn[k]; }
+        out[0] = w; out[1] = e; out[2] = (double)n;
+    }
+}
+
+// One thread per hypothesis: the certified interval [lo, hi] of its score (DESIGN.md §5).  A hypothesis whose bound is not
+// finite gets [-inf, +inf] ("must rescore").  nst = stencil cells (bounds the fp64 path's summation depth).
+__global__ void k_ndt_screen_finish(const double* __restrict__ part, int nchunks, int64_t h, int n_src, int nst, double d1, double d3,
+                                    double* __restrict__ lo, double* __restrict__ hi) {
+    const int64_t a = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
+    if (a >= h) return;
+    double W = 0.0, err = 0.0, N = 0.0;
+    for (int c = 0; c < nchunks; ++c) {
+        const double* p = part + ((size_t)a * nchunks + c) * 3;
+        W += p[0];
+        err += p[1];
+        N += p[2];
+    }
+    const double center = (-d1 * W - d3 * N) / (double)n_src;
+    // |d1| err: the fp32 screen; the rest: rounding of the fp64 path (summation depth <= 8 nst + 64 + nchunks) and of ours
+    const double mass = fabs(d1) * (W + err) + fabs(d3) * N;
+    const double rad = 1.001 * (fabs(d1) * err + (8.0 * nst + 64.0 + nchunks) * 4.440892098500626e-16 * mass) / (double)n_src;
+    if (isfinite(center) && isfinite(rad)) {
+        lo[a] = __dsub_rd(center, rad);
+        hi[a] = __dadd_ru(center, rad);
+    } else {
+        lo[a] = -CUDART_INF;
+        hi[a] = CUDART_INF;
+    }
+}
+
+// One block: LB = the best lo of the slice; list[1 + j] = the local indices with hi >= LB (ties and [-inf, +inf] included)
+// in ascending order, list[0] = how many.
+__global__ void __launch_bounds__(1024) k_ndt_screen_select(const double* __restrict__ lo, const double* __restrict__ hi, int64_t h,
+                                                            int32_t* __restrict__ list) {
+    __shared__ double sb[32];
+    __shared__ int wcnt[32];
+    __shared__ int base;
+    const int tid = threadIdx.x, lane = tid & 31, w = tid >> 5;
+    double lb = -CUDART_INF;
+    for (int64_t i = tid; i < h; i += blockDim.x) lb = fmax(lb, lo[i]);
+    for (int o = 16; o > 0; o >>= 1) lb = fmax(lb, __shfl_xor_sync(0xffffffffu, lb, o));
+    if (lane == 0) sb[w] = lb;
+    if (tid == 0) base = 0;
+    __syncthreads();
+    lb = sb[0];
+    for (int k = 1; k < (int)(blockDim.x >> 5); ++k) lb = fmax(lb, sb[k]);
+    for (int64_t b0 = 0; b0 < h; b0 += blockDim.x) {
+        const int64_t i = b0 + tid;
+        const bool keep = i < h && !(hi[i] < lb);
+        const unsigned m = __ballot_sync(0xffffffffu, keep);
+        if (lane == 0) wcnt[w] = __popc(m);
+        __syncthreads();
+        int off = base;
+        for (int k = 0; k < w; ++k) off += wcnt[k];
+        if (keep) list[1 + off + __popc(m & ((1u << lane) - 1u))] = (int32_t)i;
+        __syncthreads();
+        if (tid == 0) {
+            int t = 0;
+            for (int k = 0; k < (int)(blockDim.x >> 5); ++k) t += wcnt[k];
+            base += t;
+        }
+        __syncthreads();
+    }
+    if (tid == 0) list[0] = base;
+}
+
+// grid = (point chunks, SCREEN_CAP): the fp64 partials of the listed hypotheses, each exactly as k_ndt_score_batch computes
+// it (same chunks, same code).  Block row j takes list entries j, j + CAP, ...; rows without work exit.
+template <int NST>
+__global__ void __launch_bounds__(SCORE_THREADS) k_ndt_score_rescore(View v, const float* __restrict__ poses, const float4* __restrict__ src_yaw,
+                                                                     const int32_t* __restrict__ yaw_slot, int yaw_bins,
+                                                                     const int32_t* __restrict__ list, double* __restrict__ partial) {
+    __shared__ float M[12];
+    __shared__ double red[SCORE_THREADS / 32];
+    __shared__ const float4* src_s;
+    const int n = list[0];
+    for (int j = blockIdx.y; j < n; j += gridDim.y) {
+        __syncthreads();  // the previous hypothesis is done with the shared memory
+        score_chunk<NST>(v, poses, src_yaw, yaw_slot, yaw_bins, list[1 + j], blockIdx.x, gridDim.x, partial, M, red, &src_s);
+    }
+}
+// the listed hypotheses' scores as k_ndt_score_finish computes them
+__global__ void k_ndt_score_finish_list(const double* __restrict__ partial, int nchunks, const int32_t* __restrict__ list, int n_src,
+                                        double* __restrict__ scores) {
+    const int n = list[0];
+    for (int j = blockIdx.x * blockDim.x + threadIdx.x; j < n; j += gridDim.x * blockDim.x) {
+        const int64_t a = list[1 + j];
+        scores[a] = score_finish_one(partial, nchunks, a, n_src);
+    }
 }
 
 // number of occupied (point, voxel) pairs of one evaluation, summed over a batch of poses (col-major 4x4 each; roofline
@@ -1527,6 +1748,8 @@ struct Ndt {
     DevBuf<LeafD> d_leafD;
     DevBuf<Dbl4> d_sA, d_sB;   // score store (k_ndt_score_store)
     DevBuf<double> d_sC;
+    DevBuf<float4> d_fA, d_fB;  // fp32 screen store (k_ndt_score_store)
+    DevBuf<float> d_fC;
     DevBuf<double> d_cov, d_sums;
     DevBuf<float> d_centroid;
     DevBuf<int32_t> d_npts, d_vals_in, d_vals_out, d_run_cnt, d_run_off, d_small;
@@ -1583,6 +1806,11 @@ struct Ndt {
     int32_t until_done(int h, int max_launches, int& launches, Launch launch);
     int32_t yaw_orderings(const float* d_poses16, int64_t h);
     int32_t score_batch_device(const float* d_poses16, int64_t h, double* d_out);
+    int32_t score_screen_device(const float* d_poses16, int64_t h, double* d_lo, double* d_hi);
+    int32_t reloc_scores_device(const float* d_poses16, int64_t h, double* d_out);
+    bool reloc_screen = true;  // relocalization: certified fp32 screen + fp64 rescore of the survivors (b200_ndt_set_reloc_screen)
+    DevBuf<double> d_spart, d_lo, d_hi;
+    DevBuf<int32_t> d_surv;
     int32_t fitness(const float* T16_colmajor, double max_range, double* score, int64_t* nr);
 };
 
@@ -1615,7 +1843,7 @@ void Ndt::destroy() {
     cudaSetDevice(device);
     if (stream) cudaStreamSynchronize(stream);
     d_tgt.release(); d_src.release(); d_src_raw.release(); d_tgt_sorted.release(); s_keys_in.release(); s_keys_out.release();
-    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_fitcall.release(); h_fitcall.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_sA.release(); d_sB.release(); d_sC.release(); d_cov.release(); d_sums.release(); d_centroid.release();
+    s_vals_in.release(); s_vals_out.release(); d_src_yaw.release(); d_yaw_slot.release(); d_yaw_need.release(); d_yaw_list.release(); h_yaw.release(); y_keys_in.release(); y_keys_out.release(); y_vals_in.release(); y_vals_out.release(); d_cell2run.release(); s_tmp.release(); d_fit.release(); d_fitcall.release(); h_fitcall.release(); d_cell2leaf.release(); d_nbr7.release(); d_leafF.release(); d_leafD.release(); d_sA.release(); d_sB.release(); d_sC.release(); d_fA.release(); d_fB.release(); d_fC.release(); d_spart.release(); d_lo.release(); d_hi.release(); d_surv.release(); d_cov.release(); d_sums.release(); d_centroid.release();
     d_npts.release(); d_vals_in.release(); d_vals_out.release(); d_run_cnt.release(); d_run_off.release(); d_small.release();
     d_keys_in.release(); d_keys_out.release(); d_uniq.release(); d_valid.release(); cub_tmp.release();
     d_off.release(); h_off.release(); d_mm.release(); h_mm.release(); d_pg.release(); h_pg.release();
@@ -1849,7 +2077,9 @@ int32_t Ndt::build_target(int64_t n) {
     rc = build_leaves(1, (unsigned)((n + 255) / 256), n, ncells);
     if (rc) return rc;
     CUDA_TRY(d_sA.reserve(nruns)); CUDA_TRY(d_sB.reserve(nruns)); CUDA_TRY(d_sC.reserve(nruns));
-    k_ndt_score_store<<<(nruns + 127) / 128, 128, 0, stream>>>(d_leafD.p, d_valid.p, nruns, d_sA.p, d_sB.p, d_sC.p);
+    CUDA_TRY(d_fA.reserve(nruns)); CUDA_TRY(d_fB.reserve(nruns)); CUDA_TRY(d_fC.reserve(nruns));
+    k_ndt_score_store<<<(nruns + 127) / 128, 128, 0, stream>>>(d_leafD.p, d_valid.p, d_uniq.p, nruns, gd, prm.resolution, d_sA.p, d_sB.p, d_sC.p,
+                                                               d_fA.p, d_fB.p, d_fC.p);
     LAUNCH_COUNT(1);
     have_nbr7 = prm.search == 7 && ncells <= ((int64_t)1 << 26);  // 32 B per cell: at most 2 GB
     if (have_nbr7) {
@@ -2052,6 +2282,55 @@ int32_t Ndt::score_batch_device(const float* d_poses16, int64_t h, double* d_out
     CUDA_TRY(cudaEventRecord(evs1, stream));
     k_ndt_score_finish<<<(unsigned)((h + 127) / 128), 128, 0, stream>>>(d_partials.p, nch, h, n_src, d_out);
     LAUNCH_COUNT(2);
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}
+
+// The certified score interval of every pose (k_ndt_score_screen + k_ndt_screen_finish); no host synchronisation.  The
+// caller has checked the arguments and built the yaw orderings of the poses (Ndt::yaw_orderings).
+int32_t Ndt::score_screen_device(const float* d_poses16, int64_t h, double* d_lo, double* d_hi) {
+    gauss();
+    const int nch = (n_src + SCORE_CHUNK - 1) / SCORE_CHUNK;
+    CUDA_TRY(d_spart.reserve((size_t)h * nch * 3));
+    const dim3 grid(nch, (unsigned)h);
+    const View v = view();
+    const float kq = (float)(-d2 * 0.5 * 1.4426950408889634);
+    const float kD = (float)(d2 * 0.5 * 16.0 * 5.9604644775390625e-8 * (1.0 + 1e-6));
+    if (prm.search == 1) k_ndt_score_screen<1><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_fA.p, d_fB.p, d_fC.p, kq, kD, d_spart.p);
+    else if (nst() == 27) k_ndt_score_screen<27><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_fA.p, d_fB.p, d_fC.p, kq, kD, d_spart.p);
+    else k_ndt_score_screen<7><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_fA.p, d_fB.p, d_fC.p, kq, kD, d_spart.p);
+    k_ndt_screen_finish<<<(unsigned)((h + 127) / 128), 128, 0, stream>>>(d_spart.p, nch, h, n_src, nst(), d1, d3, d_lo, d_hi);
+    LAUNCH_COUNT(2);
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}
+
+// Relocalization scores: with the screen on, d_out holds the fp64 score (the bits of score_batch_device) of every hypothesis
+// that can still be the winner and NaN elsewhere, which k_local_best never picks; the survivor count stays on the device.
+// evs0 / evs1 bracket all of the scoring work: screen, selection, rescore and finish.
+int32_t Ndt::reloc_scores_device(const float* d_poses16, int64_t h, double* d_out) {
+    if (!reloc_screen) return score_batch_device(d_poses16, h, d_out);
+    if (!have_target) B200_FAIL(B200_ERR_ARG, "no target set");
+    if (n_src < 1) B200_FAIL(B200_ERR_ARG, "no source set");
+    if (h > 65535) B200_FAIL(B200_ERR_ARG, "at most 65535 hypotheses per call");
+    const int32_t rc0 = yaw_orderings(d_poses16, h);  // before evs0, as in score_batch_device
+    if (rc0) return rc0;
+    const int nch = (n_src + SCORE_CHUNK - 1) / SCORE_CHUNK;
+    CUDA_TRY(d_lo.reserve(h)); CUDA_TRY(d_hi.reserve(h)); CUDA_TRY(d_surv.reserve(h + 1));
+    CUDA_TRY(d_partials.reserve((size_t)h * nch));
+    CUDA_TRY(cudaEventRecord(evs0, stream));
+    const int32_t rc = score_screen_device(d_poses16, h, d_lo.p, d_hi.p);
+    if (rc) return rc;
+    k_ndt_screen_select<<<1, 1024, 0, stream>>>(d_lo.p, d_hi.p, h, d_surv.p);
+    CUDA_TRY(cudaMemsetAsync(d_out, 0xFF, (size_t)h * sizeof(double), stream));  // all-ones = NaN
+    const View v = view();
+    const dim3 grid(nch, SCREEN_CAP);
+    if (prm.search == 1) k_ndt_score_rescore<1><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_surv.p, d_partials.p);
+    else if (nst() == 27) k_ndt_score_rescore<27><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_surv.p, d_partials.p);
+    else k_ndt_score_rescore<7><<<grid, SCORE_THREADS, 0, stream>>>(v, d_poses16, d_src_yaw.p, d_yaw_slot.p, yaw_bins, d_surv.p, d_partials.p);
+    k_ndt_score_finish_list<<<(unsigned)std::min<int64_t>((h + 127) / 128, 64), 128, 0, stream>>>(d_partials.p, nch, d_surv.p, n_src, d_out);
+    CUDA_TRY(cudaEventRecord(evs1, stream));
+    LAUNCH_COUNT(3);
     CUDA_TRY(cudaGetLastError());
     return B200_OK;
 }
@@ -2831,7 +3110,7 @@ static int32_t reloc_argmin_impl(b200_comm* comm, b200_ndt* n, const float* pose
     int32_t rc_local = B200_OK;
     std::string err_local;
     if (h) {
-        rc_local = k.score_batch_device(k.d_poses.p, h, k.d_scores.p);
+        rc_local = k.reloc_scores_device(k.d_poses.p, h, k.d_scores.p);
         if (rc_local) err_local = g_last_error;
     }
     ndt::k_local_best<<<1, 256, 0, k.stream>>>(k.d_scores.p, rc_local ? 0 : h, h_begin, h_stride, d);
@@ -2858,7 +3137,34 @@ static int32_t reloc_argmin_impl(b200_comm* comm, b200_ndt* n, const float* pose
     if (best_score) *best_score = sc;
     return B200_OK;
 }
-/* device time of the k_ndt_score_batch launch of the last score / relocalization call (CUDA events around that kernel alone) */
+/* relocalization through the certified fp32 screen (default) or the fp64 score of every hypothesis; same results */
+int32_t b200_ndt_set_reloc_screen(b200_ndt* n, int32_t on) {
+    if (!n) B200_FAIL(B200_ERR_ARG, "bad argument");
+    n->k.reloc_screen = on != 0;
+    return B200_OK;
+}
+/* the certified interval [lo, hi] of calculateScore of each of h poses; [-inf, +inf] where the bound is not finite */
+int32_t b200_ndt_score_screen(b200_ndt* n, const float* poses16, int64_t h, double* lo, double* hi) {
+    if (!n || !poses16 || h < 1 || h > 65535 || !lo || !hi) B200_FAIL(B200_ERR_ARG, "bad argument");
+    Ndt& k = n->k;
+    CUDA_SET_DEVICE(k.device);
+    CUDA_TRY(k.d_poses.reserve((size_t)h * 16)); CUDA_TRY(k.h_poses.reserve((size_t)h * 16));
+    CUDA_TRY(k.d_lo.reserve(h)); CUDA_TRY(k.d_hi.reserve(h));
+    memcpy(k.h_poses.p, poses16, (size_t)h * 16 * sizeof(float));
+    CUDA_TRY(cudaMemcpyAsync(k.d_poses.p, k.h_poses.p, (size_t)h * 16 * sizeof(float), cudaMemcpyHostToDevice, k.stream));
+    if (!k.have_target || k.n_src < 1) B200_FAIL(B200_ERR_ARG, "no target / source set");
+    int32_t rc = k.yaw_orderings(k.d_poses.p, h);
+    if (rc) return rc;
+    rc = k.score_screen_device(k.d_poses.p, h, k.d_lo.p, k.d_hi.p);
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(lo, k.d_lo.p, (size_t)h * sizeof(double), cudaMemcpyDeviceToHost, k.stream));
+    CUDA_TRY(cudaMemcpyAsync(hi, k.d_hi.p, (size_t)h * sizeof(double), cudaMemcpyDeviceToHost, k.stream));
+    CUDA_TRY(cudaStreamSynchronize(k.stream));
+    CUDA_TRY(cudaGetLastError());
+    return B200_OK;
+}
+/* device time of the scoring of the last score / relocalization call: the k_ndt_score_batch launch of a score call; for a
+ * relocalization with the screen on, everything from the screen kernel to the survivors' scores */
 float b200_ndt_last_score_kernel_ms(b200_ndt* n) {
     if (!n) return 0.f;
     float ms = 0.f;

@@ -18,6 +18,10 @@
 //     sA[L]   32 B   {mean_x, mean_y, mean_z, icov00}
 //     sB[L]   32 B   {icov01 + icov10, icov02 + icov20, icov11, icov12 + icov21}
 //     sC[L]    8 B   icov22
+//   fp32 screen store, 36 B per leaf, the same numbers narrowed (what the relocalization screen reads; 8 leaves per line)
+//     fA[L]   16 B   {m_x, m_y, m_z, icov00}      m = fp32(mean - o), o = corner of the leaf's cell (cell_origin)
+//     fB[L]   16 B   {s01, s02, icov11, s12}
+//     fC[L]    4 B   icov22
 //   cov[L] 72 B, npts[L], ids[L], valid[L]                   only read back by b200_ndt_leaves
 // The TU is compiled with -fmad=false: every fp32/fp64 operation below is individually rounded, in the
 // evaluation order of the reference C++ (Eigen fixed-size products accumulate k = 0..3 left to right).
@@ -78,6 +82,9 @@ struct View {
     int nst;   // 1, 7, 27
     double d1, d2, d3;
 };
+
+// Corner of grid cell i along one axis, as the screen store and the screen kernel both compute it (same bits on both sides)
+__device__ __forceinline__ float cell_origin(int i, float leaf) { return __fmul_rn((float)i, leaf); }
 
 // DIRECT7 order (voxel_grid_covariance_omp_impl.hpp:423-430); DIRECT26 = pcl::getAllNeighborCellIndices()
 // (27 cells, x slowest); DIRECT1 = the cell itself.
