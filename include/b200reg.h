@@ -246,6 +246,10 @@ int32_t b200_keyframes_destroy(b200_keyframes* h);
 /* cornerCloudKeyFrames / surfCloudKeyFrames.push_back + cloudKeyPoses3D / cloudKeyPoses6D.push_back (saveKeyFramesAndFactor):
  * records x y z[ intensity] at stride_bytes (>= 16 carries the intensity, 12 stores 0); *key = the keyframe's index (may be NULL) */
 int32_t b200_keyframes_add(b200_keyframes* h, const float* xyzi, int64_t n, int64_t stride_bytes, const float* pose6, double time, int64_t* key);
+/* the same keyframe given as its two LOAM feature clouds: stores exactly what b200_keyframes_add stores for corner followed by
+ * surf, and remembers n_corner so that the local map (b200_loam_set_map_from_keyframes) can split the cloud again */
+int32_t b200_keyframes_add_features(b200_keyframes* h, const float* corner, int64_t n_corner, int64_t stride_corner, const float* surf, int64_t n_surf,
+                                    int64_t stride_surf, const float* pose6, double time, int64_t* key);
 /* correctPoses(): poses of keyframes first .. first+count-1 replaced by poses6 (count x 6 floats); clouds untouched */
 int32_t b200_keyframes_set_poses(b200_keyframes* h, int64_t first, int64_t count, const float* poses6);
 int64_t b200_keyframes_count(b200_keyframes* h); /* -1 for a NULL handle */
@@ -284,6 +288,31 @@ int32_t b200_loop_submap(b200_keyframes* h, int64_t key, int32_t search_num, flo
  * The store and the pairs handle must be on the same device. */
 int32_t b200_loop_close(b200_comm* comm, b200_ndt_pairs* ndt, b200_keyframes* h, const int64_t* cur, const int64_t* pre, int64_t Q,
                         const b200_loop_params* prm, b200_loop_result* results);
+
+/* extractSurroundingKeyFrames (LIO-SAM mapOptmization.cpp) from the store, for the scan at time_cur when keyframe cur is the
+ * newest (only keyframes 0 .. cur exist; cur = -1: the last one):
+ *   extractNearby: keyframes j <= cur strictly inside search_radius of keyframe cur (b200_loop_detect's squared distance and
+ *     r^2), in ascending (d2, j) order -> VoxelGrid(density) of their positions -> each centroid's nearest keyframe among
+ *     0 .. cur (ties to the lower index) -> then keyframes cur, cur-1, .. while time_cur - time_j < 10.0;
+ *   extractCloud: entries whose point (centroid, or the keyframe's own position) lies farther than search_radius from
+ *     keyframe cur (sqrtf of the squared distance) are skipped; each remaining keyframe's corner / surf cloud is moved into
+ *     the world by its pose and appended (a keyframe listed twice is appended twice); VoxelGrid(corner_leaf) and
+ *     VoxelGrid(surf_leaf), min points 0, give laserCloud{Corner,Surf}FromMapDS.
+ * Every listed keyframe must have been added with b200_keyframes_add_features (otherwise B200_ERR_ARG).  An empty store is
+ * B200_NO_EFFECTIVE_POINTS; a grid of more than 9e18 leaves is B200_ERR_RANGE. */
+typedef struct {
+    float search_radius; /* surroundingKeyframeSearchRadius (50) */
+    float density;       /* surroundingKeyframeDensity (2.0) */
+    float corner_leaf;   /* mappingCornerLeafSize (0.2) */
+    float surf_leaf;     /* mappingSurfLeafSize (0.4) */
+} b200_surround_params;
+/* parity probe: the list after extractCloud's distance gate, in extraction order (at most max_keys written), *n_keys = its length */
+int32_t b200_keyframes_surrounding(b200_keyframes* h, int64_t cur, double time_cur, const b200_surround_params* prm, int64_t* keys, int64_t max_keys,
+                                   int64_t* n_keys);
+/* parity probe: laserCloudCornerFromMapDS / laserCloudSurfFromMapDS, 4 floats per point in ascending leaf order (at most max_*
+ * written), *n_* = their sizes */
+int32_t b200_keyframes_surrounding_map(b200_keyframes* h, int64_t cur, double time_cur, const b200_surround_params* prm, float* corner_xyzi,
+                                       int64_t max_corner, int64_t* n_corner, float* surf_xyzi, int64_t max_surf, int64_t* n_surf);
 
 /* ------------------------------------------------------------------------- *
  * B3 (alternative) — Generalized ICP.  Replaces pclomp::GeneralizedIterativeClosestPoint<PointT, PointT>
@@ -468,6 +497,21 @@ int32_t b200_loam_optimize(b200_loam* h, const float* corner_xyz, int64_t n_corn
 /* one cornerOptimization + surfOptimization pass at t6 (parity probe) */
 int32_t b200_loam_features(b200_loam* h, const float* corner_xyz, int64_t n_corner, int64_t stride_corner, const float* surf_xyz, int64_t n_surf,
                            int64_t stride_surf, const float* t6, uint8_t* flags, float* coeff4, int32_t* n_sel);
+typedef struct {
+    int64_t n_list;                 /* surroundingKeyPosesDS entries (centroids + recent keyframes) */
+    int64_t n_kept;                 /* entries left by extractCloud's distance gate */
+    int64_t n_corner_raw, n_surf_raw; /* laserCloud{Corner,Surf}FromMap sizes */
+    int64_t n_corner, n_surf;       /* laserCloudCornerFromMapDSNum, laserCloudSurfFromMapDSNum */
+    float gpu_ms;                   /* device time of the call, selection to the last insert */
+    int32_t pad;
+} b200_surround_info;
+/* extractSurroundingKeyFrames (b200_keyframes_surrounding_map) followed by b200_loam_set_map with the two clouds, without the
+ * points leaving the device: the maps afterwards are byte for byte those b200_loam_set_map builds from the probe's clouds.
+ * The store and the handle must be on the same device.  B200_NO_EFFECTIVE_POINTS (empty store), B200_ERR_CAPACITY (a
+ * downsampled map larger than max_map_points) and the argument / range errors leave the previous maps in place.  info may be
+ * NULL. */
+int32_t b200_loam_set_map_from_keyframes(b200_loam* h, b200_keyframes* store, int64_t cur, double time_cur, const b200_surround_params* prm,
+                                         b200_surround_info* info);
 
 #ifdef __cplusplus
 }

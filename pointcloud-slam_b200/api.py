@@ -76,6 +76,18 @@ class LoopResult(C.Structure):
                 ("reg", NdtPairResult)]
 
 
+class SurroundParams(C.Structure):
+    """b200_surround_params: extractSurroundingKeyFrames' settings (surroundingKeyframeSearchRadius, surroundingKeyframeDensity,
+    mappingCornerLeafSize, mappingSurfLeafSize)."""
+    _fields_ = [("search_radius", C.c_float), ("density", C.c_float), ("corner_leaf", C.c_float), ("surf_leaf", C.c_float)]
+
+
+class SurroundInfo(C.Structure):
+    """b200_surround_info: list length before / after extractCloud's distance gate, raw and downsampled map sizes, device time."""
+    _fields_ = [("n_list", C.c_int64), ("n_kept", C.c_int64), ("n_corner_raw", C.c_int64), ("n_surf_raw", C.c_int64), ("n_corner", C.c_int64),
+                ("n_surf", C.c_int64), ("gpu_ms", C.c_float), ("pad", C.c_int32)]
+
+
 class GicpParams(C.Structure):
     _fields_ = [("k_correspondences", C.c_int32), ("gicp_epsilon", C.c_double), ("rotation_epsilon", C.c_double),
                 ("transformation_epsilon", C.c_double), ("corr_dist_threshold", C.c_double), ("max_iterations", C.c_int32),
@@ -209,6 +221,11 @@ def lib():
         L.b200_loop_detect.argtypes = [vp, vp, i64, C.POINTER(LoopParams), vp, vp]
         L.b200_loop_submap.argtypes = [vp, i64, i32, C.c_float, vp, i64, vp]
         L.b200_loop_close.argtypes = [vp, vp, vp, vp, vp, i64, C.POINTER(LoopParams), vp]
+    if hasattr(L, "b200_keyframes_add_features"):  # absent from builds older than the LOAM local map (B200REG_LIB A/B timing)
+        L.b200_keyframes_add_features.argtypes = [vp, vp, i64, i64, vp, i64, i64, vp, C.c_double, vp]
+        L.b200_keyframes_surrounding.argtypes = [vp, i64, C.c_double, C.POINTER(SurroundParams), vp, i64, vp]
+        L.b200_keyframes_surrounding_map.argtypes = [vp, i64, C.c_double, C.POINTER(SurroundParams), vp, i64, vp, vp, i64, vp]
+        L.b200_loam_set_map_from_keyframes.argtypes = [vp, vp, i64, C.c_double, C.POINTER(SurroundParams), C.POINTER(SurroundInfo)]
     L.b200_downsampler_create.argtypes = [i32, C.POINTER(vp)]
     L.b200_downsampler_destroy.argtypes = [vp]
     L.b200_voxel_downsample.argtypes = [vp, vp, i64, i64, C.c_float, i32, vp, vp, i64, vp]
@@ -907,6 +924,48 @@ class KeyframeStore:
         _check(lib().b200_loop_submap(self.h, key, search_num, leaf, _p(out), n.value, C.byref(n)))
         return out[: n.value]
 
+    _SURROUND = dict(search_radius=50.0, density=2.0, corner_leaf=0.2, surf_leaf=0.4)   # LIO-SAM's defaults
+
+    @classmethod
+    def surround_params(cls, **kw) -> SurroundParams:
+        unknown = set(kw) - set(cls._SURROUND)
+        if unknown:
+            raise TypeError(f"unknown surrounding-keyframe parameter(s): {sorted(unknown)}")
+        v = dict(cls._SURROUND, **kw)
+        return SurroundParams(v["search_radius"], v["density"], v["corner_leaf"], v["surf_leaf"])
+
+    def add_features(self, corner, surf, pose6, time) -> int:
+        """Appends a keyframe from its corner and surf clouds ([n, 3] or [n, 4] float32, lidar frame): the stored cloud is
+        corner followed by surf, as add() stores it, and the split is kept for the LOAM local map.  Returns its index."""
+        c, s = (np.ascontiguousarray(np.asarray(a, dtype=np.float32).reshape(-1, np.shape(a)[-1] if np.ndim(a) == 2 else 4)) for a in (corner, surf))
+        pose = np.ascontiguousarray(pose6, dtype=np.float32).reshape(6)
+        key = C.c_int64()
+        _check(lib().b200_keyframes_add_features(self.h, _p(c) if len(c) else None, len(c), c.strides[0], _p(s) if len(s) else None, len(s), s.strides[0],
+                                                 _p(pose), float(time), C.byref(key)))
+        return key.value
+
+    def surrounding(self, cur, time_cur, **surround):
+        """extractSurroundingKeyFrames' keyframe list after extractCloud's distance gate (int64, extraction order), keyframe cur
+        the newest (-1: the last); None for an empty store."""
+        prm = self.surround_params(**surround)
+        n = C.c_int64()
+        if _check(lib().b200_keyframes_surrounding(self.h, cur, time_cur, C.byref(prm), None, 0, C.byref(n)), soft=(0, 1)):
+            return None
+        out = np.empty(max(n.value, 1), np.int64)
+        _check(lib().b200_keyframes_surrounding(self.h, cur, time_cur, C.byref(prm), _p(out), n.value, C.byref(n)))
+        return out[: n.value]
+
+    def surrounding_map(self, cur, time_cur, **surround):
+        """laserCloudCornerFromMapDS and laserCloudSurfFromMapDS (float32 [m, 4], x y z intensity) of
+        extractSurroundingKeyFrames; None for an empty store."""
+        prm = self.surround_params(**surround)
+        nc, ns = C.c_int64(), C.c_int64()
+        if _check(lib().b200_keyframes_surrounding_map(self.h, cur, time_cur, C.byref(prm), None, 0, C.byref(nc), None, 0, C.byref(ns)), soft=(0, 1)):
+            return None
+        co, so = np.empty((max(nc.value, 1), 4), np.float32), np.empty((max(ns.value, 1), 4), np.float32)
+        _check(lib().b200_keyframes_surrounding_map(self.h, cur, time_cur, C.byref(prm), _p(co), nc.value, C.byref(nc), _p(so), ns.value, C.byref(ns)))
+        return co[: nc.value], so[: ns.value]
+
 
 class Communicator:
     """NCCL communicator over the ranks of a torch.distributed-style job (one process per GPU)."""
@@ -1261,6 +1320,13 @@ class ScanToMap:
     def setInputCloud(self, corner_map, surf_map):
         c, s = _cloud(corner_map), _cloud(surf_map)
         _check(lib().b200_loam_set_map(self.h, _p(c), c.shape[0], c.strides[0], _p(s), s.shape[0], s.strides[0]))
+
+    def extractSurroundingKeyFrames(self, store, cur, timeLaserInfoCur, **surround):
+        """extractSurroundingKeyFrames from a KeyframeStore (keyframe cur the newest, -1: the last) followed by setInputCloud,
+        the maps built and inserted on the device.  Returns the SurroundInfo, or None for an empty store (the maps stay)."""
+        info = SurroundInfo()
+        rc = lib().b200_loam_set_map_from_keyframes(self.h, store.h, cur, timeLaserInfoCur, C.byref(store.surround_params(**surround)), C.byref(info))
+        return None if _check(rc, soft=(0, 1)) else info
 
     def scan2MapOptimization(self, corner, surf, t6, iter_num=30):
         c, s = _cloud(corner), _cloud(surf)

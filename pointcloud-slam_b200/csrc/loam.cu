@@ -2,7 +2,8 @@
 //
 // Replaces, in jueying_slam/src/mapOptmization.cpp: cornerOptimization (:1255-1347), surfOptimization (:1349-1419),
 // combineOptimizationCoeffs (:1420-1440), LMOptimization (:1442-1558) and the loop of scan2MapOptimization (:1560-1590);
-// kdtree{Corner,Surf}FromMap->setInputCloud (:1568-1569) becomes b200_loam_set_map.
+// kdtree{Corner,Surf}FromMap->setInputCloud (:1568-1569) becomes b200_loam_set_map, or b200_loam_set_map_from_keyframes, which
+// builds the two maps from the device keyframe store (extractSurroundingKeyFrames, loop.cu) and inserts them from the device.
 //
 // pcl::KdTreeFLANN::nearestKSearch(pointSel, 5) followed by the gate pointSearchSqDis[4] < 1.0 is an exact 5-NN query
 // whose answer only matters when all five neighbours lie within 1 m: on a voxel index with 1 m cells that is precisely
@@ -14,6 +15,7 @@
 // plane fit, coefficient, Jacobian row; fp64 block sums of A^T A, A^T b; the last block reduces the partials in block
 // order and takes the LM step: 6x6 solve, degeneracy projection, transform update, convergence test).  The host polls a
 // done flag every few iterations.  Arithmetic is fp32 in the reference's order (TU built with -fmad=false).
+#include "loop.cuh"
 #include "map.cuh"
 #include "pointmath.cuh"
 
@@ -540,6 +542,50 @@ int32_t b200_loam_features(b200_loam* h, const float* corner_xyz, int64_t n_corn
     CUDA_TRY(cudaStreamSynchronize(h->stream));
     CUDA_TRY(cudaGetLastError());
     if (n_sel) { int s = 0; for (int64_t i = 0; i < n; ++i) s += flags[i]; *n_sel = s; }
+    return B200_OK;
+}
+
+/* extractSurroundingKeyFrames from the store + setInputCloud of both maps, the points staying on the device.  Host syncs: the
+ * keyframe list, the per-segment min / max, the run ranges (loop::surrounding), then one insert counter read per map. */
+int32_t b200_loam_set_map_from_keyframes(b200_loam* h, b200_keyframes* store, int64_t cur, double time_cur, const b200_surround_params* prm,
+                                         b200_surround_info* info) {
+    if (!h || !store) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (const int32_t rc = loop::check_surround(store, cur, time_cur, prm)) return rc;
+    if (loop::device_of(store) != h->device) B200_FAIL(B200_ERR_ARG, "keyframe store and LOAM handle are on different devices");
+    CUDA_SET_DEVICE(h->device);
+    cudaStream_t ss = loop::stream_of(store);
+    CUDA_TRY(cudaEventRecord(h->ev0, ss));
+    loop::Surround sr;
+    if (const int32_t rc = loop::surrounding(store, cur, time_cur, *prm, sr)) return rc;
+    const int64_t nc = sr.sm.count[0], ns = sr.sm.count[1];
+    if ((uint64_t)nc > h->corner.prm.max_points || (uint64_t)ns > h->surf.prm.max_points)
+        B200_FAIL(B200_ERR_CAPACITY, "feature map larger than max_map_points of b200_loam_create");
+    // the centroids are written on the store's stream; both maps read them on their own streams
+    CUDA_TRY(cudaEventRecord(h->ev_map, ss));
+    CUDA_TRY(cudaStreamWaitEvent(h->corner.stream, h->ev_map, 0));
+    CUDA_TRY(cudaStreamWaitEvent(h->surf.stream, h->ev_map, 0));
+    int32_t rc = h->corner.clear();
+    if (rc == B200_OK) rc = h->surf.clear();
+    if (rc == B200_OK && nc) rc = h->corner.insert_device(sr.sm.pts + sr.sm.first[0], nc);
+    if (rc == B200_OK && ns) rc = h->surf.insert_device(sr.sm.pts + sr.sm.first[1], ns);
+    if (rc != B200_OK) return rc;
+    CUDA_TRY(cudaEventRecord(h->ev_map, h->surf.stream));
+    CUDA_TRY(cudaStreamWaitEvent(h->corner.stream, h->ev_map, 0));
+    CUDA_TRY(cudaEventRecord(h->ev1, h->corner.stream));
+    CUDA_TRY(cudaStreamSynchronize(h->corner.stream));
+    CUDA_TRY(cudaStreamSynchronize(h->surf.stream));
+    h->have_maps = true;
+    if (info) {
+        info->n_list = sr.n_list;
+        info->n_kept = (int64_t)sr.keys.size();
+        info->n_corner_raw = sr.raw[0];
+        info->n_surf_raw = sr.raw[1];
+        info->n_corner = nc;
+        info->n_surf = ns;
+        info->gpu_ms = 0.f;
+        cudaEventElapsedTime(&info->gpu_ms, h->ev0, h->ev1);
+        info->pad = 0;
+    }
     return B200_OK;
 }
 

@@ -18,6 +18,9 @@ struct Seg {  // loopFindNearKeyframes(key, num)
     int64_t key;
     int32_t num;
 };
+struct Part {  // points begin .. begin+count-1 of keyframe kf's cloud
+    int64_t kf, begin, count;
+};
 struct GatherEntry {  // gather(): count points from pts[src ..) to dst[which][dst ..)
     int64_t src, count, dst;
     int64_t which;
@@ -41,8 +44,28 @@ int32_t detect(b200_keyframes* h, cudaStream_t s, const int64_t* cur, int64_t Q,
 // groups of `group`; the call ends after the last whole group whose leaves still fit the 64-bit sort key (at least one group).
 // Out-of-range raw sizes are the caller's: the raw points of all segments must stay below 2^31.
 int32_t submaps(b200_keyframes* h, cudaStream_t s, const Seg* segs, int64_t nseg, int64_t group, float leaf, Submaps& out);
+// The same for general segments: segment j is parts[part_off[j] .. part_off[j+1]) appended in order, downsampled with leaf[j].
+int32_t assemble(b200_keyframes* h, cudaStream_t s, const Part* parts, const int64_t* part_off, const float* leaf, int64_t nseg, int64_t group,
+                 Submaps& out);
+// loopFindNearKeyframes(key, num) as parts
+void near_parts(const b200_keyframes* h, int64_t key, int32_t num, std::vector<Part>& parts);
 // e[0 .. n) from pts into dst0 / dst1 as (x, y, z, 0) records, one launch on stream s
 int32_t gather(b200_keyframes* h, cudaStream_t s, const float4* pts, const GatherEntry* e, int64_t n, float4* dst0, float4* dst1);
+cudaStream_t stream_of(const b200_keyframes* h);
+
+// extractSurroundingKeyFrames from the store (arguments checked by check_surround; cur = -1: the last keyframe): the keyframe
+// list after extractCloud's distance gate, and the corner map (segment 0) and surf map (segment 1) downsampled with their
+// leaves in out.sm.  One read-back of its own (the list; a list past 4096 entries takes one more copy) plus the two of
+// assemble.  B200_NO_EFFECTIVE_POINTS on an empty store; a keyframe without a corner / surf split is B200_ERR_ARG; a
+// key-pose or map grid out of range is B200_ERR_RANGE.
+struct Surround {
+    std::vector<int64_t> keys;  // the list after the gate, in extraction order
+    int64_t n_list = 0;         // its length before the gate
+    int64_t raw[2] = {0, 0};    // laserCloud{Corner,Surf}FromMap sizes
+    Submaps sm;
+};
+int32_t check_surround(const b200_keyframes* h, int64_t cur, double time_cur, const b200_surround_params* prm);
+int32_t surrounding(b200_keyframes* h, int64_t cur, double time_cur, const b200_surround_params& prm, Surround& out);
 
 }  // namespace loop
 }  // namespace b200

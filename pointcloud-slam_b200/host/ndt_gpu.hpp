@@ -236,12 +236,15 @@ class KeyframeStore {
     KeyframeStore(const KeyframeStore&) = delete;
     KeyframeStore& operator=(const KeyframeStore&) = delete;
 
+    /// the corner / surf split is kept for ScanToMap::extractSurroundingKeyFrames (b200_keyframes_add_features)
     int64_t add(const CloudT& corner, const CloudT& surf, const float pose6[6], double time) {
         xyzi_.clear();
         for (const CloudT* c : {&corner, &surf})
             for (const auto& q : c->points) { xyzi_.push_back(q.x); xyzi_.push_back(q.y); xyzi_.push_back(q.z); xyzi_.push_back(q.intensity); }
+        const int64_t nc = (int64_t)corner.points.size(), ns = (int64_t)surf.points.size();
         int64_t key = -1;
-        check(b200_keyframes_add(h_, xyzi_.empty() ? nullptr : xyzi_.data(), (int64_t)xyzi_.size() / 4, 16, pose6, time, &key), "b200_keyframes_add");
+        check(b200_keyframes_add_features(h_, nc ? xyzi_.data() : nullptr, nc, 16, ns ? xyzi_.data() + 4 * nc : nullptr, ns, 16, pose6, time, &key),
+              "b200_keyframes_add_features");
         return key;
     }
     void setPoses(int64_t first, int64_t count, const float* poses6) { check(b200_keyframes_set_poses(h_, first, count, poses6), "b200_keyframes_set_poses"); }

@@ -24,6 +24,15 @@ class ScanToMap {
                                 surf_map.points.empty() ? nullptr : &surf_map.points[0].x, (int64_t)surf_map.points.size(), sizeof(P)),
               "b200_loam_set_map");
     }
+    /// extractSurroundingKeyFrames from a device keyframe store (b200host::KeyframeStore, ndt_gpu.hpp; cur = -1: its last keyframe)
+    /// followed by setInputCloud, the two maps never leaving the device; false when the store is empty (the maps stay)
+    template <class Store>
+    bool extractSurroundingKeyFrames(Store& store, int64_t cur, double timeLaserInfoCur, const b200_surround_params& params) {
+        const int32_t rc = b200_loam_set_map_from_keyframes(h_, store.handle(), cur, timeLaserInfoCur, &params, &info_);
+        check(rc, "b200_loam_set_map_from_keyframes");
+        return rc == B200_OK;
+    }
+    const b200_surround_info& surroundInfo() const { return info_; }
     /// the iterCount loop of scan2MapOptimization; returns LMOptimization's convergence flag, isDegenerate in degenerate()
     bool scan2MapOptimization(const CloudT& corner_last_ds, const CloudT& surf_last_ds, float transformTobeMapped[6], int iter_num = 30) {
         using P = typename std::remove_reference<decltype(corner_last_ds.points[0])>::type;
@@ -39,6 +48,7 @@ class ScanToMap {
    private:
     b200_loam* h_ = nullptr;
     b200_loam_stats stats_{};
+    b200_surround_info info_{};
 };
 
 /// raw scan -> (undistort) -> voxel downsample, result left on the device for Esekf::update on device points
