@@ -513,6 +513,66 @@ typedef struct {
 int32_t b200_loam_set_map_from_keyframes(b200_loam* h, b200_keyframes* store, int64_t cur, double time_cur, const b200_surround_params* prm,
                                          b200_surround_info* info);
 
+/* the scan-to-map optimisation on clouds that already sit on the device (float4 x y z intensity records, b200_features_device_cloud):
+ * b200_loam_optimize with a device copy in place of the pack and upload; the same t6 bits and stats.  Buffers on another device
+ * than the handle are B200_ERR_ARG. */
+int32_t b200_loam_optimize_device(b200_loam* h, const void* d_corner, int64_t n_corner, const void* d_surf, int64_t n_surf, float* t6, int32_t iter_num,
+                                  b200_loam_stats* stats);
+/* b200_keyframes_add_features from device clouds (float4 x y z intensity): stores the bytes b200_keyframes_add_features stores
+ * for their host copies at a stride of 16 bytes.  Buffers on another device than the store are B200_ERR_ARG. */
+int32_t b200_keyframes_add_features_device(b200_keyframes* h, const void* d_corner, int64_t n_corner, const void* d_surf, int64_t n_surf,
+                                           const float* pose6, double time, int64_t* key);
+
+/* ------------------------------------------------------------------------- *
+ * LOAM front end (LIO-SAM imageProjection without deskew, featureExtraction, mapOptimization's downsampleCurrentScan), the
+ * contract restated in oracle/feature_oracle.cpp.  One scan per call on one device.
+ * ------------------------------------------------------------------------- */
+typedef struct b200_features b200_features;
+typedef struct {
+    int32_t n_scan;          /* N_SCAN, 1 .. 1024 */
+    int32_t horizon_scan;    /* Horizon_SCAN; n_scan * horizon_scan <= 2^26 */
+    int32_t downsample_rate; /* >= 1 */
+    int32_t sensor;          /* 0: velodyne / ouster (column from the azimuth), 1: livox (column = arrival order in the line) */
+    float min_range, max_range;          /* lidarMinRange, lidarMaxRange */
+    float edge_threshold, surf_threshold; /* edgeThreshold, surfThreshold */
+    float odometry_surf_leaf;            /* odometrySurfLeafSize (per-ring surf VoxelGrid) */
+    float mapping_corner_leaf, mapping_surf_leaf; /* downsampleCurrentScan */
+    int32_t pad;
+} b200_feature_params;
+typedef struct {
+    int64_t n_in;
+    int64_t dropped_nonfinite, dropped_range, dropped_row, dropped_col, dropped_dup;
+    int64_t n_extracted;                /* extracted cloud (cloud_info) */
+    int64_t n_corner, n_surface;        /* cornerCloud, surfaceCloud */
+    int64_t n_corner_ds, n_surf_ds;     /* laserCloud{Corner,Surf}LastDS */
+    float gpu_ms;                       /* device time of the call, upload to the last downsample */
+    int32_t pad;
+} b200_feature_info;
+#define B200_FEATURES_CORNER 0
+#define B200_FEATURES_SURFACE 1
+#define B200_FEATURES_CORNER_DS 2
+#define B200_FEATURES_SURF_DS 3
+/* parameters out of bounds are B200_ERR_ARG */
+int32_t b200_features_create(const b200_feature_params* prm, int32_t device, b200_features** out);
+int32_t b200_features_destroy(b200_features* h);
+/* steps 1-6 for one scan: n records of stride bytes (a multiple of 4; x y z the first three floats), the intensity a float at
+ * intensity_offset (< 0: none, 0 is used), the ring an unsigned integer of ring_bytes (1 or 2) at ring_offset.  One upload of
+ * the scan; synchronises before it returns.  An empty extracted cloud is B200_NO_EFFECTIVE_POINTS with empty clouds; a
+ * VoxelGrid of more than 9e18 leaves is B200_ERR_RANGE.  info may be NULL. */
+int32_t b200_features_extract(b200_features* h, const void* points, int64_t n, int64_t stride, int64_t intensity_offset, int64_t ring_offset,
+                              int32_t ring_bytes, b200_feature_info* info);
+/* parity probes of the last extract (any output may be NULL; *n the full size, at most max written): the extracted cloud (x y z
+ * intensity), pointColInd, pointRange, start / endRingIndex (n_scan each); curvature, label, picked flags */
+int32_t b200_features_cloud_info(b200_features* h, float* cloud_xyzi, int32_t* col, float* range, int32_t* start_ring, int32_t* end_ring, int64_t max,
+                                 int64_t* n);
+int32_t b200_features_labels(b200_features* h, float* curvature, int8_t* label, uint8_t* picked, int64_t max, int64_t* n);
+/* cornerCloud (pick order), surfaceCloud, or the two DS clouds (which = B200_FEATURES_*), x y z intensity */
+int32_t b200_features_cloud(b200_features* h, int32_t which, float* out_xyzi, int64_t max, int64_t* n);
+/* the same cloud as it sits on the device (float4 per point), valid until the next extract: pass it to
+ * b200_loam_optimize_device / b200_keyframes_add_features_device */
+const void* b200_features_device_cloud(b200_features* h, int32_t which, int64_t* n);
+int32_t b200_features_device(b200_features* h);
+
 #ifdef __cplusplus
 }
 #endif

@@ -105,6 +105,17 @@ class LoamStats(C.Structure):
                 ("AtA_first", C.c_double * 36)]
 
 
+class FeatureParams(C.Structure):
+    _fields_ = [("n_scan", C.c_int32), ("horizon_scan", C.c_int32), ("downsample_rate", C.c_int32), ("sensor", C.c_int32), ("min_range", C.c_float),
+                ("max_range", C.c_float), ("edge_threshold", C.c_float), ("surf_threshold", C.c_float), ("odometry_surf_leaf", C.c_float),
+                ("mapping_corner_leaf", C.c_float), ("mapping_surf_leaf", C.c_float), ("pad", C.c_int32)]
+
+
+class FeatureInfo(C.Structure):
+    _fields_ = [(k, C.c_int64) for k in ("n_in", "dropped_nonfinite", "dropped_range", "dropped_row", "dropped_col", "dropped_dup", "n_extracted",
+                                         "n_corner", "n_surface", "n_corner_ds", "n_surf_ds")] + [("gpu_ms", C.c_float), ("pad", C.c_int32)]
+
+
 def lib_path() -> str:
     # B200REG_LIB: development override for A/B timing of two builds of the SAME engine (never a different implementation)
     return os.environ.get("B200REG_LIB") or os.path.join(_HERE, "libb200reg.so")
@@ -221,6 +232,17 @@ def lib():
         L.b200_loop_detect.argtypes = [vp, vp, i64, C.POINTER(LoopParams), vp, vp]
         L.b200_loop_submap.argtypes = [vp, i64, i32, C.c_float, vp, i64, vp]
         L.b200_loop_close.argtypes = [vp, vp, vp, vp, vp, i64, C.POINTER(LoopParams), vp]
+    if hasattr(L, "b200_features_create"):  # absent from builds older than the LOAM front end (B200REG_LIB A/B timing)
+        L.b200_features_create.argtypes = [C.POINTER(FeatureParams), i32, C.POINTER(vp)]
+        L.b200_features_destroy.argtypes = [vp]
+        L.b200_features_extract.argtypes = [vp, vp, i64, i64, i64, i64, i32, C.POINTER(FeatureInfo)]
+        L.b200_features_cloud_info.argtypes = [vp, vp, vp, vp, vp, vp, i64, vp]
+        L.b200_features_labels.argtypes = [vp, vp, vp, vp, i64, vp]
+        L.b200_features_cloud.argtypes = [vp, i32, vp, i64, vp]
+        L.b200_features_device_cloud.restype = vp
+        L.b200_features_device_cloud.argtypes = [vp, i32, vp]
+        L.b200_loam_optimize_device.argtypes = [vp, vp, i64, vp, i64, vp, i32, C.POINTER(LoamStats)]
+        L.b200_keyframes_add_features_device.argtypes = [vp, vp, i64, vp, i64, vp, C.c_double, vp]
     if hasattr(L, "b200_keyframes_add_features"):  # absent from builds older than the LOAM local map (B200REG_LIB A/B timing)
         L.b200_keyframes_add_features.argtypes = [vp, vp, i64, i64, vp, i64, i64, vp, C.c_double, vp]
         L.b200_keyframes_surrounding.argtypes = [vp, i64, C.c_double, C.POINTER(SurroundParams), vp, i64, vp]
@@ -944,6 +966,14 @@ class KeyframeStore:
                                                  _p(pose), float(time), C.byref(key)))
         return key.value
 
+    def add_features_device(self, corner, surf, pose6, time) -> int:
+        """add_features from device clouds: corner / surf = (device pointer, n) of float4 records, as FeatureExtraction.device_cloud
+        returns them.  Stores what add_features stores for their host copies.  Returns the keyframe index."""
+        pose = np.ascontiguousarray(pose6, dtype=np.float32).reshape(6)
+        key = C.c_int64()
+        _check(lib().b200_keyframes_add_features_device(self.h, corner[0], corner[1], surf[0], surf[1], _p(pose), float(time), C.byref(key)))
+        return key.value
+
     def surrounding(self, cur, time_cur, **surround):
         """extractSurroundingKeyFrames' keyframe list after extractCloud's distance gate (int64, extraction order), keyframe cur
         the newest (-1: the last); None for an empty store."""
@@ -1335,6 +1365,13 @@ class ScanToMap:
         _check(rc, soft=(0, 2))
         return t, rc
 
+    def scan2MapOptimization_device(self, corner, surf, t6, iter_num=30):
+        """scan2MapOptimization on device clouds: corner / surf = (device pointer, n) of float4 records (FeatureExtraction.device_cloud)."""
+        t = np.array(t6, dtype=np.float32)
+        rc = lib().b200_loam_optimize_device(self.h, corner[0], corner[1], surf[0], surf[1], _p(t), iter_num, C.byref(self.stats))
+        _check(rc, soft=(0, 2))
+        return t, rc
+
     def features(self, corner, surf, t6):
         c, s = _cloud(corner), _cloud(surf)
         t = np.ascontiguousarray(t6, dtype=np.float32)
@@ -1344,6 +1381,75 @@ class ScanToMap:
         nsel = C.c_int32(0)
         _check(lib().b200_loam_features(self.h, _p(c), c.shape[0], c.strides[0], _p(s), s.shape[0], s.strides[0], _p(t), _p(flags), _p(coeff), C.byref(nsel)))
         return nsel.value, flags, coeff
+
+
+class FeatureExtraction:
+    """LIO-SAM's imageProjection (projection and cloud extraction, no deskew), featureExtraction and mapOptimization's
+    downsampleCurrentScan on the GPU (b200_features_*), the contract restated in oracle/feature_oracle.cpp.  Parameters take
+    LIO-SAM's names and defaults; sensor 0 = velodyne / ouster, 1 = livox."""
+
+    CORNER, SURFACE, CORNER_DS, SURF_DS = 0, 1, 2, 3
+    _DEFAULTS = dict(n_scan=16, horizon_scan=1800, downsample_rate=1, sensor=0, min_range=1.0, max_range=1000.0, edge_threshold=1.0,
+                     surf_threshold=0.1, odometry_surf_leaf=0.4, mapping_corner_leaf=0.2, mapping_surf_leaf=0.4)
+
+    def __init__(self, device=0, **prm):
+        unknown = set(prm) - set(self._DEFAULTS)
+        if unknown:
+            raise TypeError(f"unknown feature parameter(s): {sorted(unknown)}")
+        self.prm = dict(self._DEFAULTS, **prm)
+        self.device = device
+        self.h = C.c_void_p()
+        self.info = FeatureInfo()
+        _check(lib().b200_features_create(C.byref(FeatureParams(**self.prm)), device, C.byref(self.h)))
+
+    def close(self):
+        if getattr(self, "h", None):
+            try:
+                lib().b200_features_destroy(self.h)
+            except TypeError:  # interpreter shutdown: module globals are already torn down
+                pass
+            self.h = None
+
+    __del__ = close
+
+    def extract(self, records, stride, intensity_offset, ring_offset, ring_bytes):
+        """Steps 1-6 for one scan of raw records (a uint8 / structured array of stride-byte records): returns the status
+        (0, or 1 = B200_NO_EFFECTIVE_POINTS for an empty extracted cloud); self.info holds the counts and the device time."""
+        rec = np.ascontiguousarray(records)
+        n = rec.nbytes // stride
+        return _check(lib().b200_features_extract(self.h, _p(rec) if n else None, n, stride, intensity_offset, ring_offset, ring_bytes,
+                                                  C.byref(self.info)), soft=(0, 1))
+
+    def cloud_info(self):
+        """(extracted cloud [m, 4], pointColInd, pointRange, startRingIndex, endRingIndex) of the last extract."""
+        m = int(self.info.n_extracted)
+        cloud, col, rng = np.zeros((m, 4), np.float32), np.zeros(m, np.int32), np.zeros(m, np.float32)
+        start, end = np.zeros(self.prm["n_scan"], np.int32), np.zeros(self.prm["n_scan"], np.int32)
+        n = C.c_int64()
+        _check(lib().b200_features_cloud_info(self.h, _p(cloud), _p(col), _p(rng), _p(start), _p(end), m, C.byref(n)))
+        return cloud, col, rng, start, end
+
+    def labels(self):
+        """(curvature, label, picked) of the last extract."""
+        m = int(self.info.n_extracted)
+        curv, label, picked = np.zeros(m, np.float32), np.zeros(m, np.int8), np.zeros(m, np.uint8)
+        n = C.c_int64()
+        _check(lib().b200_features_labels(self.h, _p(curv), _p(label), _p(picked), m, C.byref(n)))
+        return curv, label, picked
+
+    def cloud(self, which):
+        """cornerCloud, surfaceCloud, laserCloudCornerLastDS or laserCloudSurfLastDS ([n, 4] x y z intensity)."""
+        n = C.c_int64()
+        lib().b200_features_device_cloud(self.h, which, C.byref(n))
+        out = np.zeros((n.value, 4), np.float32)
+        _check(lib().b200_features_cloud(self.h, which, _p(out), n.value, C.byref(n)))
+        return out
+
+    def device_cloud(self, which):
+        """(device pointer, n) of a cloud of the last extract, valid until the next extract."""
+        n = C.c_int64()
+        ptr = lib().b200_features_device_cloud(self.h, which, C.byref(n))
+        return ptr, n.value
 
 
 class GeneralizedIterativeClosestPoint:

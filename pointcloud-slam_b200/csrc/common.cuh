@@ -153,6 +153,18 @@ __host__ __device__ inline uint32_t hash_key(uint64_t k) {  // 32-bit multiply-x
 __host__ __device__ inline uint32_t next_slot(uint32_t slot, uint32_t tmask) { return (slot + 9u) & tmask; }
 
 // Pass a strided host cloud through a pinned staging buffer as packed float4 (x,y,z,0).
+// a caller's device buffer: B200_ERR_ARG unless it is device memory of `device` (n == 0 needs no buffer)
+inline int32_t check_device_buffer(const void* p, int64_t n, int device) {
+    if (n == 0) return B200_OK;
+    cudaPointerAttributes a{};
+    if (!p || cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        cudaGetLastError();
+        B200_FAIL(B200_ERR_ARG, "not a device buffer");
+    }
+    if (a.type != cudaMemoryTypeDevice || a.device != device) B200_FAIL(B200_ERR_ARG, "buffer is not on the handle's device");
+    return B200_OK;
+}
+
 inline void pack_xyz_float4(const float* xyz, int64_t n, int64_t stride, float4* dst) {
     const char* src = (const char*)xyz;
     for (int64_t i = 0; i < n; ++i) {

@@ -399,6 +399,27 @@ static int32_t loam_stage(b200_loam* h, const float* corner, int64_t nc, int64_t
     return B200_OK;
 }
 
+// the device-resident twin of pack_xyz_float4: (x, y, z, 0)
+__global__ void k_loam_stage_device(const float4* __restrict__ c, int64_t nc, const float4* __restrict__ s, int64_t n, float4* __restrict__ out) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const float4 p = i < nc ? c[i] : s[i - nc];
+    out[i] = make_float4(p.x, p.y, p.z, 0.0f);
+}
+static int32_t loam_stage_device(b200_loam* h, const float4* corner, int64_t nc, const float4* surf, int64_t ns, const float* t6, int max_iter) {
+    const int64_t n = nc + ns;
+    CUDA_TRY(h->d_pts.reserve(n)); CUDA_TRY(h->d_nb.reserve(n * 5)); CUDA_TRY(h->d_cnt.reserve(n));
+    CUDA_TRY(h->d_t6.reserve(8)); CUDA_TRY(h->h_t6.reserve(8));
+    memcpy(h->h_t6.p, t6, 6 * sizeof(float));
+    k_loam_stage_device<<<(unsigned)((n + 255) / 256), 256, 0, h->stream>>>(corner, nc, surf, n, h->d_pts.p);
+    CUDA_TRY(cudaMemcpyAsync(h->d_t6.p, h->h_t6.p, 6 * sizeof(float), cudaMemcpyHostToDevice, h->stream));
+    loam::k_loam_init<<<1, 32, 0, h->stream>>>(h->d_ctl, h->d_t6.p, max_iter);
+    LAUNCH_COUNT(2);
+    return B200_OK;
+}
+
+static int32_t loam_iterate(b200_loam* h, int64_t n_corner, int64_t n_surf, float* t6, int32_t iter_num, b200_loam_stats* stats);
+
 static void loam_search(b200_loam* h, int64_t nc, int64_t ns) {
     using namespace loam;
     if (nc) {
@@ -490,6 +511,24 @@ int32_t b200_loam_optimize(b200_loam* h, const float* corner_xyz, int64_t n_corn
     CUDA_SET_DEVICE(h->device);
     int32_t rc = loam_stage(h, corner_xyz, n_corner, stride_corner, surf_xyz, n_surf, stride_surf, t6, iter_num);
     if (rc) return rc;
+    return loam_iterate(h, n_corner, n_surf, t6, iter_num, stats);
+}
+int32_t b200_loam_optimize_device(b200_loam* h, const void* d_corner, int64_t n_corner, const void* d_surf, int64_t n_surf, float* t6, int32_t iter_num,
+                                  b200_loam_stats* stats) {
+    if (!h || !t6 || n_corner < 0 || n_surf < 0 || n_corner + n_surf < 1 || iter_num < 1 || iter_num > 1000 || n_corner + n_surf > (1 << 26))
+        B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (!h->have_maps) B200_FAIL(B200_ERR_ARG, "no feature maps set");
+    CUDA_SET_DEVICE(h->device);
+    if (const int32_t rc = check_device_buffer(d_corner, n_corner, h->device)) return rc;
+    if (const int32_t rc = check_device_buffer(d_surf, n_surf, h->device)) return rc;
+    const int32_t rc = loam_stage_device(h, (const float4*)d_corner, n_corner, (const float4*)d_surf, n_surf, t6, iter_num);
+    if (rc) return rc;
+    return loam_iterate(h, n_corner, n_surf, t6, iter_num, stats);
+}
+}  // extern "C"
+
+// the loop of scan2MapOptimization on the staged scan
+static int32_t loam_iterate(b200_loam* h, int64_t n_corner, int64_t n_surf, float* t6, int32_t iter_num, b200_loam_stats* stats) {
     const int64_t n = n_corner + n_surf;
     const int nbx = (int)std::min<int64_t>((n + loam::ACC_THREADS - 1) / loam::ACC_THREADS, loam::MAXB);
     CUDA_TRY(cudaEventRecord(h->ev0, h->stream));
@@ -521,6 +560,8 @@ int32_t b200_loam_optimize(b200_loam* h, const float* corner_xyz, int64_t n_corn
     }
     return c.converged ? B200_OK : B200_NOT_CONVERGED;
 }
+
+extern "C" {
 /* one cornerOptimization + surfOptimization pass at t6 (parity probe): flags[n_corner + n_surf], coeff4[(n_corner + n_surf) * 4];
  * *n_sel = number of selected features */
 int32_t b200_loam_features(b200_loam* h, const float* corner_xyz, int64_t n_corner, int64_t stride_corner, const float* surf_xyz, int64_t n_surf,

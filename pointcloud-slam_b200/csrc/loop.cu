@@ -292,7 +292,7 @@ __global__ void __launch_bounds__(1024) k_surr_list(const KfRec* __restrict__ re
 using namespace b200;
 using namespace b200::loop;
 
-struct b200_keyframes {
+struct b200_keyframes : loop::SegWork {
     int device = 0;
     cudaStream_t stream = nullptr;
     float4* d_pool = nullptr;  // keyframe clouds end to end; grows by doubling
@@ -303,17 +303,9 @@ struct b200_keyframes {
     std::vector<int64_t> n_corner;  // corner points at the head of each cloud (b200_keyframes_add_features); -1: no split
     PinnedBuf<float4> h_stage;
     PinnedBuf<KfRec> h_rec;
-    // detection and submap scratch
-    PinnedBuf<uint8_t> h_tab;
-    DevBuf<uint8_t> d_tab;
-    DevBuf<int64_t> d_io;
-    PinnedBuf<int64_t> h_io;
-    DevBuf<float4> d_raw, d_cent;
-    DevBuf<int32_t> d_mm;
-    PinnedBuf<int32_t> h_mm;
-    DevBuf<unsigned long long> k_in, k_out, k_uniq, d_cells;
-    DevBuf<int32_t> v_in, v_out, run_cnt, run_off, d_cnt, d_small;
-    DevBuf<uint8_t> keep, cub_tmp;
+    // detection and submap scratch (the rest is SegWork's)
+    DevBuf<float4> d_raw;
+    DevBuf<unsigned long long> d_cells;
     // local-map selection scratch
     DevBuf<float4> d_kpos;
     DevBuf<int64_t> d_sel;
@@ -416,15 +408,23 @@ int32_t assemble(b200_keyframes* h, cudaStream_t s, const Part* parts, const int
         k_loop_assemble<<<(unsigned)ent.size(), 256, 0, s>>>(h->d_pool, h->d_rec.p, (const AsmEntry*)(h->d_tab.p + off_bytes), h->d_raw.p);
         LAUNCH_COUNT(1);
     }
+    return seg_downsample(*h, s, h->d_raw.p, d_off, off.data(), off_bytes, leaf, nseg, group, out);
+}
+
+int32_t seg_downsample(SegWork& w, cudaStream_t s, const float4* pts, const int64_t* d_off, const int64_t* off, size_t grid_at, const float* leaf,
+                       int64_t nseg, int64_t group, Submaps& out) {
+    const size_t off_bytes = grid_at;
+    CUDA_TRY(w.h_tab.reserve(grid_at + nseg * (sizeof(SegGrid) + sizeof(unsigned long long))));
+    CUDA_TRY(w.d_tab.reserve(grid_at + nseg * (sizeof(SegGrid) + sizeof(unsigned long long))));
     // per-segment min / max, read back once
     int64_t max_n = 1;
     for (int64_t j = 0; j < nseg; ++j) max_n = std::max(max_n, off[j + 1] - off[j]);
-    CUDA_TRY(h->d_mm.reserve(6 * (size_t)nseg));
-    CUDA_TRY(h->h_mm.reserve(6 * (size_t)nseg));
-    ndt::k_ndt_minmax_init<<<(unsigned)((6 * nseg + 255) / 256), 256, 0, s>>>(h->d_mm.p, (int)nseg);
-    ndt::k_ndt_minmax<<<dim3((unsigned)std::min<int64_t>((max_n + 1023) / 1024, 256), (unsigned)nseg), 256, 0, s>>>(h->d_raw.p, d_off, h->d_mm.p);
+    CUDA_TRY(w.d_mm.reserve(6 * (size_t)nseg));
+    CUDA_TRY(w.h_mm.reserve(6 * (size_t)nseg));
+    ndt::k_ndt_minmax_init<<<(unsigned)((6 * nseg + 255) / 256), 256, 0, s>>>(w.d_mm.p, (int)nseg);
+    ndt::k_ndt_minmax<<<dim3((unsigned)std::min<int64_t>((max_n + 1023) / 1024, 256), (unsigned)nseg), 256, 0, s>>>(pts, d_off, w.d_mm.p);
     LAUNCH_COUNT(2);
-    CUDA_TRY(cudaMemcpyAsync(h->h_mm.p, h->d_mm.p, 6 * nseg * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(w.h_mm.p, w.d_mm.p, 6 * nseg * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     CUDA_TRY(cudaGetLastError());
     // every segment's grid as b200_voxel_downsample derives it; the cell ranges end to end
@@ -443,7 +443,7 @@ int32_t assemble(b200_keyframes* h, cudaStream_t s, const Part* parts, const int
             SegGrid& q = sg[j];
             memset(&q, 0, sizeof q);
             const std::string err = g_last_error;
-            out.status[j] = vox::grid_from_minmax(h->h_mm.p + 6 * j, leaf[j], g, cells[j]);
+            out.status[j] = vox::grid_from_minmax(w.h_mm.p + 6 * j, leaf[j], g, cells[j]);
             if (out.status[j]) { g_last_error = err; cells[j] = 0; continue; }  // reported in the segment's status
             for (int k = 0; k < 3; ++k) { q.min_b[k] = g.min_b[k]; q.div_b[k] = g.div_b[k]; }
             q.inv_leaf = 1.0f / leaf[j];
@@ -462,43 +462,43 @@ int32_t assemble(b200_keyframes* h, cudaStream_t s, const Part* parts, const int
     while (end_bit < 64 && (1ull << end_bit) <= sentinel) ++end_bit;
     // the grids replace the keyframe table (consumed by k_loop_assemble, which precedes on the stream)
     CUDA_TRY(cudaStreamSynchronize(s));
-    memcpy(h->h_tab.p + off_bytes, sg.data(), done * sizeof(SegGrid));
-    memcpy(h->h_tab.p + off_bytes + done * sizeof(SegGrid), cells.data(), done * sizeof(unsigned long long));
-    CUDA_TRY(cudaMemcpyAsync(h->d_tab.p + off_bytes, h->h_tab.p + off_bytes, done * (sizeof(SegGrid) + sizeof(unsigned long long)), cudaMemcpyHostToDevice, s));
-    const SegGrid* d_sg = (const SegGrid*)(h->d_tab.p + off_bytes);
-    const unsigned long long* d_cells = (const unsigned long long*)(h->d_tab.p + off_bytes + done * sizeof(SegGrid));
-    CUDA_TRY(h->k_in.reserve(n)); CUDA_TRY(h->k_out.reserve(n)); CUDA_TRY(h->k_uniq.reserve(n));
-    CUDA_TRY(h->v_in.reserve(n)); CUDA_TRY(h->v_out.reserve(n)); CUDA_TRY(h->run_cnt.reserve(n)); CUDA_TRY(h->run_off.reserve(n));
-    CUDA_TRY(h->d_cent.reserve(n)); CUDA_TRY(h->d_cnt.reserve(n)); CUDA_TRY(h->keep.reserve(n)); CUDA_TRY(h->d_small.reserve(4));
-    CUDA_TRY(h->d_io.reserve(2 * (size_t)done)); CUDA_TRY(h->h_io.reserve(2 * (size_t)done));
-    k_loop_keys<<<dim3((unsigned)std::min<int64_t>((max_n + 255) / 256, 1024), (unsigned)done), 256, 0, s>>>(h->d_raw.p, d_off, d_sg, sentinel, h->k_in.p,
-                                                                                                          h->v_in.p);
-    int32_t* d_nruns = h->d_small.p;
+    memcpy(w.h_tab.p + off_bytes, sg.data(), done * sizeof(SegGrid));
+    memcpy(w.h_tab.p + off_bytes + done * sizeof(SegGrid), cells.data(), done * sizeof(unsigned long long));
+    CUDA_TRY(cudaMemcpyAsync(w.d_tab.p + off_bytes, w.h_tab.p + off_bytes, done * (sizeof(SegGrid) + sizeof(unsigned long long)), cudaMemcpyHostToDevice, s));
+    const SegGrid* d_sg = (const SegGrid*)(w.d_tab.p + off_bytes);
+    const unsigned long long* d_cells = (const unsigned long long*)(w.d_tab.p + off_bytes + done * sizeof(SegGrid));
+    CUDA_TRY(w.k_in.reserve(n)); CUDA_TRY(w.k_out.reserve(n)); CUDA_TRY(w.k_uniq.reserve(n));
+    CUDA_TRY(w.v_in.reserve(n)); CUDA_TRY(w.v_out.reserve(n)); CUDA_TRY(w.run_cnt.reserve(n)); CUDA_TRY(w.run_off.reserve(n));
+    CUDA_TRY(w.d_cent.reserve(n)); CUDA_TRY(w.d_cnt.reserve(n)); CUDA_TRY(w.keep.reserve(n)); CUDA_TRY(w.d_small.reserve(4));
+    CUDA_TRY(w.d_io.reserve(2 * (size_t)done)); CUDA_TRY(w.h_io.reserve(2 * (size_t)done));
+    k_loop_keys<<<dim3((unsigned)std::min<int64_t>((max_n + 255) / 256, 1024), (unsigned)done), 256, 0, s>>>(pts, d_off, d_sg, sentinel, w.k_in.p,
+                                                                                                          w.v_in.p);
+    int32_t* d_nruns = w.d_small.p;
     size_t t1 = 0, t2 = 0, t3 = 0;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, t1, h->k_in.p, h->k_out.p, h->v_in.p, h->v_out.p, (int)n, 0, end_bit, s));
-    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, t2, h->k_out.p, h->k_uniq.p, h->run_cnt.p, d_nruns, (int)n, s));
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, t3, h->run_cnt.p, h->run_off.p, (int)n, s));
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(nullptr, t1, w.k_in.p, w.k_out.p, w.v_in.p, w.v_out.p, (int)n, 0, end_bit, s));
+    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(nullptr, t2, w.k_out.p, w.k_uniq.p, w.run_cnt.p, d_nruns, (int)n, s));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(nullptr, t3, w.run_cnt.p, w.run_off.p, (int)n, s));
     const size_t tmp = std::max(t1, std::max(t2, t3));
-    CUDA_TRY(h->cub_tmp.reserve(tmp));
+    CUDA_TRY(w.cub_tmp.reserve(tmp));
     size_t tt = tmp;
-    CUDA_TRY(cub::DeviceRadixSort::SortPairs(h->cub_tmp.p, tt, h->k_in.p, h->k_out.p, h->v_in.p, h->v_out.p, (int)n, 0, end_bit, s));
+    CUDA_TRY(cub::DeviceRadixSort::SortPairs(w.cub_tmp.p, tt, w.k_in.p, w.k_out.p, w.v_in.p, w.v_out.p, (int)n, 0, end_bit, s));
     tt = tmp;
-    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(h->cub_tmp.p, tt, h->k_out.p, h->k_uniq.p, h->run_cnt.p, d_nruns, (int)n, s));
+    CUDA_TRY(cub::DeviceRunLengthEncode::Encode(w.cub_tmp.p, tt, w.k_out.p, w.k_uniq.p, w.run_cnt.p, d_nruns, (int)n, s));
     tt = tmp;
-    CUDA_TRY(cub::DeviceScan::ExclusiveSum(h->cub_tmp.p, tt, h->run_cnt.p, h->run_off.p, (int)n, s));
+    CUDA_TRY(cub::DeviceScan::ExclusiveSum(w.cub_tmp.p, tt, w.run_cnt.p, w.run_off.p, (int)n, s));
     const unsigned nb = (unsigned)((n + 255) / 256);
-    vox::k_centroids<<<nb, 256, 0, s>>>(h->d_raw.p, h->v_out.p, h->k_uniq.p, h->run_off.p, h->run_cnt.p, d_nruns, sentinel, 0, h->d_cent.p, h->d_cnt.p,
-                                        h->keep.p);
-    k_loop_seg_runs<<<(unsigned)((done + 255) / 256), 256, 0, s>>>(h->k_uniq.p, d_nruns, d_sg, d_cells, (int)done, h->d_io.p);
+    vox::k_centroids<<<nb, 256, 0, s>>>(pts, w.v_out.p, w.k_uniq.p, w.run_off.p, w.run_cnt.p, d_nruns, sentinel, 0, w.d_cent.p, w.d_cnt.p,
+                                        w.keep.p);
+    k_loop_seg_runs<<<(unsigned)((done + 255) / 256), 256, 0, s>>>(w.k_uniq.p, d_nruns, d_sg, d_cells, (int)done, w.d_io.p);
     LAUNCH_COUNT(3);
-    CUDA_TRY(cudaMemcpyAsync(h->h_io.p, h->d_io.p, 2 * done * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
+    CUDA_TRY(cudaMemcpyAsync(w.h_io.p, w.d_io.p, 2 * done * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
     CUDA_TRY(cudaStreamSynchronize(s));
     CUDA_TRY(cudaGetLastError());
     for (int64_t j = 0; j < done; ++j) {
-        out.first[j] = h->h_io.p[2 * j];
-        out.count[j] = h->h_io.p[2 * j + 1];
+        out.first[j] = w.h_io.p[2 * j];
+        out.count[j] = w.h_io.p[2 * j + 1];
     }
-    out.pts = h->d_cent.p;
+    out.pts = w.d_cent.p;
     return B200_OK;
 }
 
@@ -640,19 +640,9 @@ int64_t b200_keyframes_count(b200_keyframes* h) { return h ? h->count() : -1; }
 
 }  // extern "C"
 
-// appends one keyframe whose cloud is the concatenation of the nparts clouds src[i] (n[i] records at stride[i] bytes)
-static int32_t keyframes_add(b200_keyframes* h, int nparts, const float* const* src, const int64_t* np, const int64_t* stride, const float* pose6,
-                             double time, int64_t n_corner, int64_t* key) {
-    int64_t n = 0;
-    for (int i = 0; i < nparts; ++i) {
-        if (np[i] < 0 || (np[i] > 0 && !src[i]) || stride[i] < 12) B200_FAIL(B200_ERR_ARG, "bad argument");
-        n += np[i];
-    }
-    if (!h || !pose6 || n > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_ARG, "bad argument");
-    if (h->count() >= (int64_t)0x7fffffff) B200_FAIL(B200_ERR_ARG, "keyframe store full");
-    CUDA_SET_DEVICE(h->device);
+// room for n more points in the pool
+static int32_t pool_reserve(b200_keyframes* h, int64_t n) {
     cudaStream_t s = h->stream;
-    const int64_t K = h->count();
     if (h->pool_used + n > h->pool_cap) {  // double the pool, keep what it holds
         const int64_t cap = std::max<int64_t>(std::max<int64_t>(2 * h->pool_cap, h->pool_used + n), 1 << 20);
         float4* q = nullptr;
@@ -666,6 +656,23 @@ static int32_t keyframes_add(b200_keyframes* h, int nparts, const float* const* 
         h->d_pool = q;
         h->pool_cap = cap;
     }
+    return B200_OK;
+}
+
+// appends one keyframe whose cloud is the concatenation of the nparts clouds src[i] (n[i] records at stride[i] bytes)
+static int32_t keyframes_add(b200_keyframes* h, int nparts, const float* const* src, const int64_t* np, const int64_t* stride, const float* pose6,
+                             double time, int64_t n_corner, int64_t* key) {
+    int64_t n = 0;
+    for (int i = 0; i < nparts; ++i) {
+        if (np[i] < 0 || (np[i] > 0 && !src[i]) || stride[i] < 12) B200_FAIL(B200_ERR_ARG, "bad argument");
+        n += np[i];
+    }
+    if (!h || !pose6 || n > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (h->count() >= (int64_t)0x7fffffff) B200_FAIL(B200_ERR_ARG, "keyframe store full");
+    CUDA_SET_DEVICE(h->device);
+    cudaStream_t s = h->stream;
+    const int64_t K = h->count();
+    if (const int32_t rc = pool_reserve(h, n)) return rc;
     KfRec r;
     pose_matrix(pose6, r.T);
     r.time = time;
@@ -704,6 +711,35 @@ int32_t b200_keyframes_add_features(b200_keyframes* h, const float* corner, int6
     const float* src[2] = {corner, surf};
     const int64_t np[2] = {n_corner, n_surf}, stride[2] = {stride_corner, stride_surf};
     return keyframes_add(h, 2, src, np, stride, pose6, time, n_corner, key);
+}
+
+int32_t b200_keyframes_add_features_device(b200_keyframes* h, const void* d_corner, int64_t n_corner, const void* d_surf, int64_t n_surf,
+                                           const float* pose6, double time, int64_t* key) {
+    if (!h || !pose6 || n_corner < 0 || n_surf < 0 || n_corner + n_surf > (int64_t)0x7fffff00) B200_FAIL(B200_ERR_ARG, "bad argument");
+    if (h->count() >= (int64_t)0x7fffffff) B200_FAIL(B200_ERR_ARG, "keyframe store full");
+    CUDA_SET_DEVICE(h->device);
+    if (const int32_t rc = check_device_buffer(d_corner, n_corner, h->device)) return rc;
+    if (const int32_t rc = check_device_buffer(d_surf, n_surf, h->device)) return rc;
+    cudaStream_t s = h->stream;
+    const int64_t K = h->count(), n = n_corner + n_surf;
+    if (const int32_t rc = pool_reserve(h, n)) return rc;
+    KfRec r;
+    pose_matrix(pose6, r.T);
+    r.time = time;
+    CUDA_TRY(h->d_rec.reserve_keep((size_t)K + 1, (size_t)K, s));
+    CUDA_TRY(h->h_rec.reserve(1));
+    h->h_rec.p[0] = r;
+    if (n_corner) CUDA_TRY(cudaMemcpyAsync(h->d_pool + h->pool_used, d_corner, (size_t)n_corner * sizeof(float4), cudaMemcpyDeviceToDevice, s));
+    if (n_surf) CUDA_TRY(cudaMemcpyAsync(h->d_pool + h->pool_used + n_corner, d_surf, (size_t)n_surf * sizeof(float4), cudaMemcpyDeviceToDevice, s));
+    CUDA_TRY(cudaMemcpyAsync(h->d_rec.p + K, h->h_rec.p, sizeof(KfRec), cudaMemcpyHostToDevice, s));
+    CUDA_TRY(cudaStreamSynchronize(s));
+    h->rec.push_back(r);
+    h->off.push_back(h->pool_used);
+    h->n.push_back(n);
+    h->n_corner.push_back(n_corner);
+    h->pool_used += n;
+    if (key) *key = K;
+    return B200_OK;
 }
 
 int32_t b200_keyframes_set_poses(b200_keyframes* h, int64_t first, int64_t count, const float* poses6) {

@@ -32,6 +32,20 @@ struct Submaps {
     int64_t done = 0;                  // segments assembled: a prefix of whole groups
 };
 
+// scratch of the segmented VoxelGrid (seg_downsample), kept by its owner between calls
+struct SegWork {
+    PinnedBuf<uint8_t> h_tab;
+    DevBuf<uint8_t> d_tab;
+    DevBuf<int64_t> d_io;
+    PinnedBuf<int64_t> h_io;
+    DevBuf<float4> d_cent;
+    DevBuf<int32_t> d_mm;
+    PinnedBuf<int32_t> h_mm;
+    DevBuf<unsigned long long> k_in, k_out, k_uniq;
+    DevBuf<int32_t> v_in, v_out, run_cnt, run_off, d_cnt, d_small;
+    DevBuf<uint8_t> keep, cub_tmp;
+};
+
 int32_t check_params(const b200_loop_params* prm);
 // keys[0 .. n) in [0, count); with allow_none, -1 too
 int32_t check_keys(const b200_keyframes* h, const int64_t* keys, int64_t n, bool allow_none);
@@ -47,6 +61,11 @@ int32_t submaps(b200_keyframes* h, cudaStream_t s, const Seg* segs, int64_t nseg
 // The same for general segments: segment j is parts[part_off[j] .. part_off[j+1]) appended in order, downsampled with leaf[j].
 int32_t assemble(b200_keyframes* h, cudaStream_t s, const Part* parts, const int64_t* part_off, const float* leaf, int64_t nseg, int64_t group,
                  Submaps& out);
+// The VoxelGrid half of assemble for device-resident segments: segment j = pts[off[j] .. off[j+1]) (off[0] = 0; d_off the same
+// offsets on the device, outside w.d_tab's bytes from grid_at on, where the grids go), downsampled with leaf[j]; non-finite
+// points are skipped.  Two read-backs (min / max, run ranges); out.pts = w.d_cent, valid until w is used again.
+int32_t seg_downsample(SegWork& w, cudaStream_t s, const float4* pts, const int64_t* d_off, const int64_t* off, size_t grid_at, const float* leaf,
+                       int64_t nseg, int64_t group, Submaps& out);
 // loopFindNearKeyframes(key, num) as parts
 void near_parts(const b200_keyframes* h, int64_t key, int32_t num, std::vector<Part>& parts);
 // e[0 .. n) from pts into dst0 / dst1 as (x, y, z, 0) records, one launch on stream s

@@ -247,6 +247,12 @@ class KeyframeStore {
               "b200_keyframes_add_features");
         return key;
     }
+    /// the same from clouds on the device (b200host::FeatureExtraction::deviceCloud, float4 records)
+    int64_t add(const void* d_corner, int64_t n_corner, const void* d_surf, int64_t n_surf, const float pose6[6], double time) {
+        int64_t key = -1;
+        check(b200_keyframes_add_features_device(h_, d_corner, n_corner, d_surf, n_surf, pose6, time, &key), "b200_keyframes_add_features_device");
+        return key;
+    }
     void setPoses(int64_t first, int64_t count, const float* poses6) { check(b200_keyframes_set_poses(h_, first, count, poses6), "b200_keyframes_set_poses"); }
     int64_t size() const { return b200_keyframes_count(h_); }
     /// detectLoopClosureDistance for the query keyframes cur: pre[q] = -1 without a candidate

@@ -2,6 +2,7 @@
 //
 // ScanToMap mirrors the members mapOptimization uses around scan2MapOptimization (jueying_slam/src/mapOptmization.cpp:1560-1590):
 // the two feature maps (kdtree{Corner,Surf}FromMap->setInputCloud) and transformTobeMapped[6] = roll, pitch, yaw, x, y, z.
+// FeatureExtraction runs imageProjection / featureExtraction / downsampleCurrentScan (LIO-SAM) on raw scans, clouds left on the device.
 // ScanPreprocessor chains ImuProcess::UndistortPcl's backward half (jueying_lio/include/imu_processing.hpp:247-284) and
 // pcl::VoxelGrid::filter (jueying_lio/src/laser_mapping.cc:323-328) on the device.
 #pragma once
@@ -42,6 +43,13 @@ class ScanToMap {
         check(rc, "b200_loam_optimize");
         return rc == B200_OK;
     }
+    /// the same on laserCloud{Corner,Surf}LastDS as FeatureExtraction left them on the device (deviceCloud)
+    bool scan2MapOptimization(const void* d_corner_last_ds, int64_t n_corner, const void* d_surf_last_ds, int64_t n_surf, float transformTobeMapped[6],
+                              int iter_num = 30) {
+        const int32_t rc = b200_loam_optimize_device(h_, d_corner_last_ds, n_corner, d_surf_last_ds, n_surf, transformTobeMapped, iter_num, &stats_);
+        check(rc, "b200_loam_optimize_device");
+        return rc == B200_OK;
+    }
     bool degenerate() const { return stats_.degenerate != 0; }
     const b200_loam_stats& stats() const { return stats_; }
 
@@ -49,6 +57,45 @@ class ScanToMap {
     b200_loam* h_ = nullptr;
     b200_loam_stats stats_{};
     b200_surround_info info_{};
+};
+
+/// imageProjection (projection and cloud extraction, no deskew), featureExtraction and downsampleCurrentScan on the device for
+/// raw scans of PointT (x, y, z and intensity floats, an unsigned 1- or 2-byte `ring`, as velodyne / ouster / livox point types
+/// carry them); the four clouds stay on the device for ScanToMap::scan2MapOptimization and KeyframeStore::add
+template <typename PointT>
+class FeatureExtraction {
+   public:
+    explicit FeatureExtraction(const b200_feature_params& params, int device = 0) { check(b200_features_create(&params, device, &h_), "b200_features_create"); }
+    ~FeatureExtraction() { b200_features_destroy(h_); }
+    FeatureExtraction(const FeatureExtraction&) = delete;
+    FeatureExtraction& operator=(const FeatureExtraction&) = delete;
+
+    /// one scan (laserCloudIn in input order); false when no point survives the projection (empty clouds)
+    template <typename Alloc>
+    bool extract(const std::vector<PointT, Alloc>& scan) {
+        static_assert(sizeof(PointT{}.ring) == 1 || sizeof(PointT{}.ring) == 2, "ring must be a 1- or 2-byte unsigned integer");
+        const PointT p{};
+        const int64_t int_off = (const char*)&p.intensity - (const char*)&p, ring_off = (const char*)&p.ring - (const char*)&p;
+        const int32_t rc = b200_features_extract(h_, scan.empty() ? nullptr : scan.data(), (int64_t)scan.size(), sizeof(PointT), int_off, ring_off,
+                                                 (int32_t)sizeof(p.ring), &info_);
+        check(rc, "b200_features_extract");
+        return rc == B200_OK;
+    }
+    const b200_feature_info& info() const { return info_; }
+    /// B200_FEATURES_CORNER / SURFACE / CORNER_DS / SURF_DS as float4 (x, y, z, intensity) on the device, valid until the next extract
+    const void* deviceCloud(int which, int64_t* n) const { return b200_features_device_cloud(h_, which, n); }
+    /// a copy on the host (x y z intensity per point)
+    std::vector<float> cloud(int which) const {
+        int64_t n = 0;
+        b200_features_device_cloud(h_, which, &n);
+        std::vector<float> out(4 * (size_t)n);
+        check(b200_features_cloud(h_, which, out.data(), n, &n), "b200_features_cloud");
+        return out;
+    }
+
+   private:
+    b200_features* h_ = nullptr;
+    b200_feature_info info_{};
 };
 
 /// raw scan -> (undistort) -> voxel downsample, result left on the device for Esekf::update on device points

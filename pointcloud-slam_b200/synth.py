@@ -389,3 +389,32 @@ def loop_session(K=2000, n_points=1000, laps=2, radius=18.0, drift=(0.3, 1.0), s
         clouds = [_loop_cloud(j) for j in jobs]
     return dict(clouds=clouds, poses=drift6, poses_true=true6, times=np.arange(K, dtype=np.float64),
                 T_true=np.array([pose6_matrix(p) for p in true6]), T_drift=np.array([pose6_matrix(p) for p in drift6]))
+
+
+def spinning_scan(n_scan=16, horizon=1800, seed: int = SEED, fov_deg=(-15.0, 15.0), dup=0.0, origin=(2.0, 1.0, 1.2)):
+    """A spinning-lidar scan of the warehouse world (make_world): n_scan rings x horizon azimuths, returned in firing order
+    (azimuth after azimuth, the rings of one azimuth together).  Returns (xyz float32 [n, 3] in the sensor frame, ring ids
+    uint16 [n], intensities float32 [n]).  dup: the fraction of returns followed by a second return of the same beam, 1 % farther."""
+    rng = np.random.default_rng(seed + 5)
+    az = 2 * np.pi * np.arange(horizon) / horizon
+    el = np.deg2rad(np.linspace(fov_deg[0], fov_deg[1], n_scan))
+    A, E = np.meshgrid(az, el, indexing="ij")
+    dirs = np.stack([np.cos(E) * np.cos(A), np.cos(E) * np.sin(A), np.sin(E)], -1).reshape(-1, 3)
+    xyz = raycast(origin, np.eye(3), dirs, make_world(seed), rmin=-np.inf, rmax=np.inf, seed=seed)
+    ring = np.tile(np.arange(n_scan, dtype=np.uint16), horizon)
+    inten = rng.uniform(0.0, 255.0, len(xyz)).astype(np.float32)
+    if dup:
+        k = np.flatnonzero(rng.random(len(xyz)) < dup)
+        at = np.concatenate([np.arange(len(xyz)), k]) * 2 + np.concatenate([np.zeros(len(xyz), int), np.ones(len(k), int)])
+        order = np.argsort(at, kind="stable")
+        xyz = np.concatenate([xyz, xyz[k] * np.float32(1.01)])[order]
+        ring, inten = np.concatenate([ring, ring[k]])[order], np.concatenate([inten, inten[k]])[order]
+    return xyz, ring, inten
+
+
+def livox_line_scan(n_points=20_000, n_lines=6, seed: int = SEED, origin=(2.0, 1.0, 1.2)):
+    """A Livox-shaped scan of the warehouse world (livox_dirs) tagged with line ids (point i on line i % n_lines), in arrival
+    order.  Returns (xyz float32 [n, 3], line ids uint8 [n], intensities float32 [n])."""
+    rng = np.random.default_rng(seed + 6)
+    xyz = raycast(origin, np.eye(3), livox_dirs(n_points, seed), make_world(seed), rmin=-np.inf, rmax=np.inf, seed=seed)
+    return xyz, (np.arange(len(xyz)) % n_lines).astype(np.uint8), rng.uniform(0.0, 255.0, len(xyz)).astype(np.float32)
